@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this engine
     python bench.py --impl reference --gpus N --steps K ...   # reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's proofs as DIR/*.npy
 
 Workload (BASELINE.json configs[1]; seeding of the reference's own tests/benchmark/bench_ring_proof.py:
 47-77,140-152): one 1023-key ring, signer at index 3, per step ONE batch of `--total` (4096) proofs with
@@ -385,6 +386,8 @@ def run_ours(args) -> None:
         raise SystemExit("bench.py: proofs of the timed region do not verify; refusing to report a number")
     parity["verified_sample"] = k
     oracle_sample = [(last[i], la[i], ld[i]) for i in picks[:3]]
+    if args.dump_outputs:
+        dump_outputs(Path(args.dump_outputs), last, lo, "proofs" if world == 1 else f"proofs_rank{rank}", world)
 
     # integer-pipe ceiling measured live on this GPU (dependent-free mad.lo.u32, all SMs)
     if dry_run:
@@ -496,6 +499,27 @@ def run_ours(args) -> None:
     emit(line)
     if last:
         sys.stderr.write(f"[bench] last proof sha256 {hashlib.sha256(last[-1]).hexdigest()[:16]}\n")
+
+
+DUMP_LIMIT_BYTES = 64_000_000  # all files of one dump, over all ranks
+NPY_HEADERS_BYTES = 1024  # allowance for the headers of one rank's two .npy files
+
+
+def dump_outputs(out_dir: Path, proofs: list[bytes], first_index: int, name: str, world: int, limit: int = DUMP_LIMIT_BYTES) -> None:
+    """`<name>.npy`: the proofs of the last timed step, one row of 784 byte values per proof (float32, exact);
+    `<name>_index.npy`: the index of each row in the step's batch (float64).  The `world` ranks share `limit` bytes
+    equally; above its share a rank writes a fixed, seeded sample of its rows, so that two builds given the same
+    arguments can be compared output for output."""
+    import numpy as np
+
+    rows = np.frombuffer(b"".join(proofs), dtype=np.uint8).reshape(len(proofs), 784)
+    index = np.arange(len(proofs))
+    keep = (limit // world - NPY_HEADERS_BYTES) // (784 * 4 + 8)
+    if len(proofs) > keep:
+        index = np.sort(np.random.default_rng(0).choice(len(proofs), size=keep, replace=False))
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / f"{name}.npy", rows[index].astype(np.float32))
+    np.save(out_dir / f"{name}_index.npy", (index + first_index).astype(np.float64))
 
 
 def workload_string(strong: bool, total: int, n_dev: int, batch: int | None) -> str:
@@ -657,7 +681,14 @@ def main() -> None:
     ap.add_argument("--commit-mode", type=int, default=int(os.environ.get("DOT_RING_B200_COMMIT_MODE", "0")), help="0 XYZZ accumulation, 1 batched-affine rounds")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-workers", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the proofs of the last timed step to DIR/proofs.npy (float32 byte values, one row per proof) and their batch indices to DIR/proofs_index.npy; "
+                    "inside the repository use bench_outputs/, which git ignores")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the proofs of this engine; --impl reference keeps none")
     if args.batch is not None:
         args.scaling = "weak"
     elif args.scaling == "weak":
