@@ -4,18 +4,19 @@
 
 namespace dr {
 
-// window bits minimising W * (2n + weight * 2^(c-1)) mixed-addition equivalents over the 2n GLV halves.  For large sets a bucket costs
+// window bits minimising W * (n + weight * 2^(c-1)) mixed-addition equivalents.  For large sets a bucket costs
 // far more than the 2.8 additions of its arithmetic: the fold / running-sum / window kernels are short dependent chains on few threads
 // (measured at 2^20 points: 0.43 ns per bucket addition against ~11 ns per bucket), so the model charges a bucket 16 additions from
 // 2^18 points on.  Below, those kernels are latency-bound whatever the bucket count and the plain arithmetic count picks better
-// (measured sweep, profiles/r02_probe_msm_sweep*.json: 3.0 vs 3.4 ms at 2^16, 5.1 vs 5.3 ms at 2^18, 11.9 vs 13.3 ms at 2^20).
+// (measured with the endomorphism-split recoding this file used before, profiles/r02_probe_msm_sweep*.json: 3.0 vs 3.4 ms at 2^16,
+// 5.1 vs 5.3 ms at 2^18, 11.9 vs 13.3 ms at 2^20).
 static uint32_t msm_window_bits(size_t n) {
     uint32_t best = 4;
     double best_cost = 1e300;
     const double weight = n >= ((size_t)1 << 18) ? 16.0 : 2.8;
     for (uint32_t c = 4; c <= 17; c++) {
-        double W = (MSM_GLV_BITS + c - 1) / c;
-        double cost = W * (2.0 * (double)n + weight * (double)(1u << (c - 1)));
+        double W = (MSM_BITS + c - 1) / c;
+        double cost = W * ((double)n + weight * (double)(1u << (c - 1)));
         if (cost < best_cost) {
             best_cost = cost;
             best = c;
@@ -30,14 +31,12 @@ struct MsmWork {
     DevBuf<int32_t> digits;
     DevBuf<uint32_t> count, offset, unit_offset, cursor, totals, refs, block_tot;
     DevBuf<G1> unit_sum, bucket, seg_sum, window_sum;
-    DevBuf<G1Affine> result, vpoints;
+    DevBuf<G1Affine> result;
     void prepare(size_t n_points) {
         g.n = (uint32_t)n_points;
-        g.nv = 2 * g.n;
-        const size_t n = g.nv;  // everything below is sized by the virtual points
-        vpoints.ensure(n);
+        const size_t n = n_points;
         g.c = msm_window_bits(n_points);
-        g.W = (MSM_GLV_BITS + g.c - 1) / g.c;
+        g.W = (MSM_BITS + g.c - 1) / g.c;
         g.H = 1u << (g.c - 1);
         segs = (g.H + MSM_SEGMENT - 1) / MSM_SEGMENT;
         const size_t nb = g.buckets();
@@ -63,16 +62,15 @@ static void msm_device(Ctx* ctx, MsmWork& w, const G1Affine* points, const uint8
     const uint32_t nb = g.buckets();
     Stream st = ctx->stream;
     dev_zero(st, w.count.p, (size_t)nb * 4);
-    launch(st, Dim3((g.n + 127) / 128), 128, 0, MsmPhiBody(), points, g.n, w.vpoints.p);
     launch(st, Dim3((g.n + 127) / 128), 128, 0, MsmDigitsBody(), scalars_le32, g, w.digits.p, w.count.p);
     const uint32_t tiles = (nb + SCAN_TILE - 1) / SCAN_TILE;
     launch(st, Dim3(tiles), SCAN_TILE, 4 * SCAN_TILE * sizeof(uint32_t), MsmScanTileBody(), (const uint32_t*)w.count.p, nb, w.offset.p, w.unit_offset.p, w.block_tot.p);
     launch(st, Dim3(1), 32, 0, MsmScanBlocksBody(), w.block_tot.p, tiles, w.totals.p);
     launch(st, Dim3(tiles), SCAN_TILE, 0, MsmScanApplyBody(), nb, (const uint32_t*)w.block_tot.p, w.offset.p, w.unit_offset.p, w.cursor.p);
-    launch(st, Dim3((g.nv + 127) / 128), 128, 0, MsmScatterBody(), g, (const int32_t*)w.digits.p, (const uint32_t*)w.offset.p, w.cursor.p, w.refs.p);
+    launch(st, Dim3((g.n + 127) / 128), 128, 0, MsmScatterBody(), g, (const int32_t*)w.digits.p, (const uint32_t*)w.offset.p, w.cursor.p, w.refs.p);
     // upper bound on the unit count is known on the host; threads beyond totals[0] exit
-    const size_t max_units = (size_t)g.W * g.nv / MSM_UNIT + nb + 1;
-    launch(st, Dim3((uint32_t)((max_units + 63) / 64)), 64, 0, MsmUnitSumBody(), g, (const G1Affine*)w.vpoints.p, (const uint32_t*)w.count.p, (const uint32_t*)w.offset.p,
+    const size_t max_units = (size_t)g.W * g.n / MSM_UNIT + nb + 1;
+    launch(st, Dim3((uint32_t)((max_units + 63) / 64)), 64, 0, MsmUnitSumBody(), g, points, (const uint32_t*)w.count.p, (const uint32_t*)w.offset.p,
            (const uint32_t*)w.unit_offset.p, (const uint32_t*)w.totals.p, (const uint32_t*)w.refs.p, w.unit_sum.p);
     launch(st, Dim3((nb + 63) / 64), 64, 0, MsmBucketFoldBody(), g, (const uint32_t*)w.count.p, (const uint32_t*)w.unit_offset.p, (const G1*)w.unit_sum.p, w.bucket.p);
     launch(st, Dim3(nb), 64, 64 * sizeof(G1), MsmBucketFoldHeavyBody(), (const uint32_t*)w.count.p, (const uint32_t*)w.unit_offset.p, (const G1*)w.unit_sum.p, w.bucket.p);

@@ -173,7 +173,19 @@ static void ring_proof_verify_device(Ctx* ctx, const VerifierKeyDev& vk, size_t 
     h2d(ctx->stream, dco.p, coeffs_le32, n * 64);
     const uint32_t m = (uint32_t)n;
     launch(ctx->stream, Dim3((7 * m + 63) / 64), 64, 0, PayloadG1DecodeBody(), payloads, stride, m, vs.p);
+    // the subgroup tests of the decoded points overlap the transcript algebra; joined before the G1 terms read them
+    struct Side2Join {
+        Ctx* c;
+        bool pending;
+        ~Side2Join() {
+            if (pending) c->join_side2();
+        }
+    } side2_join{ctx, true};
+    ctx->fork_side2();
+    launch(ctx->side2, Dim3((7 * m + 63) / 64), 64, 0, PayloadG1SubgroupBody(), m, vs.p);
     launch(ctx->stream, Dim3((m + 63) / 64), 64, 0, RingVerifyAlgebraBody(), vk, payloads, stride, relations, rel_stride, (const uint8_t*)dco.p, m, vs.p);
+    ctx->join_side2();
+    side2_join.pending = false;
     uint32_t all = 0;
     const bool by_msm = aggregate && n >= RING_VERIFY_MSM_THRESHOLD.load();
     if (!by_msm) launch(ctx->stream, Dim3((2 * VERIFY_TERMS * m + 63) / 64), 64, 0, RingVerifyTermsBody(), vk, m, vs.p);

@@ -92,6 +92,26 @@ DR_HD void glv_half(const uint32_t* k, uint32_t which, uint32_t* out) {
     for (int i = 4; i < 8; i++) out[i] = 0;
 }
 
+// G1 membership (Scott, ePrint 2021/1130): a point P of E(Fq) lies in G1 iff [x^2]P == -phi^2(P) = (beta^2 X, -Y), with
+// beta^2 = -1 - beta.  Decoding checks no subgroup (blst's P1_Affine(bytes) does not), and k1 * P + k2 * phi(P) equals k * P only
+// on G1: the verifier sends the points that fail this test down a plain full-scalar path, so every curve point gets blst's k * P.
+DR_HD_COLD G1 g1_mul_abs_x(const G1& p) {  // [|x|]P, |x| = 0xd201000000010000
+    G1 acc = p;
+#pragma unroll 1
+    for (int bit = 62; bit >= 0; bit--) {
+        acc = g1_dbl(acc);
+        if ((0xd201000000010000ull >> bit) & 1) g1_add(acc, p);
+    }
+    return acc;
+}
+DR_HD_COLD bool g1_in_subgroup(const G1Affine& a) {
+    if (a.is_inf()) return true;
+    const G1 t = g1_mul_abs_x(g1_mul_abs_x(G1::from_affine(a)));
+    if (t.is_inf()) return false;
+    const Fq b2x = (a.x + a.x * glv_beta()).neg();
+    return t.X == b2x * t.ZZ && t.Y == a.y.neg() * t.ZZZ;
+}
+
 struct TableGeom {
     uint32_t c;        // bits of a (narrow) window
     uint32_t W;        // windows; W * c + wide >= 256 (128 with glv)

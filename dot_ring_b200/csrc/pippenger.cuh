@@ -23,49 +23,29 @@ namespace dr {
 constexpr uint32_t MSM_UNIT = 16;     // points per work unit (small units keep the lanes of a warp in step)
 constexpr uint32_t MSM_SEGMENT = 16;  // buckets per running-sum segment (short serial chains; the segments are tree-folded)
 
-// Every scalar is split by the G1 endomorphism (msm.cuh: k = k1 + k2 lambda, both halves below 2^128), so the bucket method runs over
-// nv = 2n "virtual" points -- P_i with k1_i and phi(P_i) = (beta x_i, y_i) with k2_i -- and 129 bits: the same number of bucket
-// additions as 256 bits over n points, but half the windows to reduce and half the doublings in the serial tail.
+// Scalars are not split by the G1 endomorphism here (the commit tables of msm.cuh are): k1 * P + k2 * phi(P) equals k * P only on G1,
+// and these point sets come from callers, where blst's mult_pippenger gives the integer multiple k * P for any curve point.  The
+// plain recoding is exact for every point without a per-point subgroup test; against the split it has the same number of bucket
+// additions and twice the windows to reduce.
 struct MsmGeom {
-    uint32_t n, nv, c, W, H;  // n points, nv = 2n virtual points, H = 2^(c-1) buckets per window
+    uint32_t n, c, W, H;  // n points, H = 2^(c-1) buckets per window
     DR_HD uint32_t buckets() const { return W * H; }
 };
-constexpr uint32_t MSM_GLV_BITS = 129;  // 128-bit halves + the carry of the signed recoding
+constexpr uint32_t MSM_BITS = 256;  // scalars below r < 2^255 + the carry of the signed recoding
 
-// vpoints[i] = P_i, vpoints[n + i] = phi(P_i)
-struct MsmPhiBody {
-    DR_HD void operator()(const BlockCtx& ctx, const G1Affine* points, uint32_t n, G1Affine* vpoints) const {
-        DR_THREAD_LOOP(t, ctx) {
-            uint32_t i = ctx.bx * ctx.nthreads + t;
-            if (i < n) {
-                G1Affine p = points[i];
-                vpoints[i] = p;
-                if (!p.is_inf()) p.x = p.x * glv_beta();
-                vpoints[n + i] = p;
-            }
-        }
-    }
-};
-
-// scalars: n x 32-byte little-endian (any value < 2^256, reduced mod r here) -> digits[w * nv + v] for the two halves v = i, n + i
+// scalars: n x 32-byte little-endian (any value < 2^256, reduced mod r here) -> digits[w * n + i]
 struct MsmDigitsBody {
     DR_HD void operator()(const BlockCtx& ctx, const uint8_t* scalars_le32, MsmGeom g, int32_t* digits, uint32_t* count) const {
         DR_THREAD_LOOP(t, ctx) {
             uint32_t i = ctx.bx * ctx.nthreads + t;
             if (i < g.n) {
                 Fr k = fp_from_le_bytes_mod<Fr>(scalars_le32 + 32 * (size_t)i, 32).from_mont();
+                uint32_t carry = 0;
 #pragma unroll 1
-                for (uint32_t h = 0; h < 2; h++) {
-                    uint32_t half[8];
-                    glv_half(k.v, h, half);
-                    const uint32_t v = h * g.n + i;
-                    uint32_t carry = 0;
-#pragma unroll 1
-                    for (uint32_t w = 0; w < g.W; w++) {
-                        int d = msm_digit(half, w, g.c, carry);
-                        digits[(size_t)w * g.nv + v] = d;
-                        if (d) atomic_add_u32(&count[w * g.H + (uint32_t)(d < 0 ? -d : d) - 1], 1u);
-                    }
+                for (uint32_t w = 0; w < g.W; w++) {
+                    int d = msm_digit(k.v, w, g.c, carry);
+                    digits[(size_t)w * g.n + i] = d;
+                    if (d) atomic_add_u32(&count[w * g.H + (uint32_t)(d < 0 ? -d : d) - 1], 1u);
                 }
             }
         }
@@ -146,10 +126,10 @@ struct MsmScatterBody {
     DR_HD void operator()(const BlockCtx& ctx, MsmGeom g, const int32_t* digits, const uint32_t* offset, uint32_t* cursor, uint32_t* refs) const {
         DR_THREAD_LOOP(t, ctx) {
             uint32_t i = ctx.bx * ctx.nthreads + t;
-            if (i < g.nv) {
+            if (i < g.n) {
 #pragma unroll 1
                 for (uint32_t w = 0; w < g.W; w++) {
-                    int d = digits[(size_t)w * g.nv + i];
+                    int d = digits[(size_t)w * g.n + i];
                     if (d) {
                         uint32_t b = w * g.H + (uint32_t)(d < 0 ? -d : d) - 1;
                         uint32_t slot = atomic_add_u32(&cursor[b], 1u);

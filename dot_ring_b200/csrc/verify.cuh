@@ -541,7 +541,8 @@ constexpr int VERIFY_TERMS = 13;  // scalar multiplications per proof (see RingV
 
 struct VerifyState {
     uint32_t status;
-    G1Affine g1[7];  // C_b, C_accip, C_accx, C_accy, C_q, Phi_zeta, Phi_zeta_omega
+    G1Affine g1[7];      // C_b, C_accip, C_accx, C_accy, C_q, Phi_zeta, Phi_zeta_omega
+    uint8_t outside[7];  // g1[j] decoded but not in G1 (g1_in_subgroup): its terms take a full-scalar multiplication
     Fr sc[VERIFY_TERMS];
     G1 term[2 * VERIFY_TERMS];  // sc[j] * base_j as two GLV halves: term[2j] = k1 * P, term[2j + 1] = k2 * phi(P)
 };
@@ -558,6 +559,20 @@ struct PayloadG1DecodeBody {
                 bool good = g1_decode(a, payloads + (size_t)stride * p + off[j], 48);
                 vs[p].g1[j] = good ? a : G1Affine::inf();
                 if (!good) vs[p].status = ST_MALFORMED;  // racing writers store the same value
+            }
+        }
+    }
+};
+
+// G1 membership of the decoded points, one thread per point: outside[j] sends g1[j]'s terms to a full-scalar multiplication
+// (RingVerifyTermsBody).  Nothing else reads it, so it runs on a side stream next to RingVerifyAlgebraBody.
+struct PayloadG1SubgroupBody {
+    DR_HD void operator()(const BlockCtx& ctx, uint32_t count, VerifyState* vs) const {
+        DR_THREAD_LOOP(t, ctx) {
+            uint32_t i = ctx.bx * ctx.nthreads + t;
+            if (i < 7 * count) {
+                uint32_t p = i / 7, j = i % 7;
+                vs[p].outside[j] = g1_in_subgroup(vs[p].g1[j]) ? 0 : 1;  // infinity (and a malformed point, stored as infinity) is in G1
             }
         }
     }
@@ -722,7 +737,9 @@ DR_HD_COLD G1 g1_mul_raw(const G1Affine& p, const uint32_t* k, int nlimbs) {
 }
 
 // one thread per (proof, term, GLV half): sc * P = k1 * P + k2 * phi(P) with 128-bit k1, k2 (msm.cuh glv_half), phi(x, y) = (beta x, y):
-// half the doublings of a 255-bit multiplication, on twice the threads
+// half the doublings of a 255-bit multiplication, on twice the threads.  A decoded point outside G1 takes sc * P whole on the first
+// half's thread (the split is exact only on G1; g1_mul_raw's affine table assumes no multiple 2P .. 15P is infinity, which a
+// small-order component breaks); the fixed points are commitments over the SRS, in G1.
 struct RingVerifyTermsBody {
     DR_HD void operator()(const BlockCtx& ctx, VerifierKeyDev vk, uint32_t count, VerifyState* vs) const {
         DR_THREAD_LOOP(t, ctx) {
@@ -730,14 +747,19 @@ struct RingVerifyTermsBody {
             if (i < 2 * VERIFY_TERMS * count) {
                 uint32_t p = i / (2 * VERIFY_TERMS), r = i % (2 * VERIFY_TERMS), j = r >> 1, h = r & 1;
                 VerifyState& s = vs[p];
-                G1Affine base = j < 7 ? s.g1[j] : j < 9 ? s.g1[j - 2] : vk.fixed[j - 9];
+                const uint32_t src = j < 7 ? j : j - 2;  // index into s.g1 for j < 9
+                G1Affine base = j < 9 ? s.g1[src] : vk.fixed[j - 9];
                 G1 out = G1::inf();
                 if (!(s.status & ST_MALFORMED) && !base.is_inf()) {
                     Fr k = s.sc[j].from_mont();
-                    uint32_t half[8];
-                    glv_half(k.v, h, half);
-                    if (h) base.x = base.x * glv_beta();
-                    out = g1_mul_raw(base, half, 4);
+                    if (j < 9 && s.outside[src]) {
+                        if (!h) out = g1_mul_limbs(G1::from_affine(base), k.v);  // XYZZ table: multiples of a small-order point may be infinity
+                    } else {
+                        uint32_t half[8];
+                        glv_half(k.v, h, half);
+                        if (h) base.x = base.x * glv_beta();
+                        out = g1_mul_raw(base, half, 4);
+                    }
                 }
                 s.term[r] = out;
             }

@@ -115,6 +115,12 @@ int ht_g1_decode(const uint8_t* in, int len, uint8_t* out96) {
     g1_serialize(out96, a);
     return 1;
 }
+int ht_g1_in_subgroup(const uint8_t* in96) {
+    G1Affine a;
+    if (!g1_decode(a, in96, 96)) return -1;
+    return g1_in_subgroup(a) ? 1 : 0;
+}
+
 void ht_g1_compress(const uint8_t* in96, uint8_t* out48) {
     G1Affine a;
     g1_decode(a, in96, 96);
@@ -146,6 +152,14 @@ void ht_g1_mul(const uint8_t* a96, const uint8_t* k32le, uint8_t* out96) {
         base = g1_dbl(base);
     }
     g1_serialize(out96, g1_to_affine(acc));
+}
+// out = k * a by g1_mul_limbs (4-bit windows over an XYZZ table: the verifier's multiplication for points outside G1)
+void ht_g1_mul_limbs(const uint8_t* a96, const uint8_t* k32le, uint8_t* out96) {
+    G1Affine a;
+    g1_decode(a, a96, 96);
+    uint32_t k[8];
+    memcpy(k, k32le, 32);
+    g1_serialize(out96, g1_to_affine(g1_mul_limbs(G1::from_affine(a), k)));
 }
 // out = k * a using mixed additions only (left-to-right)
 void ht_g1_mul_mixed(const uint8_t* a96, const uint8_t* k32le, uint8_t* out96) {

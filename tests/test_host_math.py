@@ -127,6 +127,28 @@ def test_g1_group_law_and_codecs(lib):
     assert lib.ht_g1_decode(bytes([0xC0]) + bytes(47), 48, out96) and out96.raw == inf
 
 
+def test_g1_subgroup_membership(lib):
+    """msm.cuh g1_in_subgroup (the verifier's switch between the GLV split and a full multiplication) against [r]P == O."""
+    from tests.adversarial_cases import in_g1, membership_points
+
+    lib.ht_g1_in_subgroup.argtypes = [ctypes.c_char_p]
+    for pt in membership_points(6):
+        assert lib.ht_g1_in_subgroup(bls.g1_serialize(pt)) == int(in_g1(pt)), bls.g1_to_affine(pt)
+
+
+def test_g1_full_multiplication_outside_the_subgroup(lib):
+    """g1_mul_limbs on small-order points and points with a small-order component: multiples inside its window table reach
+    infinity (3T, 6T, ... for a point T of order 3), and the product must still be the integer multiple k * P."""
+    from tests.adversarial_cases import membership_points
+
+    rng = random.Random(12)
+    for pt in membership_points(4):
+        for k in (1, 2, 3, 6, 11, 15, 0x1234567, bls.R - 1, rng.randrange(bls.R)):
+            out = _buf(96)
+            lib.ht_g1_mul_limbs(bls.g1_serialize(pt), k.to_bytes(32, "little"), out)
+            assert out.raw == bls.g1_serialize(bls.g1_mul_raw(pt, k)), (bls.g1_to_affine(pt), k)
+
+
 def test_batched_affine_round_exceptional_cases(lib):
     """msm.cuh affine_round: generic pairs share one inversion with P + P (denominator 2y), P - P and infinity operands."""
     rng = random.Random(9)
