@@ -10,8 +10,8 @@ Public names mirror ``dot_ring`` (dot_ring/__init__.py:32-77) for the path this 
 from .curve import Bandersnatch, Bandersnatch_SHAKE128
 from .kzg import KZG
 from .params import RingProofParams
-from .ring import Ring, RingRoot
+from .ring import Ring, RingRoot, RingVerifier
 from .vrf import PedersenVRF, RingVRF, ThinVRF, TinyVRF
 
-__all__ = ["Bandersnatch", "Bandersnatch_SHAKE128", "KZG", "RingProofParams", "Ring", "RingRoot", "RingVRF", "PedersenVRF", "TinyVRF", "ThinVRF", "__version__"]
+__all__ = ["Bandersnatch", "Bandersnatch_SHAKE128", "KZG", "RingProofParams", "Ring", "RingRoot", "RingVerifier", "RingVRF", "PedersenVRF", "TinyVRF", "ThinVRF", "__version__"]
 __version__ = "0.1.0"

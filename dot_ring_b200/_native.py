@@ -114,6 +114,10 @@ class Library:
         L.dr_ring_proof_verify_batch.argtypes = [c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_int, c_void_p, POINTER(c_int)]
         L.dr_ring_verify_batch.argtypes = [c_void_p, c_void_p, c_size_t] + [c_void_p] * 7 + [c_int, c_void_p, POINTER(c_int)]
         L.dr_ring_verify_set_msm_threshold.argtypes = [c_size_t]
+        L.dr_ring_verifier_create.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, POINTER(c_void_p)]
+        L.dr_ring_verifier_destroy.argtypes = [c_void_p]
+        L.dr_ring_verifier_destroy.restype = None
+        L.dr_ring_verify_multi.argtypes = [c_void_p, c_void_p, c_size_t, c_void_p, c_size_t] + [c_void_p] * 7 + [c_int, c_void_p, POINTER(c_int)]
         L.dr_vrf_verify_set_coop_threshold.argtypes = [c_size_t]
         L.dr_pairing_check_batch.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
         L.dr_te_decode_batch.argtypes = [c_void_p, c_void_p, c_size_t, c_int, c_void_p, c_void_p]
@@ -593,6 +597,23 @@ def _fill(arr, data: bytes) -> None:
     _put(arr, bytes(data))
 
 
+def make_ring_params(*, domain_size: int, omega: int, seed, blinding_base, generator, suite_id: bytes, h2c_dst: bytes, hash_name: str = "sha512", max_ring_size: int = 0,
+                     padding_rows: int = 0, radix_omega: int = 0, padding_point=(0, 0)) -> RingParamsStruct:
+    p = RingParamsStruct()
+    p.domain_size, p.max_ring_size, p.padding_rows = domain_size, max_ring_size, padding_rows
+    p.suite_id_len, p.h2c_dst_len = len(suite_id), len(h2c_dst)
+    p.hash_id = HASH_IDS[hash_name]
+    _fill(p.omega, int(omega).to_bytes(32, "little"))
+    _fill(p.radix_omega, int(radix_omega).to_bytes(32, "little"))
+    _fill(p.seed, _xy(seed))
+    _fill(p.blinding_base, _xy(blinding_base))
+    _fill(p.padding_point, _xy(padding_point))
+    _fill(p.generator, _xy(generator))
+    _fill(p.suite_id, suite_id)
+    _fill(p.h2c_dst, h2c_dst)
+    return p
+
+
 def _xy(pt) -> bytes:
     return int(pt[0]).to_bytes(32, "little") + int(pt[1]).to_bytes(32, "little")
 
@@ -604,18 +625,8 @@ class NativeRing:
                  seed, blinding_base, padding_point, generator, suite_id: bytes, h2c_dst: bytes, hash_name: str = "sha512"):
         self.srs = srs
         self.ctx = srs.ctx
-        p = RingParamsStruct()
-        p.domain_size, p.max_ring_size, p.padding_rows = domain_size, max_ring_size, padding_rows
-        p.suite_id_len, p.h2c_dst_len = len(suite_id), len(h2c_dst)
-        p.hash_id = HASH_IDS[hash_name]
-        _fill(p.omega, int(omega).to_bytes(32, "little"))
-        _fill(p.radix_omega, int(radix_omega).to_bytes(32, "little"))
-        _fill(p.seed, _xy(seed))
-        _fill(p.blinding_base, _xy(blinding_base))
-        _fill(p.padding_point, _xy(padding_point))
-        _fill(p.generator, _xy(generator))
-        _fill(p.suite_id, suite_id)
-        _fill(p.h2c_dst, h2c_dst)
+        p = make_ring_params(domain_size=domain_size, max_ring_size=max_ring_size, padding_rows=padding_rows, omega=omega, radix_omega=radix_omega, seed=seed,
+                             blinding_base=blinding_base, padding_point=padding_point, generator=generator, suite_id=suite_id, h2c_dst=h2c_dst, hash_name=hash_name)
         for key in keys:
             if len(key) != 32:
                 raise ValueError("ring keys must be 32 bytes")
@@ -734,3 +745,61 @@ class NativeRing:
         arr = (c_float * 6)()
         self.ctx.library.check(self.ctx.library.lib.dr_ring_prove_phase_ms(self.ctx.handle, ctypes.byref(arr)))
         return [float(x) for x in arr]
+
+
+class NativeRingVerifier:
+    """dr_ring_verifier: the verifier key of one ring built from its 144-byte root alone (no keys, no SRS window table)."""
+
+    def __init__(self, ctx: Context, root144: bytes, g1_0_be96: bytes, g2_be192: bytes, *, domain_size: int, omega: int, seed, blinding_base, generator,
+                 suite_id: bytes, h2c_dst: bytes, hash_name: str = "sha512"):
+        if len(root144) != 144:
+            raise ValueError(f"invalid ring root length: ring root must be exactly 144 bytes, got {len(root144)}")
+        if len(g1_0_be96) != 96 or len(g2_be192) != 384:
+            raise ValueError("expected [1]_1 (96 bytes) and [1]_2 | [tau]_2 (384 bytes)")
+        self.ctx = ctx
+        self.domain_size = domain_size
+        self.handle = c_void_p()
+        p = make_ring_params(domain_size=domain_size, omega=omega, seed=seed, blinding_base=blinding_base, generator=generator, suite_id=suite_id, h2c_dst=h2c_dst,
+                             hash_name=hash_name)
+        lib = ctx.library
+        lib.check(lib.lib.dr_ring_verifier_create(ctx.handle, ctypes.byref(p), bytes(g1_0_be96), bytes(g2_be192), bytes(root144), ctypes.byref(self.handle)))
+
+    def close(self) -> None:
+        if self.handle:
+            self.ctx.library.lib.dr_ring_verifier_destroy(self.handle)
+            self.handle = c_void_p()
+
+    def __del__(self):  # pragma: no cover
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @staticmethod
+    def verify_multi(verifiers: list["NativeRingVerifier"], index: list[int], inputs: list[bytes], ads: list[bytes], proofs: list[bytes], coeffs: list[int],
+                     aggregate: bool = False):
+        """Item i against verifiers[index[i]] (one call, one context) -> (per-item verdicts 1 / 0 / 2, all_ok); aggregate folds every item
+        into one pairing check."""
+        n = len(proofs)
+        if not verifiers:
+            raise ValueError("at least one ring verifier is required")
+        if any(len(p) != 784 for p in proofs):
+            raise ValueError("invalid Ring VRF proof length: Ring VRF proof must be exactly 784 bytes")
+        if len(coeffs) != 2 * n or len(index) != n:
+            raise ValueError("one ring index and two batching coefficients per proof are required")
+        if any(not 0 <= int(k) < len(verifiers) for k in index):
+            raise ValueError("ring index out of range")
+        ctx = verifiers[0].ctx
+        blob, a, b, c, d = pack_items(inputs, ads)
+        handles = (c_void_p * len(verifiers))(*[v.handle for v in verifiers])
+        idx = np.ctypeslib.as_ctypes(np.array(index if n else [0], dtype=np.uint32))
+        out = ctypes.create_string_buffer(max(n, 1))
+        all_ok = c_int(0)
+        lib = ctx.library
+        lib.check(
+            lib.lib.dr_ring_verify_multi(
+                ctx.handle, handles, len(verifiers), idx, n, blob, a, b, c, d, b"".join(proofs), b"".join(int(v).to_bytes(32, "little") for v in coeffs),
+                1 if aggregate else 0, out, ctypes.byref(all_ok),
+            )
+        )
+        return list(out.raw[:n]), bool(all_ok.value)

@@ -97,6 +97,14 @@ struct Ctx {
     static constexpr size_t FIXED_TABLE_CAP = 16;
     std::vector<std::shared_ptr<FixedTable>> fixed_tables;
     std::shared_ptr<FixedTable> fixed_table(const TEAffine& base);
+    // Miller-loop lines of one ([1]_2, [tau]_2) pair (pairing_warp.cuh), shared by every verifier key over those points: a batch
+    // that mixes rings of one SRS folds into one pairing check with one set of lines
+    struct G2Lines {
+        uint8_t g2_be192[384];
+        DevBuf<LineCoeffs> lines;
+    };
+    std::vector<std::shared_ptr<G2Lines>> g2_lines;  // the most recent FIXED_TABLE_CAP pairs
+    std::shared_ptr<G2Lines> pairing_lines(const uint8_t* g2_be192, const G2Affine g2[2]);
     bool have_pairing_consts = false;
     PairingConsts pairing_k;
     const PairingConsts& pairing_consts() {
@@ -210,14 +218,15 @@ struct Ring {
     TEAffine padding;
     const struct LagrangeTable* lag = nullptr;  // owned by the Srs (shared by every ring on the same domain)
     VerifierKeyDev vk{};
-    DevBuf<LineCoeffs> vk_lines;
+    std::shared_ptr<Ctx::G2Lines> vk_lines;
+    DevBuf<VerifierKeyDev> vk_dev;  // vk on the device: the one-entry key table of the verification kernels
     SuiteDev suite{};
     std::shared_ptr<Ctx::FixedTable> g_table, b_table;
 };
 
 
 VerifierKeyDev make_verifier_key(Ctx* ctx, uint32_t N, const Fr& omega, const TEAffine& seed, const uint8_t* label, uint32_t label_len, const uint8_t* g1_0_be96,
-                                 const uint8_t* g2_be192, const uint8_t* fixed_be96, DevBuf<LineCoeffs>& lines);
+                                 const uint8_t* g2_be192, const uint8_t* fixed_be96, std::shared_ptr<Ctx::G2Lines>& lines);
 
 // Fixed-base window table (msm.cuh) for n affine points already on the device.
 void build_window_table(Ctx* ctx, const G1Affine* points, const TableGeom& geom, DevBuf<G1Affine>& table);

@@ -175,9 +175,6 @@ int dr_kzg_pairing_check(dr_ctx* c, dr_srs* s, const uint8_t* lhs_points_be96, c
     if (!ctx || !srs || !ok || (n_lhs && (!lhs_points_be96 || !lhs_scalars_le32)) || (n_rhs && (!rhs_points_be96 || !rhs_scalars_le32))) throw Error(DR_EINVAL, "bad argument");
     ctx->activate();
     *ok = 0;
-    VerifierKeyDev vk{};
-    vk.lines = srs->pairing_lines();
-    vk.pc = ctx->pairing_consts();
     const uint32_t parts = 8;
     DevBuf<G1> pairs(2 * parts);  // (lhs, rhs) interleaved, as RingVerifyAggregateBody folds them
     DevBuf<uint32_t> bad(1), dall(1);
@@ -193,7 +190,7 @@ int dr_kzg_pairing_check(dr_ctx* c, dr_srs* s, const uint8_t* lhs_points_be96, c
     d2h(ctx->stream, &bad_h, bad.p, 4);
     stream_sync(ctx->stream);
     if (bad_h) throw Error(DR_EINVAL, "invalid BLS12-381 G1 encoding");
-    launch(ctx->stream, Dim3(1), 32, ring_verify_warp_smem(), RingVerifyAggregateBody(), vk, (const G1*)pairs.p, parts, (const uint32_t*)bad.p, dall.p);
+    launch(ctx->stream, Dim3(1), 32, ring_verify_warp_smem(), RingVerifyAggregateBody(), srs->pairing_lines(), ctx->pairing_consts(), (const G1*)pairs.p, parts, (const uint32_t*)bad.p, dall.p);
     d2h(ctx->stream, &all, dall.p, 4);
     stream_sync(ctx->stream);
     *ok = (int)all;

@@ -237,6 +237,9 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
         stream_sync(ctx->stream);
     }
     ring->vk = make_verifier_key(ctx, N, d.omega, d.seed, d.suite_id, d.suite_id_len, srs->g1_0_be96, srs->g2_be192, ring->commit_be96, ring->vk_lines);
+    ring->vk_dev.alloc(1);
+    h2d(ctx->stream, ring->vk_dev.p, &ring->vk, sizeof(VerifierKeyDev));
+    stream_sync(ctx->stream);
     ring->suite.generator = d.generator;
     ring->suite.blinding_base = d.blinding_base;
     ring->suite.g_tab = d.g_tab;

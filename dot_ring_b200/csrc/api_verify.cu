@@ -24,8 +24,24 @@ struct PairingCheckBody {
 };
 
 
+std::shared_ptr<Ctx::G2Lines> Ctx::pairing_lines(const uint8_t* g2_be192, const G2Affine g2[2]) {
+    for (auto& l : g2_lines)
+        if (!memcmp(l->g2_be192, g2_be192, 384)) return l;
+    auto l = std::make_shared<G2Lines>();
+    memcpy(l->g2_be192, g2_be192, 384);
+    std::vector<LineCoeffs> host(2 * MILLER_LINES);
+    miller_precompute_lines(g2[0], host.data());
+    miller_precompute_lines(g2[1], host.data() + MILLER_LINES);
+    l->lines.alloc(host.size());
+    h2d(stream, l->lines.p, host.data(), host.size() * sizeof(LineCoeffs));
+    stream_sync(stream);
+    if (g2_lines.size() >= FIXED_TABLE_CAP) g2_lines.erase(g2_lines.begin());
+    g2_lines.push_back(l);
+    return l;
+}
+
 VerifierKeyDev make_verifier_key(Ctx* ctx, uint32_t N, const Fr& omega, const TEAffine& seed, const uint8_t* label, uint32_t label_len, const uint8_t* g1_0_be96,
-                                 const uint8_t* g2_be192, const uint8_t* fixed_be96, DevBuf<LineCoeffs>& lines) {
+                                 const uint8_t* g2_be192, const uint8_t* fixed_be96, std::shared_ptr<Ctx::G2Lines>& lines) {
     if (N < 8 || (N & (N - 1))) throw Error(DR_EINVAL, "domain_size must be a power of two");
     VerifierKeyDev vk{};
     vk.N = N;
@@ -52,15 +68,8 @@ VerifierKeyDev make_verifier_key(Ctx* ctx, uint32_t N, const Fr& omega, const TE
     for (int i = 0; i < 2; i++)
         if (!g2_decode_uncompressed(vk.g2[i], g2_be192 + 192 * i)) throw Error(DR_EINVAL, "invalid BLS12-381 G2 encoding in verifier key");
     vk.pc = ctx->pairing_consts();
-    {  // Miller-loop lines of the two fixed G2 points (pairing_warp.cuh), once per verifier key
-        std::vector<LineCoeffs> host(2 * MILLER_LINES);
-        miller_precompute_lines(vk.g2[0], host.data());
-        miller_precompute_lines(vk.g2[1], host.data() + MILLER_LINES);
-        lines.alloc(host.size());
-        h2d(ctx->stream, lines.p, host.data(), host.size() * sizeof(LineCoeffs));
-        stream_sync(ctx->stream);
-        vk.lines = lines.p;
-    }
+    lines = ctx->pairing_lines(g2_be192, vk.g2);  // once per context and G2 pair
+    vk.lines = lines->lines.p;
     // transcript prefix (root.py:54-71, phases.py:72-74): label | "vk" | G1[0] | G2[0..1] | 3 fixed commitments
     Shake128 tr;
     tr.init();
@@ -149,8 +158,17 @@ static void status_to_verdict(const std::vector<uint32_t>& st, uint8_t* verdict)
 // latency floor of a few ms, below this size the per-proof scalar multiplications are faster); tests lower it
 static std::atomic<size_t> RING_VERIFY_MSM_THRESHOLD{8192};  // process-wide test knob; read once per call
 
-// shared tail of the two ring-verification entry points; relations / payloads already on the device
-static void ring_proof_verify_device(Ctx* ctx, const VerifierKeyDev& vk, size_t n, const uint8_t* payloads, uint32_t stride, const TEAffine* relations, uint32_t rel_stride,
+// The verifier keys of one verification call: a device table of nkeys keys and, per item, the index of its key.
+struct VerifyKeys {
+    const VerifierKeyDev* table = nullptr;  // device
+    uint32_t nkeys = 1;
+    const uint32_t* index = nullptr;       // device, one entry per item; nullptr: every item uses table[0]
+    const uint32_t* host_index = nullptr;  // the same on the host (grouping of the two-MSM route)
+    const LineCoeffs* lines = nullptr;     // Miller-loop lines of the G2 points every key shares (aggregated check)
+};
+
+// shared tail of the ring-verification entry points; relations / payloads already on the device
+static void ring_proof_verify_device(Ctx* ctx, const VerifyKeys& keys, size_t n, const uint8_t* payloads, uint32_t stride, const TEAffine* relations, uint32_t rel_stride,
                                      const uint8_t* coeffs_le32, const uint32_t* extra_status, int aggregate, uint8_t* verdict, int* all_ok, bool extra_on_side = false) {
     // extra_on_side: extra_status is being written by work on ctx->side (forked by the caller); joined before its first reader
     struct SideJoin {  // an exception below must not leave the side stream running into freed buffers
@@ -183,32 +201,47 @@ static void ring_proof_verify_device(Ctx* ctx, const VerifierKeyDev& vk, size_t 
     } side2_join{ctx, true};
     ctx->fork_side2();
     launch(ctx->side2, Dim3((7 * m + 63) / 64), 64, 0, PayloadG1SubgroupBody(), m, vs.p);
-    launch(ctx->stream, Dim3((m + 63) / 64), 64, 0, RingVerifyAlgebraBody(), vk, payloads, stride, relations, rel_stride, (const uint8_t*)dco.p, m, vs.p);
+    launch(ctx->stream, Dim3((m + 63) / 64), 64, 0, RingVerifyAlgebraBody(), keys.table, keys.index, payloads, stride, relations, rel_stride, (const uint8_t*)dco.p, m, vs.p);
     ctx->join_side2();
     side2_join.pending = false;
     uint32_t all = 0;
     const bool by_msm = aggregate && n >= RING_VERIFY_MSM_THRESHOLD.load();
-    if (!by_msm) launch(ctx->stream, Dim3((2 * VERIFY_TERMS * m + 63) / 64), 64, 0, RingVerifyTermsBody(), vk, m, vs.p);
+    if (!by_msm) launch(ctx->stream, Dim3((2 * VERIFY_TERMS * m + 63) / 64), 64, 0, RingVerifyTermsBody(), keys.table, keys.index, m, vs.p);
     if (side_join.pending) {
         ctx->join_side();
         side_join.pending = false;
     }
     if (by_msm) {
-        // two variable-base MSMs instead of 13 scalar multiplications per proof
-        const uint32_t threads = 64, nparts = (m + threads - 1) / threads;
-        DevBuf<G1Affine> lhs_pts(7 * n + 4), rhs_pts(2 * n), sides(2);
-        DevBuf<uint8_t> lhs_sc(32 * (7 * n + 4)), rhs_sc(32 * 2 * n);
-        DevBuf<Fr> fixed_partial(4 * (size_t)nparts);
+        // two variable-base MSMs instead of 13 scalar multiplications per proof; the fixed commitments enter once per key, with
+        // the scalars of that key's proofs summed (proofs grouped by key: grouped[start[k] .. start[k + 1]))
+        const uint32_t threads = 64, nparts = (m + threads - 1) / threads, K = keys.nkeys;
+        const size_t n_lhs = 7 * n + 3 * (size_t)K + 1;
+        DevBuf<G1Affine> lhs_pts(n_lhs), rhs_pts(2 * n), sides(2);
+        DevBuf<uint8_t> lhs_sc(32 * n_lhs), rhs_sc(32 * 2 * n);
+        DevBuf<Fr> fixed_sc(3 * n), one_partial(nparts);
         DevBuf<G1> partial(2);
-        DevBuf<uint32_t> bad(1);
+        DevBuf<uint32_t> bad(1), dstart, dgrouped;
+        if (keys.index) {
+            std::vector<uint32_t> start(K + 1, 0), grouped(n);
+            for (size_t i = 0; i < n; i++) start[keys.host_index[i] + 1]++;
+            for (uint32_t k = 0; k < K; k++) start[k + 1] += start[k];
+            std::vector<uint32_t> fill(start.begin(), start.end() - 1);
+            for (size_t i = 0; i < n; i++) grouped[fill[keys.host_index[i]]++] = (uint32_t)i;
+            dstart.alloc(K + 1);
+            dgrouped.alloc(n);
+            h2d(ctx->stream, dstart.p, start.data(), (K + 1) * sizeof(uint32_t));
+            h2d(ctx->stream, dgrouped.p, grouped.data(), n * sizeof(uint32_t));
+            stream_sync(ctx->stream);  // start / grouped go out of scope
+        }
         dev_zero(ctx->stream, bad.p, 4);
-        launch(ctx->stream, Dim3(nparts), threads, 4 * threads * sizeof(Fr), RingVerifyGatherBody(), m, (const VerifyState*)vs.p, extra_status, dverdict.p, lhs_pts.p, lhs_sc.p,
-               rhs_pts.p, rhs_sc.p, fixed_partial.p, bad.p);
-        launch(ctx->stream, Dim3(1), 32, 0, RingVerifyFixedBody(), vk, m, (const Fr*)fixed_partial.p, nparts, lhs_pts.p, lhs_sc.p);
-        msm_points_device(ctx, lhs_pts.p, lhs_sc.p, 7 * n + 4, sides.p);
+        launch(ctx->stream, Dim3(nparts), threads, threads * sizeof(Fr), RingVerifyGatherBody(), m, (const VerifyState*)vs.p, extra_status, dverdict.p, lhs_pts.p, lhs_sc.p,
+               rhs_pts.p, rhs_sc.p, fixed_sc.p, one_partial.p, bad.p);
+        launch(ctx->stream, Dim3(K), threads, 3 * threads * sizeof(Fr), RingVerifyFixedBody(), keys.table, K, (const uint32_t*)dstart.p, (const uint32_t*)dgrouped.p, m,
+               (const Fr*)fixed_sc.p, (const Fr*)one_partial.p, nparts, lhs_pts.p, lhs_sc.p);
+        msm_points_device(ctx, lhs_pts.p, lhs_sc.p, n_lhs, sides.p);
         msm_points_device(ctx, rhs_pts.p, rhs_sc.p, 2 * n, sides.p + 1);
         launch(ctx->stream, Dim3(1), 32, 0, RingVerifySidesFromAffineBody(), (const G1Affine*)sides.p, partial.p);
-        launch(ctx->stream, Dim3(1), 32, ring_verify_warp_smem(), RingVerifyAggregateBody(), vk, (const G1*)partial.p, 1u, (const uint32_t*)bad.p, dall.p);
+        launch(ctx->stream, Dim3(1), 32, ring_verify_warp_smem(), RingVerifyAggregateBody(), keys.lines, ctx->pairing_consts(), (const G1*)partial.p, 1u, (const uint32_t*)bad.p, dall.p);
         d2h(ctx->stream, &all, dall.p, 4);
         d2h(ctx->stream, verdict, dverdict.p, n);
         stream_sync(ctx->stream);
@@ -220,7 +253,7 @@ static void ring_proof_verify_device(Ctx* ctx, const VerifierKeyDev& vk, size_t 
         DevBuf<uint32_t> bad(1);
         dev_zero(ctx->stream, bad.p, 4);
         launch(ctx->stream, Dim3(nparts), threads, 2 * threads * sizeof(G1), RingVerifyPartialSumBody(), m, (const VerifyState*)vs.p, extra_status, dverdict.p, partial.p, bad.p);
-        launch(ctx->stream, Dim3(1), 32, ring_verify_warp_smem(), RingVerifyAggregateBody(), vk, (const G1*)partial.p, nparts, (const uint32_t*)bad.p, dall.p);
+        launch(ctx->stream, Dim3(1), 32, ring_verify_warp_smem(), RingVerifyAggregateBody(), keys.lines, ctx->pairing_consts(), (const G1*)partial.p, nparts, (const uint32_t*)bad.p, dall.p);
         d2h(ctx->stream, &all, dall.p, 4);
         d2h(ctx->stream, verdict, dverdict.p, n);
         stream_sync(ctx->stream);  // partial / bad go out of scope
@@ -228,7 +261,8 @@ static void ring_proof_verify_device(Ctx* ctx, const VerifierKeyDev& vk, size_t 
 #ifndef DR_PAIRING_MINB
 #define DR_PAIRING_MINB 8
 #endif
-        launch_lb<32, DR_PAIRING_MINB>(ctx->stream, Dim3(m), 32, ring_verify_warp_smem(), RingVerifyFinishBody(), vk, m, (const VerifyState*)vs.p, extra_status, dverdict.p);
+        launch_lb<32, DR_PAIRING_MINB>(ctx->stream, Dim3(m), 32, ring_verify_warp_smem(), RingVerifyFinishBody(), keys.table, keys.index, m, (const VerifyState*)vs.p,
+                                       extra_status, dverdict.p);
     }
     d2h(ctx->stream, verdict, dverdict.p, n);
     stream_sync(ctx->stream);
@@ -238,6 +272,43 @@ static void ring_proof_verify_device(Ctx* ctx, const VerifierKeyDev& vk, size_t 
             if (verdict[i] != 1) all = 0;
     }
     if (all_ok) *all_ok = (int)all;
+}
+
+// RingVRF.decode + verify / batch_verify (vrf/ring/vrf.py:60-93,226-283) of n 784-byte proofs: the Pedersen part, then the ring proof
+// with the relation Ybar under the item's verifier key
+static void ring_vrf_verify(Ctx* ctx, const SuiteDev& suite, const VerifyKeys& keys, size_t n, const uint8_t* blob, const uint32_t* in_off, const uint32_t* in_len,
+                            const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* proofs784, const uint8_t* coeffs_le32, int aggregate, uint8_t* verdict,
+                            int* all_ok) {
+    ItemsDev items;
+    upload_items(ctx, items, n, blob, in_off, in_len, ad_off, ad_len);
+    const uint32_t m = (uint32_t)n;
+    DevBuf<uint8_t> dpr(n * 784), dok(4 * n);
+    DevBuf<TEAffine> pts(4 * n);
+    DevBuf<uint32_t> dst(n);
+    h2d(ctx->stream, dpr.p, proofs784, n * 784);
+    launch(ctx->stream, Dim3((4 * m + 63) / 64), 64, 0, TeDecodeManyBody(), (const uint8_t*)dpr.p, 784u, 4u, 4 * m, pts.p, dok.p);
+    // The Pedersen equations only meet the ring proof at the verdict, so they run on the side stream next to the payload decode, the
+    // transcript algebra and the G1 terms (a single verification is a chain of latency-bound kernels: this takes the longest one
+    // off the critical path; large batches lose nothing).
+    ctx->fork_side();
+    launch_pedersen_verify(ctx, ctx->side, suite, (const VerifyInput*)items.in.p, (const uint8_t*)items.blob.p, (const uint8_t*)dpr.p, 784u, (const TEAffine*)pts.p,
+                           (const uint8_t*)dok.p, m, dst.p);
+    // relation = blinded public key (second Pedersen point); payload follows the 192-byte Pedersen part
+    ring_proof_verify_device(ctx, keys, n, dpr.p + 192, 784, pts.p + 1, 4, coeffs_le32, dst.p, aggregate, verdict, all_ok, true);
+}
+
+// dr_ring_verifier: the verifier key of one ring, built from its 144-byte root, and the suite of its Pedersen part
+struct RingVerifier {
+    Ctx* ctx = nullptr;
+    VerifierKeyDev vk{};
+    std::shared_ptr<Ctx::G2Lines> lines;
+    SuiteDev suite{};
+    uint8_t g1_0_be96[96];
+};
+
+static bool same_suite(const SuiteDev& a, const SuiteDev& b) {
+    return a.suite_id_len == b.suite_id_len && !memcmp(a.suite_id, b.suite_id, a.suite_id_len) && a.dst_len == b.dst_len && !memcmp(a.dst, b.dst, a.dst_len) &&
+           a.hash_kind == b.hash_kind && a.generator == b.generator && a.blinding_base == b.blinding_base;
 }
 
 }  // namespace dr
@@ -429,16 +500,21 @@ int dr_ring_proof_verify_batch(dr_ctx* c, const dr_verifier_key* key, size_t n, 
     ctx->activate();
     if (all_ok) *all_ok = 1;
     if (!n) return DR_OK;
-    DevBuf<LineCoeffs> lines;
+    std::shared_ptr<Ctx::G2Lines> lines;
     VerifierKeyDev vk = make_verifier_key(ctx, key->domain_size, fr_param(key->omega), te_param(key->seed), key->label, key->label_len, key->g1_0_be96, key->g2_be192,
                                           key->fixed_be96, lines);
+    DevBuf<VerifierKeyDev> dvk(1);
+    h2d(ctx->stream, dvk.p, &vk, sizeof(VerifierKeyDev));
+    VerifyKeys keys;
+    keys.table = dvk.p;
+    keys.lines = vk.lines;
     std::vector<TEAffine> rel(n);
     for (size_t i = 0; i < n; i++) rel[i] = {fr_param(relations_xy64 + 64 * i), fr_param(relations_xy64 + 64 * i + 32)};
     DevBuf<TEAffine> drel(n);
     DevBuf<uint8_t> dpl(n * 592);
     h2d(ctx->stream, drel.p, rel.data(), n * sizeof(TEAffine));
     h2d(ctx->stream, dpl.p, payloads592, n * 592);
-    ring_proof_verify_device(ctx, vk, n, dpl.p, 592, drel.p, 1, coeffs_le32, nullptr, aggregate, verdict, all_ok);
+    ring_proof_verify_device(ctx, keys, n, dpl.p, 592, drel.p, 1, coeffs_le32, nullptr, aggregate, verdict, all_ok);
     DR_API_END
 }
 
@@ -451,22 +527,81 @@ int dr_ring_verify_batch(dr_ctx* c, dr_ring* r, size_t n, const uint8_t* blob, c
     ctx->activate();
     if (all_ok) *all_ok = 1;
     if (!n) return DR_OK;
-    ItemsDev items;
-    upload_items(ctx, items, n, blob, in_off, in_len, ad_off, ad_len);
-    const uint32_t m = (uint32_t)n;
-    DevBuf<uint8_t> dpr(n * 784), dok(4 * n);
-    DevBuf<TEAffine> pts(4 * n);
-    DevBuf<uint32_t> dst(n);
-    h2d(ctx->stream, dpr.p, proofs784, n * 784);
-    launch(ctx->stream, Dim3((4 * m + 63) / 64), 64, 0, TeDecodeManyBody(), (const uint8_t*)dpr.p, 784u, 4u, 4 * m, pts.p, dok.p);
-    // The Pedersen equations only meet the ring proof at the verdict, so they run on the side stream next to the payload decode, the
-    // transcript algebra and the G1 terms (a single verification is a chain of latency-bound kernels: this takes the longest one
-    // off the critical path; large batches lose nothing).
-    ctx->fork_side();
-    launch_pedersen_verify(ctx, ctx->side, ring->suite, (const VerifyInput*)items.in.p, (const uint8_t*)items.blob.p, (const uint8_t*)dpr.p, 784u, (const TEAffine*)pts.p,
-                           (const uint8_t*)dok.p, m, dst.p);
-    // relation = blinded public key (second Pedersen point); payload follows the 192-byte Pedersen part
-    ring_proof_verify_device(ctx, ring->vk, n, dpr.p + 192, 784, pts.p + 1, 4, coeffs_le32, dst.p, aggregate, verdict, all_ok, true);
+    VerifyKeys keys;
+    keys.table = ring->vk_dev.p;
+    keys.lines = ring->vk.lines;
+    ring_vrf_verify(ctx, ring->suite, keys, n, blob, in_off, in_len, ad_off, ad_len, proofs784, coeffs_le32, aggregate, verdict, all_ok);
+    DR_API_END
+}
+
+int dr_ring_verifier_create(dr_ctx* c, const dr_ring_params* prm, const uint8_t* g1_0_be96, const uint8_t* g2_be192, const uint8_t root144[144], dr_ring_verifier** out) {
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || !prm || !g1_0_be96 || !g2_be192 || !root144 || !out) throw Error(DR_EINVAL, "bad argument");
+    const uint32_t N = prm->domain_size;
+    if (N < 512 || N > 65536 || (N & (N - 1))) throw Error(DR_EINVAL, "domain_size must be a power of two in [512, 65536]");
+    if (prm->suite_id_len > 32 || prm->h2c_dst_len > 64) throw Error(DR_EINVAL, "suite id / DST too long");
+    if (prm->hash_id > 1) throw Error(DR_EINVAL, "unknown suite hash");
+    ctx->activate();
+    auto v = std::make_unique<RingVerifier>();
+    v->ctx = ctx;
+    // RingRoot.decode (root.py:89-109): three compressed points, no subgroup check (blst); the transcript absorbs their
+    // uncompressed encodings
+    uint8_t fixed_be96[288];
+    for (int i = 0; i < 3; i++) {
+        G1Affine a;
+        if (!g1_decode(a, root144 + 48 * i, 48)) throw Error(DR_EINVAL, "invalid BLS12-381 G1 encoding in ring root");
+        g1_serialize(fixed_be96 + 96 * i, a);
+    }
+    v->vk = make_verifier_key(ctx, N, fr_param(prm->omega), te_param(prm->seed), prm->suite_id, prm->suite_id_len, g1_0_be96, g2_be192, fixed_be96, v->lines);
+    for (int i = 0; i < 3; i++) v->vk.fixed_outside[i] = g1_in_subgroup(v->vk.fixed[i]) ? 0 : 1;
+    v->suite.generator = te_param(prm->generator);
+    v->suite.blinding_base = te_param(prm->blinding_base);
+    v->suite.suite_id_len = prm->suite_id_len;
+    memcpy(v->suite.suite_id, prm->suite_id, 32);
+    v->suite.dst_len = prm->h2c_dst_len;
+    memcpy(v->suite.dst, prm->h2c_dst, 64);
+    v->suite.hash_kind = prm->hash_id;
+    memcpy(v->g1_0_be96, g1_0_be96, 96);
+    *out = (dr_ring_verifier*)v.release();
+    DR_API_END
+}
+
+void dr_ring_verifier_destroy(dr_ring_verifier* v) { delete (RingVerifier*)v; }
+
+int dr_ring_verify_multi(dr_ctx* c, dr_ring_verifier* const* verifiers, size_t n_verifiers, const uint32_t* verifier_index, size_t n, const uint8_t* blob,
+                         const uint32_t* in_off, const uint32_t* in_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* proofs784, const uint8_t* coeffs_le32,
+                         int aggregate, uint8_t* verdict, int* all_ok) {
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || !verifiers || !n_verifiers || n_verifiers > UINT32_MAX || (n && (!verifier_index || !proofs784 || !verdict))) throw Error(DR_EINVAL, "bad argument");
+    const RingVerifier* first = (const RingVerifier*)verifiers[0];
+    for (size_t k = 0; k < n_verifiers; k++) {
+        const RingVerifier* v = (const RingVerifier*)verifiers[k];
+        if (!v) throw Error(DR_EINVAL, "bad argument");
+        if (v->ctx != ctx) throw Error(DR_EINVAL, "ring verifier belongs to another context");
+        if (!same_suite(v->suite, first->suite)) throw Error(DR_EINVAL, "ring verifiers of one call must share the suite");
+        if (memcmp(v->g1_0_be96, first->g1_0_be96, 96) || memcmp(v->lines->g2_be192, first->lines->g2_be192, 384))
+            throw Error(DR_EINVAL, "ring verifiers of one call must share [1]_1 and the G2 points");
+    }
+    for (size_t i = 0; i < n; i++)
+        if (verifier_index[i] >= n_verifiers) throw Error(DR_EINVAL, "verifier index out of range");
+    ctx->activate();
+    if (all_ok) *all_ok = 1;
+    if (!n) return DR_OK;
+    std::vector<VerifierKeyDev> table(n_verifiers);
+    for (size_t k = 0; k < n_verifiers; k++) table[k] = ((const RingVerifier*)verifiers[k])->vk;
+    DevBuf<VerifierKeyDev> dtable(n_verifiers);
+    DevBuf<uint32_t> dindex(n);
+    h2d(ctx->stream, dtable.p, table.data(), n_verifiers * sizeof(VerifierKeyDev));
+    h2d(ctx->stream, dindex.p, verifier_index, n * sizeof(uint32_t));
+    VerifyKeys keys;
+    keys.table = dtable.p;
+    keys.nkeys = (uint32_t)n_verifiers;
+    keys.index = dindex.p;
+    keys.host_index = verifier_index;
+    keys.lines = first->vk.lines;
+    ring_vrf_verify(ctx, first->suite, keys, n, blob, in_off, in_len, ad_off, ad_len, proofs784, coeffs_le32, aggregate, verdict, all_ok);
     DR_API_END
 }
 

@@ -525,24 +525,32 @@ struct IetfProveBody {  // thin == 0: O | c | s (80 bytes);  thin != 0: O | R | 
 };
 
 // ---- ring-proof verifier ------------------------------------------------------------------------------------
+// The kernels below read every ring-dependent constant from a device table of verifier keys, item p using
+// vks[vk_index[p]] (vk_index == nullptr: every item uses vks[0]), so one launch verifies proofs of rings over different
+// domains.  All keys of one launch share [1]_1 and the G2 points, hence the Miller-loop lines and the final pairing.
 struct VerifierKeyDev {
     uint32_t N, logN;
     Fr omega, w_last, n_inv;
     Fr tail[4];         // coefficients of (X - w^(N-1))(X - w^(N-2))(X - w^(N-3))
     TEAffine seed;      // accumulator base
     G1Affine fixed[4];  // C_px, C_py, C_s, [1]_1
+    uint8_t fixed_outside[3];  // fixed[j] decoded but not in G1 (g1_in_subgroup): its term takes a full-scalar multiplication
     G2Affine g2[2];     // [1]_2, [tau]_2
     PairingConsts pc;
     const LineCoeffs* lines;  // [2][MILLER_LINES] precomputed Miller-loop lines of g2[0], g2[1] (device memory)
     Shake128 prefix;    // transcript after absorbing the verifier key (root.py:54-71)
 };
 
+DR_HD const VerifierKeyDev& item_key(const VerifierKeyDev* vks, const uint32_t* vk_index, uint32_t p) { return vks[vk_index ? vk_index[p] : 0]; }
+
 constexpr int VERIFY_TERMS = 13;  // scalar multiplications per proof (see RingVerifyAlgebraBody)
 
 struct VerifyState {
     uint32_t status;
     G1Affine g1[7];      // C_b, C_accip, C_accx, C_accy, C_q, Phi_zeta, Phi_zeta_omega
-    uint8_t outside[7];  // g1[j] decoded but not in G1 (g1_in_subgroup): its terms take a full-scalar multiplication
+    // the bases of the 13 terms (RingVerifyTermsBody: g1[0..6], then C_px, C_py, C_s, [1]_1 of the item's key) that are not in G1
+    // (g1_in_subgroup): their terms take a full-scalar multiplication.  [0..6] PayloadG1SubgroupBody, [7..9] RingVerifyAlgebraBody
+    uint8_t outside[11];
     Fr sc[VERIFY_TERMS];
     G1 term[2 * VERIFY_TERMS];  // sc[j] * base_j as two GLV halves: term[2j] = k1 * P, term[2j + 1] = k2 * phi(P)
 };
@@ -583,12 +591,14 @@ struct PayloadG1SubgroupBody {
 //   lhs = sum_j sc[j]*g1[j] (j<7) + sc[9]*C_px + sc[10]*C_py + sc[11]*C_s + sc[12]*[1]_1,  rhs = sc[7]*Phi_zeta + sc[8]*Phi_zeta_omega
 //   accept  <=>  e(lhs, [1]_2) == e(rhs, [tau]_2)
 struct RingVerifyAlgebraBody {
-    DR_HD void operator()(const BlockCtx& ctx, VerifierKeyDev vk, const uint8_t* payloads, uint32_t stride, const TEAffine* relations, uint32_t rel_stride,
-                          const uint8_t* coeffs_le32, uint32_t count, VerifyState* vs) const {
+    DR_HD void operator()(const BlockCtx& ctx, const VerifierKeyDev* vks, const uint32_t* vk_index, const uint8_t* payloads, uint32_t stride, const TEAffine* relations,
+                          uint32_t rel_stride, const uint8_t* coeffs_le32, uint32_t count, VerifyState* vs) const {
         DR_THREAD_LOOP(t, ctx) {
             uint32_t p = ctx.bx * ctx.nthreads + t;
             if (p < count) {
                 VerifyState& s = vs[p];
+                const VerifierKeyDev& vk = item_key(vks, vk_index, p);
+                for (int j = 0; j < 3; j++) s.outside[7 + j] = vk.fixed_outside[j];
                 const uint8_t* pl = payloads + (size_t)stride * p;
                 // evaluations px, py, s, b, accip, accx, accy at zeta and L(zeta w): canonical scalars only
                 Fr ev[8];
@@ -737,22 +747,23 @@ DR_HD_COLD G1 g1_mul_raw(const G1Affine& p, const uint32_t* k, int nlimbs) {
 }
 
 // one thread per (proof, term, GLV half): sc * P = k1 * P + k2 * phi(P) with 128-bit k1, k2 (msm.cuh glv_half), phi(x, y) = (beta x, y):
-// half the doublings of a 255-bit multiplication, on twice the threads.  A decoded point outside G1 takes sc * P whole on the first
-// half's thread (the split is exact only on G1; g1_mul_raw's affine table assumes no multiple 2P .. 15P is infinity, which a
-// small-order component breaks); the fixed points are commitments over the SRS, in G1.
+// half the doublings of a 255-bit multiplication, on twice the threads.  A point outside G1 takes sc * P whole on the first half's
+// thread (the split is exact only on G1; g1_mul_raw's affine table assumes no multiple 2P .. 15P is infinity, which a small-order
+// component breaks).  That covers the decoded payload points and the fixed commitments of a key built from a caller's ring root
+// (dr_ring_verifier_create tests them once); keys built from a ring or a dr_verifier_key treat their fixed commitments as in G1.
 struct RingVerifyTermsBody {
-    DR_HD void operator()(const BlockCtx& ctx, VerifierKeyDev vk, uint32_t count, VerifyState* vs) const {
+    DR_HD void operator()(const BlockCtx& ctx, const VerifierKeyDev* vks, const uint32_t* vk_index, uint32_t count, VerifyState* vs) const {
         DR_THREAD_LOOP(t, ctx) {
             uint32_t i = ctx.bx * ctx.nthreads + t;
             if (i < 2 * VERIFY_TERMS * count) {
                 uint32_t p = i / (2 * VERIFY_TERMS), r = i % (2 * VERIFY_TERMS), j = r >> 1, h = r & 1;
                 VerifyState& s = vs[p];
-                const uint32_t src = j < 7 ? j : j - 2;  // index into s.g1 for j < 9
-                G1Affine base = j < 9 ? s.g1[src] : vk.fixed[j - 9];
+                const uint32_t src = j < 7 ? j : j - 2;  // index into s.g1 for j < 9, into s.outside for every j
+                G1Affine base = j < 9 ? s.g1[src] : item_key(vks, vk_index, p).fixed[j - 9];
                 G1 out = G1::inf();
                 if (!(s.status & ST_MALFORMED) && !base.is_inf()) {
                     Fr k = s.sc[j].from_mont();
-                    if (j < 9 && s.outside[src]) {
+                    if (s.outside[src]) {
                         if (!h) out = g1_mul_limbs(G1::from_affine(base), k.v);  // XYZZ table: multiples of a small-order point may be infinity
                     } else {
                         uint32_t half[8];
@@ -779,7 +790,8 @@ DR_HD void ring_verify_sides(const VerifyState& s, G1& lhs, G1& rhs) {
 // extra_status: Pedersen status per proof (or null).
 DR_HD size_t ring_verify_warp_smem() { return sizeof(PairingWarpState) + 2 * sizeof(G1) + 16; }
 struct RingVerifyFinishBody {
-    DR_HD void operator()(const BlockCtx& ctx, VerifierKeyDev vk, uint32_t count, const VerifyState* vs, const uint32_t* extra_status, uint8_t* verdict) const {
+    DR_HD void operator()(const BlockCtx& ctx, const VerifierKeyDev* vks, const uint32_t* vk_index, uint32_t count, const VerifyState* vs, const uint32_t* extra_status,
+                          uint8_t* verdict) const {
         PairingWarpState* st = (PairingWarpState*)ctx.smem;
         G1* P = (G1*)(ctx.smem + ((sizeof(PairingWarpState) + 15) / 16) * 16);
         const uint32_t p = ctx.bx;
@@ -802,6 +814,7 @@ struct RingVerifyFinishBody {
             }
         }
         DR_BLOCK_SYNC();
+        const VerifierKeyDev& vk = item_key(vks, vk_index, p);
         pairing_product_is_one_warp(ctx, st, P, vk.lines, vk.pc);
         DR_THREAD_LOOP(t, ctx) {
             if (t == 0) verdict[p] = st->verdict ? 1 : 0;
@@ -856,15 +869,16 @@ struct RingVerifyPartialSumBody {
     }
 };
 // Large aggregated batches: instead of 13 scalar multiplications per proof (RingVerifyTermsBody), the two sides become two
-// variable-base MSMs (pippenger.cuh): lhs over 7 points per proof + the 4 fixed points, rhs over 2 points per proof.
-// This kernel lays out the operands: points, canonical little-endian scalars, and per-block sums of the fixed scalars.
+// variable-base MSMs (pippenger.cuh): lhs over 7 points per proof, the 3 fixed commitments of every key and [1]_1, rhs over 2 points
+// per proof.  This kernel lays out the per-proof operands (points, canonical little-endian scalars), each proof's three
+// fixed-commitment scalars, and per-block sums of the [1]_1 scalars.
 struct RingVerifyGatherBody {
     DR_HD void operator()(const BlockCtx& ctx, uint32_t count, const VerifyState* vs, const uint32_t* extra_status, uint8_t* verdict, G1Affine* lhs_pts, uint8_t* lhs_sc,
-                          G1Affine* rhs_pts, uint8_t* rhs_sc, Fr* fixed_partial, uint32_t* any_bad) const {
-        Fr* sm = (Fr*)ctx.smem;  // 4 * nthreads
+                          G1Affine* rhs_pts, uint8_t* rhs_sc, Fr* fixed_sc, Fr* one_partial, uint32_t* any_bad) const {
+        Fr* sm = (Fr*)ctx.smem;  // nthreads
         DR_THREAD_LOOP(t, ctx) {
             uint32_t p = ctx.bx * ctx.nthreads + t;
-            Fr f[4] = {Fr::zero(), Fr::zero(), Fr::zero(), Fr::zero()};
+            Fr one = Fr::zero();
             if (p < count) {
                 const VerifyState& s = vs[p];
                 uint32_t st = s.status | (extra_status ? extra_status[p] : 0u);
@@ -878,32 +892,56 @@ struct RingVerifyGatherBody {
                     rhs_pts[2 * (size_t)p + j] = st ? G1Affine::inf() : s.g1[5 + j];
                     fr_to_le_bytes_raw(rhs_sc + 32 * (2 * (size_t)p + j), st ? Fr::zero() : s.sc[7 + j].from_mont());
                 }
-                if (!st)
-                    for (int j = 0; j < 4; j++) f[j] = s.sc[9 + j];
+                for (int j = 0; j < 3; j++) fixed_sc[3 * (size_t)p + j] = st ? Fr::zero() : s.sc[9 + j];
+                if (!st) one = s.sc[12];
             }
-            for (int j = 0; j < 4; j++) sm[j * ctx.nthreads + t] = f[j];
+            sm[t] = one;
+        }
+        DR_BLOCK_SYNC();
+        for (uint32_t stride = ctx.nthreads >> 1; stride > 0; stride >>= 1) {
+            DR_STRIDE_LOOP(t, stride, ctx) { sm[t] = sm[t] + sm[t + stride]; }
+            DR_BLOCK_SYNC();
+        }
+        DR_THREAD_LOOP(t, ctx) {
+            if (t == 0) one_partial[ctx.bx] = sm[0];
+        }
+    }
+};
+// One block per key k: appends C_px, C_py, C_s of key k with the sums of the scalars of its proofs at lhs entry 7 * count + 3k + j;
+// block 0 also appends [1]_1 with the sum of the per-block partials at entry 7 * count + 3 * nkeys.  The proofs of key k are
+// items[start[k] .. start[k + 1]) (start == nullptr: one key, every proof).
+struct RingVerifyFixedBody {
+    DR_HD void operator()(const BlockCtx& ctx, const VerifierKeyDev* vks, uint32_t nkeys, const uint32_t* start, const uint32_t* items, uint32_t count, const Fr* fixed_sc,
+                          const Fr* one_partial, uint32_t nparts, G1Affine* lhs_pts, uint8_t* lhs_sc) const {
+        Fr* sm = (Fr*)ctx.smem;  // 3 * nthreads
+        const uint32_t k = ctx.bx;
+        const uint32_t lo = start ? start[k] : 0, hi = start ? start[k + 1] : count;
+        DR_THREAD_LOOP(t, ctx) {
+            Fr f[3] = {Fr::zero(), Fr::zero(), Fr::zero()};
+#pragma unroll 1
+            for (uint32_t i = lo + t; i < hi; i += ctx.nthreads) {
+                const uint32_t p = items ? items[i] : i;
+                for (int j = 0; j < 3; j++) f[j] = f[j] + fixed_sc[3 * (size_t)p + j];
+            }
+            for (int j = 0; j < 3; j++) sm[j * ctx.nthreads + t] = f[j];
         }
         DR_BLOCK_SYNC();
         for (uint32_t stride = ctx.nthreads >> 1; stride > 0; stride >>= 1) {
             DR_STRIDE_LOOP(t, stride, ctx) {
-                for (int j = 0; j < 4; j++) sm[j * ctx.nthreads + t] = sm[j * ctx.nthreads + t] + sm[j * ctx.nthreads + t + stride];
+                for (int j = 0; j < 3; j++) sm[j * ctx.nthreads + t] = sm[j * ctx.nthreads + t] + sm[j * ctx.nthreads + t + stride];
             }
             DR_BLOCK_SYNC();
         }
         DR_THREAD_LOOP(t, ctx) {
-            if (t < 4) fixed_partial[4 * (size_t)ctx.bx + t] = sm[t * ctx.nthreads];
-        }
-    }
-};
-// appends the 4 fixed points with their summed scalars after the 7 * count per-proof entries
-struct RingVerifyFixedBody {
-    DR_HD void operator()(const BlockCtx& ctx, VerifierKeyDev vk, uint32_t count, const Fr* fixed_partial, uint32_t nparts, G1Affine* lhs_pts, uint8_t* lhs_sc) const {
-        DR_THREAD_LOOP(t, ctx) {
-            if (t < 4) {
+            if (t < 3) {
+                lhs_pts[7 * (size_t)count + 3 * k + t] = vks[k].fixed[t];
+                fr_to_le_bytes_raw(lhs_sc + 32 * (7 * (size_t)count + 3 * k + t), sm[t * ctx.nthreads].from_mont());
+            }
+            if (t == 3 && k == 0) {
                 Fr acc = Fr::zero();
-                for (uint32_t i = 0; i < nparts; i++) acc = acc + fixed_partial[4 * (size_t)i + t];
-                lhs_pts[7 * (size_t)count + t] = vk.fixed[t];
-                fr_to_le_bytes_raw(lhs_sc + 32 * (7 * (size_t)count + t), acc.from_mont());
+                for (uint32_t i = 0; i < nparts; i++) acc = acc + one_partial[i];
+                lhs_pts[7 * (size_t)count + 3 * nkeys] = vks[0].fixed[3];
+                fr_to_le_bytes_raw(lhs_sc + 32 * (7 * (size_t)count + 3 * nkeys), acc.from_mont());
             }
         }
     }
@@ -917,9 +955,9 @@ struct RingVerifySidesFromAffineBody {
     }
 };
 
-// stage 2: one block folds the partial pairs and runs the single pairing check
+// stage 2: one block folds the partial pairs and runs the single pairing check (lines: the Miller-loop lines shared by the batch's keys)
 struct RingVerifyAggregateBody {
-    DR_HD void operator()(const BlockCtx& ctx, VerifierKeyDev vk, const G1* partial, uint32_t nparts, const uint32_t* any_bad, uint32_t* all_ok) const {
+    DR_HD void operator()(const BlockCtx& ctx, const LineCoeffs* lines, PairingConsts pc, const G1* partial, uint32_t nparts, const uint32_t* any_bad, uint32_t* all_ok) const {
         PairingWarpState* st = (PairingWarpState*)ctx.smem;
         G1* P = (G1*)(ctx.smem + ((sizeof(PairingWarpState) + 15) / 16) * 16);
         DR_THREAD_LOOP(t, ctx) {
@@ -931,7 +969,7 @@ struct RingVerifyAggregateBody {
             }
         }
         DR_BLOCK_SYNC();
-        pairing_product_is_one_warp(ctx, st, P, vk.lines, vk.pc);
+        pairing_product_is_one_warp(ctx, st, P, lines, pc);
         DR_THREAD_LOOP(t, ctx) {
             if (t == 0) *all_ok = (!*any_bad && st->verdict) ? 1u : 0u;
         }

@@ -5,6 +5,9 @@ invalid keys -> padding point), builds the public vector ``PK || padding || 2^i*
 same device object, the three fixed columns (px, py, s): coefficients, KZG commitments (= the ring
 root) and their 4x low-degree extensions.  The reference recomputes the latter on every proof
 (constraints.py:43-62); here they live in HBM for the lifetime of the ring.
+
+``RingVerifier(roots)`` verifies Ring VRF proofs against ring roots alone: the verifier needs neither the keys nor the SRS
+window table, and one batch may span several rings (one aggregated pairing check for all of them).
 """
 
 from __future__ import annotations
@@ -186,4 +189,112 @@ class RingRoot:
         return RingRoot.from_ring(ring).encode() == self.encode()
 
 
-__all__ = ["Ring", "RingRoot", "Column", "point_to_string"]
+def _suite_key(params: RingProofParams):
+    p = params.cv.curve.params
+    return (p.suite_id, p.hash_to_curve.dst, p.hash_name, tuple(p.generator), tuple(p.auxiliary_points.blinding_base))
+
+
+def _native_verifier(engine: Engine, root: bytes, params: RingProofParams) -> _native.NativeRingVerifier:
+    p = params.cv.curve.params
+    srs = engine.srs_bytes  # [1]_1 and the G2 points only: the window table (`engine.srs`) is never built here
+    return _native.NativeRingVerifier(
+        engine.ctx, root, srs.g1_be96[:96], srs.g2_be192, domain_size=params.domain_size, omega=params.omega, seed=p.auxiliary_points.accumulator_base,
+        blinding_base=p.auxiliary_points.blinding_base, generator=p.generator, suite_id=p.suite_id, h2c_dst=p.hash_to_curve.dst, hash_name=p.hash_name,
+    )  # fmt: skip
+
+
+class RingVerifier:
+    """Ring VRF verification against ring roots alone (the verifier side of vrf/ring/vrf.py:226-283 without the ``Ring``).
+
+    ``roots`` are :class:`RingRoot` values (``RingRoot.decode(data, params)`` or ``RingRoot.from_ring(ring)``), each with its
+    ``params``; they must share the suite, their domain sizes may differ.  Item i of a batch is checked against
+    ``roots[rings[i]]`` (default: every item against ``roots[0]``).  ``batch_verify`` folds the whole batch, whatever the
+    ring of each item, into one pairing check.  With an :class:`EnginePool` every device holds one verifier per root and takes a
+    contiguous shard of the batch; the aggregated result is then the conjunction of the devices' checks."""
+
+    def __init__(self, roots: Sequence[RingRoot], engine: "Engine | EnginePool | None" = None) -> None:
+        roots = list(roots)
+        if not roots:
+            raise ValueError("RingVerifier needs at least one ring root")
+        if any(r.params is None for r in roots):
+            raise ValueError("every ring root must carry its ring proof parameters")
+        if len({_suite_key(r.params) for r in roots}) != 1:
+            raise ValueError("ring roots of one RingVerifier must share the suite")
+        self.roots = roots
+        self.params = roots[0].params
+        self.engine = engine or default_engine()
+        encoded = [r.encode() for r in roots]
+
+        def build(eng: Engine):
+            out = []
+            try:
+                for data, r in zip(encoded, roots):
+                    out.append(_native_verifier(eng, data, r.params))
+            except BaseException:
+                for v in out:
+                    v.close()
+                raise
+            return out
+
+        if isinstance(self.engine, EnginePool):
+            self.replicas = self.engine.map(lambda i: build(self.engine.engines[i]))
+        else:
+            self.replicas = [build(self.engine)]
+
+    def close(self) -> None:
+        for verifiers in self.replicas:
+            for v in verifiers:
+                v.close()
+        self.replicas = []
+
+    def _verify_common(self, proofs, inputs, additional_data, rings, aggregate: bool):
+        """-> (per-item verdicts, all_ok); coefficients drawn as in RingVRF._verify_common."""
+        from .kzg import _random_nonzero_coefficients
+
+        raw = [bytes(p) if isinstance(p, (bytes, bytearray)) else p.encode() for p in proofs]
+        n = len(raw)
+        if not (len(inputs) == len(additional_data) == n):
+            raise ValueError("proofs, inputs and additional_data must have the same length")
+        index = [0] * n if rings is None else [int(k) for k in rings]
+        if len(index) != n:
+            raise ValueError("rings must give one ring index per proof")
+        if any(not 0 <= k < len(self.roots) for k in index):
+            raise ValueError("ring index out of range")
+        if n == 0:
+            return [], True
+        order = self.params.prime
+        if aggregate:
+            coeffs = _random_nonzero_coefficients(2 * n, order)
+        else:  # independent checks: (1, r) per proof
+            coeffs = [v for r in _random_nonzero_coefficients(n + 1, order)[1:] for v in (1, r)]
+        inputs = [bytes(a) for a in inputs]
+        ads = [bytes(d) for d in additional_data]
+        bounds = EnginePool.shard_bounds(n, len(self.replicas))
+
+        def run(i):
+            lo, hi = bounds[i]
+            return _native.NativeRingVerifier.verify_multi(self.replicas[i], index[lo:hi], inputs[lo:hi], ads[lo:hi], raw[lo:hi], coeffs[2 * lo : 2 * hi], aggregate)
+
+        if len(bounds) <= 1:
+            return run(0)
+        parts = self.engine.map(run, range(len(bounds)))
+        return [v for verdicts, _ in parts for v in verdicts], all(ok for _, ok in parts)
+
+    def verify(self, proof, input: bytes, ad: bytes, ring: int = 0) -> bool:
+        """vrf/ring/vrf.py:226-232 against roots[ring]."""
+        return self._verify_common([proof], [input], [ad], [ring], False)[0][0] == 1
+
+    def verify_batch(self, proofs, inputs, additional_data, rings: Sequence[int] | None = None) -> list[int]:
+        """Independent verifications, item i against roots[rings[i]]: 1 valid, 0 invalid, 2 malformed encoding."""
+        return self._verify_common(proofs, inputs, additional_data, rings, False)[0]
+
+    def batch_verify(self, proofs, inputs, additional_data, rings: Sequence[int] | None = None) -> bool:
+        """vrf/ring/vrf.py:239-283 over a batch that may span all the roots: one pairing check (one per device of a pool);
+        any error -> False."""
+        try:
+            return self._verify_common(proofs, inputs, additional_data, rings, True)[1]
+        except (AssertionError, AttributeError, TypeError, ValueError):
+            return False
+
+
+__all__ = ["Ring", "RingRoot", "RingVerifier", "Column", "point_to_string"]

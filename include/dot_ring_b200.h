@@ -271,6 +271,27 @@ int dr_ring_proof_verify_batch(dr_ctx* ctx, const dr_verifier_key* key, size_t n
 int dr_ring_verify_batch(dr_ctx* ctx, dr_ring* ring, size_t n, const uint8_t* blob, const uint32_t* in_off, const uint32_t* in_len, const uint32_t* ad_off,
                          const uint32_t* ad_len, const uint8_t* proofs784, const uint8_t* coeffs_le32, int aggregate, uint8_t* verdict, int* all_ok);
 
+/* ---- ring verification from ring roots -------------------------------------------------------------------------
+ * A verifier needs nothing of a ring but its root (the fixed commitments): `Verify(...)` runs on them alone (verify.py:213-324), and
+ * RingRoot.matches_ring (root.py:111-112) is the only use the reference makes of the keys.  A dr_ring_verifier is the verifier key of
+ * one ring, built from its 144-byte root = compress(C_px) | compress(C_py) | compress(C_s) (root.py:74-87): no keys, no SRS handle,
+ * no window table.  params: domain_size, omega, seed, generator, blinding_base, suite_id, h2c_dst, hash_id are read (the rest of
+ * dr_ring_params is ignored); g1_0_be96 = [1]_1, g2_be192 = [1]_2 | [tau]_2 as in dr_srs_load.  DR_EINVAL where RingRoot.decode raises
+ * (any of the three encodings rejected as by dr_g1_decompress) or on bad params; domain_size as in dr_ring_create.  Decoding checks no
+ * subgroup (blst); a commitment on the curve but outside G1 is tested once here and then multiplied exactly.
+ * dr_ring_verify_multi is dr_ring_verify_batch for a batch whose item i is checked against verifiers[verifier_index[i]], with the same
+ * blob / offsets / proofs / coefficients / verdict / all_ok conventions; domain sizes may differ between the verifiers.
+ * aggregate != 0 folds ALL items, whatever their ring, into one pairing check (rings over one SRS share [1]_2 and [tau]_2).
+ * DR_EINVAL when a verifier belongs to another context, when the verifiers differ in suite (id, DST, hash, generator, blinding base),
+ * in [1]_1 or in the G2 points, or when an index is out of range. */
+typedef struct dr_ring_verifier dr_ring_verifier;
+int dr_ring_verifier_create(dr_ctx* ctx, const dr_ring_params* params, const uint8_t* g1_0_be96, const uint8_t* g2_be192, const uint8_t root144[144],
+                            dr_ring_verifier** out);
+void dr_ring_verifier_destroy(dr_ring_verifier* v);
+int dr_ring_verify_multi(dr_ctx* ctx, dr_ring_verifier* const* verifiers, size_t n_verifiers, const uint32_t* verifier_index, size_t n, const uint8_t* blob,
+                         const uint32_t* in_off, const uint32_t* in_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* proofs784,
+                         const uint8_t* coeffs_le32, int aggregate, uint8_t* verdict, int* all_ok);
+
 /* Aggregated batches of at least `n` proofs fold the two sides with two variable-base MSMs instead of 13 scalar multiplications
  * per proof (default 8192; same verdicts, tests lower it to exercise the path on small batches). */
 int dr_ring_verify_set_msm_threshold(size_t n);
