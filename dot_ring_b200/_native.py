@@ -95,6 +95,7 @@ class Library:
         L.dr_ring_fixed_commitments.argtypes = [c_void_p, c_void_p]
         L.dr_ring_points.argtypes = [c_void_p, c_void_p, c_size_t]
         L.dr_ring_prove_batch.argtypes = [c_void_p, c_void_p, c_size_t] + [c_void_p] * 10
+        L.dr_ring_prove_multi.argtypes = [c_void_p, c_void_p, c_size_t, c_void_p, c_size_t] + [c_void_p] * 10
         L.dr_ring_prove_phase_ms.argtypes = [c_void_p, POINTER(c_float * 6)]
         L.dr_ring_prove_commit_kernel_ms.argtypes = [c_void_p, POINTER(c_float), POINTER(c_uint32)]
         L.dr_ring_witness_table_bits.argtypes = [c_void_p]
@@ -666,14 +667,21 @@ class NativeRing:
         return [(int.from_bytes(raw[64 * i : 64 * i + 32], "little"), int.from_bytes(raw[64 * i + 32 : 64 * i + 64], "little")) for i in range(n)]
 
     @staticmethod
-    def pack_prove_inputs(alphas: list[bytes], ads: list[bytes], secret_keys: list[bytes], producer_index: list[int], zk_rows=None) -> dict:
+    def pack_prove_inputs(alphas: list[bytes], ads: list[bytes], secret_keys: list[bytes], producer_index: list[int], zk_rows=None, ring_index=None) -> dict:
         """Host-side packing of a prove batch into the flat buffers of dr_ring_prove_batch (done once per batch, also when the batch
-        is then sharded over several devices: the offsets are absolute, so a shard is just a sub-range of every array)."""
+        is then sharded over several devices: the offsets are absolute, so a shard is just a sub-range of every array).
+        `ring_index` (dr_ring_prove_multi): the ring of every item, an index into the call's list of rings."""
         n = len(alphas)
-        if not (len(ads) == len(secret_keys) == len(producer_index) == n):
+        if not (len(ads) == len(secret_keys) == len(producer_index) == n) or (ring_index is not None and len(ring_index) != n):
             raise ValueError("batch inputs must have equal length")
         blob, a_off, a_len, d_off, d_len = pack_items(alphas, ads)
         rows = np.ctypeslib.as_ctypes(np.array(producer_index if n else [0], dtype=np.uint32))
+        ring = None
+        if ring_index is not None:
+            idx = np.array(ring_index if n else [0], dtype=np.int64)
+            if idx.min() < 0 or idx.max() >> 32:
+                raise ValueError("ring index out of range")
+            ring = np.ctypeslib.as_ctypes(idx.astype(np.uint32))
         zk = None
         if isinstance(zk_rows, (bytes, bytearray)):  # already 12 x 32-byte little-endian values per proof
             if len(zk_rows) != 12 * 32 * n:
@@ -684,23 +692,49 @@ class NativeRing:
                 raise ValueError("zk_rows must hold 12 field elements per proof")
             zk = b"".join(int(v).to_bytes(32, "little") for v in zk_rows)
         return {"n": n, "blob": blob, "a_off": a_off, "a_len": a_len, "d_off": d_off, "d_len": d_len, "sk": b"".join(secret_keys), "rows": rows, "zk": zk,
-                "proofs": ctypes.create_string_buffer(784 * max(n, 1)), "status": (ctypes.c_uint32 * max(n, 1))()}
+                "ring": ring, "proofs": ctypes.create_string_buffer(784 * max(n, 1)), "status": (ctypes.c_uint32 * max(n, 1))()}
+
+    @staticmethod
+    def _packed_args(pk: dict, lo: int, hi: int) -> list:
+        """The batch arguments (blob ... status) of items [lo, hi) of a packed batch, as dr_ring_prove_batch / _multi take them."""
+        u32 = lambda arr: ctypes.byref(arr, 4 * lo)  # noqa: E731
+        sk = (ctypes.c_char * (32 * (hi - lo))).from_buffer_copy(pk["sk"], 32 * lo) if lo or hi != pk["n"] else pk["sk"]
+        zk = None if pk["zk"] is None else (pk["zk"] if not lo and hi == pk["n"] else (ctypes.c_char * (384 * (hi - lo))).from_buffer_copy(pk["zk"], 384 * lo))
+        return [pk["blob"], u32(pk["a_off"]), u32(pk["a_len"]), u32(pk["d_off"]), u32(pk["d_len"]), sk, u32(pk["rows"]), zk, ctypes.byref(pk["proofs"], 784 * lo),
+                ctypes.byref(pk["status"], 4 * lo)]
 
     def prove_packed(self, pk: dict, lo: int = 0, hi: int | None = None) -> None:
         """Prove items [lo, hi) of a packed batch; proofs and status words land in the batch's own output buffers."""
         hi = pk["n"] if hi is None else hi
         if hi <= lo:
             return
-        u32 = lambda arr: ctypes.byref(arr, 4 * lo)  # noqa: E731
-        sk = (ctypes.c_char * (32 * (hi - lo))).from_buffer_copy(pk["sk"], 32 * lo) if lo or hi != pk["n"] else pk["sk"]
-        zk = None if pk["zk"] is None else (pk["zk"] if not lo and hi == pk["n"] else (ctypes.c_char * (384 * (hi - lo))).from_buffer_copy(pk["zk"], 384 * lo))
+        args = self._packed_args(pk, lo, hi)
         lib = self.ctx.library
         if self.time_calls:  # one CUDA event pair on the ctx stream around the whole call (bench.py); every argument is ready by now
             self.ctx.timer_start()
-        lib.check(lib.lib.dr_ring_prove_batch(self.ctx.handle, self.handle, hi - lo, pk["blob"], u32(pk["a_off"]), u32(pk["a_len"]), u32(pk["d_off"]), u32(pk["d_len"]), sk,
-                                              u32(pk["rows"]), zk, ctypes.byref(pk["proofs"], 784 * lo), ctypes.byref(pk["status"], 4 * lo)))
+        lib.check(lib.lib.dr_ring_prove_batch(self.ctx.handle, self.handle, hi - lo, *args))
         if self.time_calls:
             self.last_call_ms = self.ctx.timer_stop()
+
+    @staticmethod
+    def prove_multi_packed(rings: list["NativeRing"], pk: dict, lo: int = 0, hi: int | None = None) -> None:
+        """dr_ring_prove_multi over items [lo, hi) of a batch packed with a ring-index column (indices into `rings`)."""
+        hi = pk["n"] if hi is None else hi
+        if hi <= lo:
+            return
+        if not rings:
+            raise ValueError("at least one ring is required")
+        ctx = rings[0].ctx
+        handles = (c_void_p * len(rings))(*[r.handle for r in rings])
+        ctx.library.check(ctx.library.lib.dr_ring_prove_multi(ctx.handle, handles, len(rings), ctypes.byref(pk["ring"], 4 * lo), hi - lo, *NativeRing._packed_args(pk, lo, hi)))
+
+    @staticmethod
+    def prove_multi(rings: list["NativeRing"], index: list[int], alphas: list[bytes], ads: list[bytes], secret_keys: list[bytes], producer_index: list[int],
+                    zk_rows=None):
+        """Item i against rings[index[i]] in one call (dr_ring_prove_multi) -> (list of 784-byte proofs, list of status words)."""
+        pk = NativeRing.pack_prove_inputs(alphas, ads, secret_keys, producer_index, zk_rows, ring_index=index)
+        NativeRing.prove_multi_packed(rings, pk)
+        return NativeRing.unpack_proofs(pk)
 
     @staticmethod
     def unpack_proofs(pk: dict):

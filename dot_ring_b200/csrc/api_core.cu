@@ -350,6 +350,10 @@ int dr_ctx_create(int device, dr_ctx** out) {
     ctx->side = 0;
     ctx->side2 = 0;
 #endif
+    {
+        std::lock_guard<std::mutex> lock(live_ctx_mutex());
+        live_ctxs().insert(ctx.get());
+    }
     *out = (dr_ctx*)ctx.release();
     DR_API_END
 }
@@ -357,6 +361,10 @@ int dr_ctx_create(int device, dr_ctx** out) {
 void dr_ctx_destroy(dr_ctx* c) {
     Ctx* ctx = (Ctx*)c;
     if (!ctx) return;
+    {
+        std::lock_guard<std::mutex> lock(live_ctx_mutex());
+        live_ctxs().erase(ctx);
+    }
 #if !defined(DR_HOST_EMULATION)
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
@@ -530,7 +538,12 @@ int dr_srs_load(dr_ctx* c, const uint8_t* g1_be96, size_t n_g1, const uint8_t* g
     DR_API_END
 }
 
-void dr_srs_destroy(dr_srs* s) { delete (Srs*)s; }
+void dr_srs_destroy(dr_srs* s) {
+    Srs* srs = (Srs*)s;
+    if (!srs) return;
+    free_on_owner_stream(srs->ctx);
+    delete srs;
+}
 size_t dr_srs_size(const dr_srs* s) { return s ? ((const Srs*)s)->n : 0; }
 void dr_srs_geometry(const dr_srs* s, uint32_t* window_bits, uint32_t* wide_windows, uint32_t* glv, uint32_t* additions) {
     const TableGeom g = s ? ((const Srs*)s)->geom : TableGeom{};

@@ -2,6 +2,8 @@
 #pragma once
 #include <chrono>
 #include <memory>
+#include <mutex>
+#include <set>
 #include <string>
 #include <vector>
 
@@ -179,6 +181,34 @@ struct Ctx {
     }
 };
 
+// Contexts created and not yet destroyed.  A ring or SRS can outlive its context (the Python wrappers are garbage-collected in any
+// order), so its destroy must not touch a context that is gone.
+inline std::mutex& live_ctx_mutex() {
+    static std::mutex m;
+    return m;
+}
+inline std::set<const Ctx*>& live_ctxs() {
+    static std::set<const Ctx*> s;
+    return s;
+}
+// Before an object's device buffers are freed: the block cache records a freed block on the calling thread's current stream
+// (rt.cuh dev_free), and that stream may belong to a context destroyed since, possibly by another thread (an EnginePool worker
+// tears its contexts down).  Free on the owning context's stream while that context is alive, else on the legacy stream.
+inline void free_on_owner_stream(const Ctx* ctx) {
+#if !defined(DR_HOST_EMULATION)
+    std::lock_guard<std::mutex> lock(live_ctx_mutex());
+    current_stream() = nullptr;
+    if (ctx && live_ctxs().count(ctx)) {
+        if (cudaSetDevice(ctx->device) == cudaSuccess)
+            current_stream() = ctx->stream;
+        else
+            cudaGetLastError();  // the failure must not surface at the next launch check
+    }
+#else
+    (void)ctx;
+#endif
+}
+
 // batch transforms of `n` Montgomery elements each, in place (or in -> out); n a power of two up to 2^22
 void ntt_device(Ctx* ctx, const NttPlan& plan, const Fr* in, Fr* out, size_t batch, bool inverse, DevBuf<Fr>& tmp);
 
@@ -209,9 +239,12 @@ struct Ring {
     Ctx* ctx = nullptr;
     Srs* srs = nullptr;
     RingDev dev{};
+    Fr radix_omega;  // w4 (Montgomery): rings proved in one pass must share it with omega
     DevBuf<TEAffine> nm;
     DevBuf<Fr> fixed_coef, fixed_lde, w4, w4inv;
     DevBuf<Shake128> prefix;
+    RingTab tab{};            // this ring's entry of a prove call's ring table
+    DevBuf<RingTab> tab_dev;  // the one-entry table of dr_ring_prove_batch
     G1Affine commitments[3];
     uint8_t commit_be96[288];
     uint8_t root144[144];
@@ -223,6 +256,12 @@ struct Ring {
     SuiteDev suite{};
     std::shared_ptr<Ctx::FixedTable> g_table, b_table;
 };
+
+// Suite identity of the Pedersen part: suite id, hash-to-curve DST, hash, generator and blinding base.
+inline bool same_suite(const SuiteDev& a, const SuiteDev& b) {
+    return a.suite_id_len == b.suite_id_len && !memcmp(a.suite_id, b.suite_id, a.suite_id_len) && a.dst_len == b.dst_len && !memcmp(a.dst, b.dst, a.dst_len) &&
+           a.hash_kind == b.hash_kind && a.generator == b.generator && a.blinding_base == b.blinding_base;
+}
 
 
 VerifierKeyDev make_verifier_key(Ctx* ctx, uint32_t N, const Fr& omega, const TEAffine& seed, const uint8_t* label, uint32_t label_len, const uint8_t* g1_0_be96,

@@ -1,6 +1,8 @@
 // C ABI, part 3: ring set-up (key ingestion, fixed columns, ring root) and batched Ring VRF proving.
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 
 #include "api_internal.cuh"
 #include "ring.cuh"
@@ -35,8 +37,11 @@ struct ProveScratch {
     DevBuf<uint8_t> out, zraw, blob;
     DevBuf<uint32_t> status;
     static size_t elements_per_proof(uint32_t N) { return (size_t)27 * N + 1; }
+    // A scratch sized for a larger domain fits a smaller one: every buffer holds per-proof rows of a size that grows with N, and
+    // the views inside `lde` stay disjoint for any pass of at most `cap` proofs at a domain of at most N.
+    bool fits(size_t n, uint32_t N_) const { return n <= cap && N_ <= N; }
     void ensure(size_t n, uint32_t N_) {
-        if (n <= cap && N_ == N) return;
+        if (fits(n, N_)) return;
         cap = n;
         N = N_;
         size_t q = 3 * (size_t)N + 1;
@@ -59,6 +64,246 @@ struct ProveScratch {
 static ProveScratch& scratch_for(Ctx* ctx) {
     if (!ctx->prove_scratch) ctx->prove_scratch = std::shared_ptr<void>(new ProveScratch(), [](void* p) { delete (ProveScratch*)p; });
     return *(ProveScratch*)ctx->prove_scratch.get();
+}
+
+// One prove call: item i against rings[ring_index[i]] (ring_index null: every item against rings[0]).  The callers have checked
+// that the rings share the context, the SRS and the suite; `dtab` holds their RingTab entries on the device, in the same order.
+// Items are grouped by domain size (ascending), in the caller's order within a group, and every group runs its own equal-width
+// passes over one scratch sized for the largest domain of the call.  Proofs and status words land at the caller's positions.
+static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const uint32_t* ring_index, size_t n, const uint8_t* blob, const uint32_t* alpha_off,
+                       const uint32_t* alpha_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* secret_keys32, const uint32_t* producer_index,
+                       const uint8_t* zk_rows, uint8_t* proofs784, uint32_t* status) {
+    auto ring_of = [&](size_t i) { return ring_index ? ring_index[i] : 0u; };
+    size_t blob_len = 0;
+    std::vector<uint32_t> domains;  // distinct domain sizes of the items' rings
+    for (size_t i = 0; i < n; i++) {
+        size_t e1 = (size_t)alpha_off[i] + alpha_len[i], e2 = (size_t)ad_off[i] + ad_len[i];
+        if (e1 > blob_len) blob_len = e1;
+        if (e2 > blob_len) blob_len = e2;
+        const uint32_t N = rings[ring_of(i)]->dev.N;
+        if (std::find(domains.begin(), domains.end(), N) == domains.end()) domains.push_back(N);
+    }
+    if (blob_len && !blob) throw Error(DR_EINVAL, "null blob");
+    std::sort(domains.begin(), domains.end());
+    // one group: the items in the caller's order, copied in and out in place; several: gathered per group and scattered back
+    const bool direct = domains.size() == 1;
+    std::vector<uint32_t> order;
+    std::vector<size_t> group_end;
+    size_t widest = n;
+    if (!direct) {
+        order.reserve(n);
+        widest = 0;
+        for (uint32_t N : domains) {
+            const size_t begin = order.size();
+            for (size_t i = 0; i < n; i++)
+                if (rings[ring_of(i)]->dev.N == N) order.push_back((uint32_t)i);
+            group_end.push_back(order.size());
+            if (order.size() - begin > widest) widest = order.size() - begin;
+        }
+    } else {
+        group_end.push_back(n);
+    }
+    const uint32_t N_max = domains.back();
+    // (the input blob goes into a buffer that lives with the scratch: no allocation on the steady-state path)
+
+    // proofs per pass: the one-thread-per-proof kernels (Pedersen part, witness chain, transcripts) are latency-bound, so
+    // a pass should be as wide as the scratch (35 N field elements + state per proof) allows
+    size_t chunk_cap = ctx->prove_chunk ? ctx->prove_chunk : 8192;
+#if !defined(DR_HOST_EMULATION)
+    // The free-memory query (like any allocation) can stall for tens of ms inside the driver, so it is only made when the scratch
+    // has to grow: a call that fits the scratch of an earlier one reuses its pass width.
+    {
+        ProveScratch& cur = scratch_for(ctx);
+        const size_t want = widest < chunk_cap ? widest : chunk_cap;
+        if (!ctx->prove_chunk && !cur.fits(want, N_max)) {
+            size_t free_b = 0, total_b = 0;
+            DR_CUDA(cudaMemGetInfo(&free_b, &total_b));
+            free_b += dev_cache().cached;  // recycled blocks are available to this call
+            size_t per_proof = (ProveScratch::elements_per_proof(N_max) + (N_max > 4096 ? 16 * (size_t)N_max : 0)) * sizeof(Fr) + sizeof(ProofState) + 4096;
+            size_t have = free_b + (cur.N == N_max ? cur.cap * per_proof : 0);
+            // keep 1 GB (or half of what is left, if less) for the other buffers of this and later calls
+            const size_t keep = have / 2 < ((size_t)1 << 30) ? have / 2 : ((size_t)1 << 30);
+            size_t fit = (have - keep) / per_proof;
+            if (getenv("DOT_RING_B200_DEBUG"))
+                fprintf(stderr, "[dot_ring_b200] prove: free %.2f GB (+%.2f GB held), %.2f MB per proof -> up to %zu proofs per pass\n", free_b / 1e9,
+                        (double)(have - free_b) / 1e9, per_proof / 1e6, fit);
+            if (fit < chunk_cap) chunk_cap = fit < 64 ? 64 : fit;
+        }
+    }
+#endif
+    // equal passes: a group of g proofs in ceil(g / cap) passes of the same width (a short last pass would pay the latency-bound
+    // kernels again for little work)
+    auto pass_width_of = [&](size_t g) {
+        const size_t passes = (g + chunk_cap - 1) / chunk_cap;
+        return (g + passes - 1) / passes;
+    };
+    ProveScratch& sc = scratch_for(ctx);
+    sc.ensure(pass_width_of(widest), N_max);
+    sc.blob.ensure(blob_len ? blob_len : 1);
+    h2d(ctx->stream, sc.blob.p, blob, blob_len);
+    PhaseTimer& pt = ctx->phases;
+    pt.reset();
+    pt.active = true;
+    struct Deactivate {
+        PhaseTimer& p;
+        ~Deactivate() { p.active = false; }
+    } deactivate{pt};
+    std::vector<ProveInput> hin;
+    std::vector<uint8_t> hzk, hout;
+    std::vector<uint32_t> hstatus;
+
+    for (size_t g = 0, group_begin = 0; g < group_end.size(); group_begin = group_end[g++]) {
+        const size_t group_n = group_end[g] - group_begin;
+        auto item = [&](size_t j) -> size_t { return direct ? j : order[group_begin + j]; };
+        // everything of a pass that depends only on N or on the suite comes from the group's first ring
+        Ring* lead = rings[ring_of(item(0))];
+        const RingDev& rg = lead->dev;
+        const uint32_t N = rg.N;
+        const uint32_t qlen = 3 * N + 1;
+        const uint32_t nthr = ntt_threads(N);
+        const size_t ntt_smem = ntt_smem_bytes(N);
+        const bool large = N > 4096 || ctx->generic_ntt_path;  // two-pass transforms + element-wise twists instead of the fused single-CTA kernels
+        const NttPlan* big_plan = large ? &ctx->plan(N, rg.omega) : nullptr;
+        const size_t pass_width = pass_width_of(group_n);
+
+        for (size_t base = 0; base < group_n; base += pass_width) {
+            const uint32_t m = (uint32_t)((group_n - base < pass_width) ? group_n - base : pass_width);
+            pt.mark(ctx, 7);
+            hin.assign(m, ProveInput{});
+            for (uint32_t i = 0; i < m; i++) {
+                const size_t it = item(base + i);
+                ProveInput& pi = hin[i];
+                pi.alpha_off = alpha_off[it];
+                pi.alpha_len = alpha_len[it];
+                pi.ad_off = ad_off[it];
+                pi.ad_len = ad_len[it];
+                pi.k = producer_index[it];
+                pi.ring = ring_of(it);
+                memcpy(pi.sk, secret_keys32 + 32 * it, 32);
+            }
+            h2d(ctx->stream, sc.in.p, hin.data(), m * sizeof(ProveInput));
+            const uint32_t tb = 64, pb = (m + tb - 1) / tb;
+
+            pt.mark(ctx, 0);
+            // zk rows (Montgomery) into the state, then Pedersen + witness
+            if (zk_rows) {
+                const uint8_t* src = zk_rows + base * 12 * 32;
+                if (!direct) {
+                    hzk.resize((size_t)m * 12 * 32);
+                    for (uint32_t i = 0; i < m; i++) memcpy(hzk.data() + (size_t)i * 12 * 32, zk_rows + item(base + i) * 12 * 32, 12 * 32);
+                    src = hzk.data();
+                }
+                h2d(ctx->stream, sc.zraw.p, src, (size_t)m * 12 * 32);
+                launch(ctx->stream, Dim3((m * 12 + 127) / 128), 128, 0, ZkRowsBody(), (const uint8_t*)sc.zraw.p, sc.st.p, m);
+            } else {
+                launch(ctx->stream, Dim3((m * 12 + 127) / 128), 128, 0, ZkRowsBody(), (const uint8_t*)nullptr, sc.st.p, m);
+            }
+            // Pedersen part: the half the ring proof needs (blinding factor, blinded key) on the main stream, eight lanes per proof; the
+            // rest (nonces, R, Ok, responses) on the side stream, joined before the proofs are assembled
+            {
+                const uint32_t per_block = tb / COOP_LANES;  // eight lanes per proof
+                launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, pedersen_start_smem(tb), PedersenStartBody(), rg, dtab, (const ProveInput*)sc.in.p,
+                       (const uint8_t*)sc.blob.p, sc.st.p, m);
+            }
+            ctx->fork_side();
+            launch(ctx->side, Dim3((m + 31) / 32), 32, 0, PedersenFinishBody(), rg, (const ProveInput*)sc.in.p, sc.st.p, m);
+            {
+                const uint32_t wt = 4 * WIT_LANES;  // four proofs per block, a warp each
+                launch(ctx->stream, Dim3((m + 3) / 4), wt, witness_coop_smem(wt), WitnessBody(), rg, dtab, sc.st.p, m);
+            }
+            pt.mark(ctx, 1);
+            // The coefficient form of the witness columns is first needed by the low-degree extension, the commitments by the transcript:
+            // on the fused path the interpolation runs on a second side stream next to the (sparse) commitments.
+            const bool overlap_intt = !large && !ctx->dense_witness_commit;
+            if (!large) {
+                if (overlap_intt) ctx->fork_side2();
+                launch(overlap_intt ? ctx->side2 : ctx->stream, Dim3(4, m), nthr, ntt_smem, WitnessInttBody(), rg, dtab, (const ProofState*)sc.st.p, sc.wit_coef.p);
+            } else {
+                launch(ctx->stream, Dim3((N + 127) / 128, 4, m), 128, 0, WitnessEvalBody(), rg, dtab, (const ProofState*)sc.st.p, sc.wit_coef.p);
+                ntt_device(ctx, *big_plan, sc.wit_coef.p, sc.wit_coef.p, 4 * (size_t)m, true, sc.ntt_tmp);
+            }
+            pt.mark(ctx, 2);
+            if (ctx->dense_witness_commit || large) {
+                commit_device(ctx, lead->srs, sc.wit_coef.p, N, N, 4 * m, sc.res.p);
+            } else {
+                // the Lagrange table is per SRS and domain: every ring of the group shares it
+                const LagrangeTable* lag = lead->lag ? lead->lag : &lead->srs->lagrange_table(N, rg.logN, rg.omega, rg.tw_inv, rg.n_inv);
+                for (size_t i = 0; i < m; i++) rings[ring_of(item(base + i))]->lag = lag;
+                ctx->partials.ensure((size_t)4 * m);
+                launch_lb<64, 8>(ctx->stream, Dim3(4, m), 64, witness_commit_smem(lag->geom.W, 64), WitnessCommitBody(), (const G1Affine*)lag->table.p, lag->geom, rg,
+                                 dtab, (const ProofState*)sc.st.p, ctx->partials.p);
+                launch_commit_finish(ctx->stream, (const G1*)ctx->partials.p, 1u, 4 * m, sc.res.p);
+            }
+            // column order (b, accx, accy, accip) -> payload slots (0, 2, 3, 1)
+            launch(ctx->stream, Dim3((4 * m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)sc.res.p, 4u, 0x01030200u, sc.st.p, m);
+            pt.mark(ctx, 5);
+            launch(ctx->stream, Dim3(pb), tb, 0, Transcript1Body(), sc.st.p, m);
+            if (overlap_intt) ctx->join_side2();
+            pt.mark(ctx, 3);
+            if (!large) {
+                launch(ctx->stream, Dim3(16, m), nthr, ntt_smem, WitnessLdeBody(), rg, dtab, (const ProofState*)sc.st.p, (const Fr*)sc.wit_coef.p, sc.lde.p);
+            } else {
+                launch(ctx->stream, Dim3((N + 127) / 128, 4, 4 * m), 128, 0, CosetTwistBody(), N, rg.w4, (const Fr*)sc.wit_coef.p, sc.lde.p);
+                ntt_device(ctx, *big_plan, sc.lde.p, sc.lde.p, 16 * (size_t)m, false, sc.ntt_tmp);
+            }
+            launch(ctx->stream, Dim3((4 * N + 127) / 128, m), 128, 0, ConstraintBody(), rg, dtab, (const ProofState*)sc.st.p, (const Fr*)sc.lde.p, sc.agg.p);
+            if (!large) {
+                launch(ctx->stream, Dim3(4, m), nthr, ntt_smem, QuotientInttBody(), rg, sc.agg.p);
+            } else {
+                ntt_device(ctx, *big_plan, sc.agg.p, sc.agg.p, 4 * (size_t)m, true, sc.ntt_tmp);
+                launch(ctx->stream, Dim3((N + 127) / 128, 4, m), 128, 0, CosetUntwistBody(), N, rg.w4inv, sc.agg.p);
+            }
+            launch(ctx->stream, Dim3((N + 127) / 128, m), 128, 0, QuotientCombineBody(), rg, (const Fr*)sc.agg.p, sc.cagg.p);
+            launch(ctx->stream, Dim3((qlen + 127) / 128, m), 128, 0, QuotientFoldBody(), rg, (const Fr*)sc.cagg.p, sc.quot.p, qlen);
+            pt.mark(ctx, 2);
+            commit_device(ctx, lead->srs, sc.quot.p, qlen, qlen, m, sc.res.p);
+            launch(ctx->stream, Dim3((m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)sc.res.p, 1u, 0x04u, sc.st.p, m);
+            pt.mark(ctx, 5);
+            launch(ctx->stream, Dim3(pb), tb, 0, Transcript2Body(), sc.st.p, m);
+            pt.mark(ctx, 4);
+            launch(ctx->stream, Dim3(7, m), 128, 128 * sizeof(Fr), EvalBody(), rg, dtab, sc.st.p, (const Fr*)sc.wit_coef.p);
+            launch(ctx->stream, Dim3((N + 127) / 128, m), 128, 0, LinPolyBody(), rg, (const ProofState*)sc.st.p, (const Fr*)sc.wit_coef.p, sc.lin.p);
+            launch(ctx->stream, Dim3(1, m), 128, 128 * sizeof(Fr), LinEvalBody(), rg, sc.st.p, (const Fr*)sc.lin.p);
+            pt.mark(ctx, 5);
+            launch(ctx->stream, Dim3(pb), tb, 0, Transcript3Body(), sc.st.p, m);
+            pt.mark(ctx, 4);
+            launch(ctx->stream, Dim3((qlen + 127) / 128, m), 128, 0, AggOpenBody(), rg, dtab, (const ProofState*)sc.st.p, (const Fr*)sc.wit_coef.p, (const Fr*)sc.quot.p, qlen,
+                   sc.aggopen.p);
+            launch(ctx->stream, Dim3(2, m), 256, synthetic_div_smem(256), OpenQuotientsBody(), rg, (const ProofState*)sc.st.p, sc.aggopen.p, qlen, sc.lin.p);
+            pt.mark(ctx, 2);
+            commit_device_pair(ctx, lead->srs, sc.aggopen.p, qlen, 3 * N, sc.lin.p, N, N - 1, m, sc.res.p);
+            launch(ctx->stream, Dim3((m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)sc.res.p, 1u, 0x05u, sc.st.p, m);
+            launch(ctx->stream, Dim3((m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)(sc.res.p + m), 1u, 0x06u, sc.st.p, m);
+            pt.mark(ctx, 5);
+            ctx->join_side();
+            launch(ctx->stream, Dim3(pb), tb, 0, FinalizeBody(), (const ProofState*)sc.st.p, m, sc.out.p, sc.status.p);
+            pt.mark(ctx, 8);
+            dev_zero(ctx->stream, sc.in.p, m * sizeof(ProveInput));  // secret keys do not outlive the pass on the device
+            if (direct) {
+                d2h(ctx->stream, proofs784 + 784 * base, sc.out.p, (size_t)m * 784);
+                d2h(ctx->stream, status + base, sc.status.p, (size_t)m * sizeof(uint32_t));
+            } else {
+                hout.resize((size_t)m * 784);
+                hstatus.resize(m);
+                d2h(ctx->stream, hout.data(), sc.out.p, (size_t)m * 784);
+                d2h(ctx->stream, hstatus.data(), sc.status.p, (size_t)m * sizeof(uint32_t));
+            }
+            pt.mark(ctx, -1);
+            stream_sync(ctx->stream);
+            pt.collect(ctx);
+            if (!direct) {
+                for (uint32_t i = 0; i < m; i++) {
+                    const size_t it = item(base + i);
+                    memcpy(proofs784 + 784 * it, hout.data() + (size_t)784 * i, 784);
+                    status[it] = hstatus[i];
+                }
+            }
+        }
+    }
+    {  // ... nor in the host staging buffer (volatile: the stores must not be optimised away)
+        volatile uint8_t* w = (volatile uint8_t*)hin.data();
+        for (size_t i = 0; i < hin.size() * sizeof(ProveInput); i++) w[i] = 0;
+    }
 }
 
 }  // namespace dr
@@ -100,10 +345,12 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     d.N = N;
     d.logN = 0;
     while ((1u << d.logN) < N) d.logN++;
-    d.max_ring = prm->max_ring_size;
+    const uint32_t max_ring = prm->max_ring_size;
+    ring->tab.max_ring = max_ring;
     d.last = N - 4;
     d.omega = fr_from_param(prm->omega);
     Fr w4 = fr_from_param(prm->radix_omega);
+    ring->radix_omega = w4;
     // sanity: w4^4 == omega, omega^N == 1, omega^(N/2) != 1
     if (w4.sqr().sqr() != d.omega) throw Error(DR_EINVAL, "radix_omega^4 != omega");
     {
@@ -163,9 +410,9 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     ring->nm.alloc(N);
     {
         std::vector<TEAffine> host(N);
-        for (uint32_t i = 0; i < d.max_ring; i++) host[i] = ring->padding;
+        for (uint32_t i = 0; i < max_ring; i++) host[i] = ring->padding;
         TEExt cur = TEExt::from_affine(d.blinding_base);
-        for (uint32_t i = d.max_ring; i < N - 4; i++) {
+        for (uint32_t i = max_ring; i < N - 4; i++) {
             host[i] = te_to_affine(cur);
             cur = te_dbl(cur);
         }
@@ -178,15 +425,15 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
             stream_sync(ctx->stream);
         }
     }
-    d.nm = ring->nm.p;
+    ring->tab.nm = ring->nm.p;
 
     // ---- fixed columns: evaluations -> coefficients -> commitments ----
     ring->fixed_coef.alloc(3 * N);
-    launch(ctx->stream, Dim3((N + 127) / 128), 128, 0, FixedColumnsBody(), (const TEAffine*)ring->nm.p, N, d.max_ring, ring->fixed_coef.p);
+    launch(ctx->stream, Dim3((N + 127) / 128), 128, 0, FixedColumnsBody(), (const TEAffine*)ring->nm.p, N, max_ring, ring->fixed_coef.p);
     const uint32_t nthr = ntt_threads(N);
     DevBuf<Fr> ntt_tmp;
     ntt_device(ctx, plan, ring->fixed_coef.p, ring->fixed_coef.p, 3, true, ntt_tmp);
-    d.fixed_coef = ring->fixed_coef.p;
+    ring->tab.fixed_coef = ring->fixed_coef.p;
     DevBuf<G1Affine> cm(3);
     commit_device(ctx, srs, ring->fixed_coef.p, N, N, 3, cm.p);
     DevBuf<uint8_t> enc96(288), enc48(144);
@@ -219,7 +466,7 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
         launch(ctx->stream, Dim3((4 * N + 127) / 128), 128, 0, NotLastBody(), N, (const Fr*)ring->w4.p, d.w_last, ring->fixed_lde.p + 5 * 4 * (size_t)N);
         stream_sync(ctx->stream);
     }
-    d.fixed_lde = ring->fixed_lde.p;
+    ring->tab.fixed_lde = ring->fixed_lde.p;
 
     // ---- verifier-key transcript prefix (root.py:54-71, phases.py:72-74) ----
     {
@@ -234,6 +481,9 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
         tr.absorb_be32(96 + 384 + 288);
         ring->prefix.alloc(1);
         h2d(ctx->stream, ring->prefix.p, &tr, sizeof(Shake128));
+        ring->tab.prefix = ring->prefix.p;
+        ring->tab_dev.alloc(1);
+        h2d(ctx->stream, ring->tab_dev.p, &ring->tab, sizeof(RingTab));
         stream_sync(ctx->stream);
     }
     ring->vk = make_verifier_key(ctx, N, d.omega, d.seed, d.suite_id, d.suite_id_len, srs->g1_0_be96, srs->g2_be192, ring->commit_be96, ring->vk_lines);
@@ -253,7 +503,12 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     DR_API_END
 }
 
-void dr_ring_destroy(dr_ring* r) { delete (Ring*)r; }
+void dr_ring_destroy(dr_ring* r) {
+    Ring* ring = (Ring*)r;
+    if (!ring) return;
+    free_on_owner_stream(ring->ctx);
+    delete ring;
+}
 
 int dr_ring_root(dr_ring* r, uint8_t root144[144]) {
     DR_API_BEGIN
@@ -294,176 +549,43 @@ int dr_ring_prove_batch(dr_ctx* c, dr_ring* r, size_t n, const uint8_t* blob, co
         throw Error(DR_EINVAL, "bad argument");
     ctx->activate();
     if (!n) return DR_OK;
-    const RingDev& rg = ring->dev;
-    const uint32_t N = rg.N;
-    const uint32_t qlen = 3 * N + 1;
-    size_t blob_len = 0;
-    for (size_t i = 0; i < n; i++) {
-        size_t e1 = (size_t)alpha_off[i] + alpha_len[i], e2 = (size_t)ad_off[i] + ad_len[i];
-        if (e1 > blob_len) blob_len = e1;
-        if (e2 > blob_len) blob_len = e2;
-    }
-    if (blob_len && !blob) throw Error(DR_EINVAL, "null blob");
-    // (the input blob goes into a buffer that lives with the scratch: no allocation on the steady-state path)
+    ring_prove(ctx, &ring, ring->tab_dev.p, nullptr, n, blob, alpha_off, alpha_len, ad_off, ad_len, secret_keys32, producer_index, zk_rows, proofs784, status);
+    DR_API_END
+}
 
-    // proofs per pass: the one-thread-per-proof kernels (Pedersen part, witness chain, transcripts) are latency-bound, so
-    // a pass should be as wide as the scratch (35 N field elements + state per proof) allows
-    size_t chunk_cap = ctx->prove_chunk ? ctx->prove_chunk : 8192;
-#if !defined(DR_HOST_EMULATION)
-    // The free-memory query (like any allocation) can stall for tens of ms inside the driver, so it is only made when the scratch
-    // has to grow: a call that fits the scratch of an earlier one reuses its pass width.
-    {
-        ProveScratch& cur = scratch_for(ctx);
-        const size_t want = n < chunk_cap ? n : chunk_cap;
-        if (!ctx->prove_chunk && !(cur.N == N && want <= cur.cap)) {
-            size_t free_b = 0, total_b = 0;
-            DR_CUDA(cudaMemGetInfo(&free_b, &total_b));
-            free_b += dev_cache().cached;  // recycled blocks are available to this call
-            size_t per_proof = (ProveScratch::elements_per_proof(N) + (N > 4096 ? 16 * (size_t)N : 0)) * sizeof(Fr) + sizeof(ProofState) + 4096;
-            size_t have = free_b + (cur.N == N ? cur.cap * per_proof : 0);
-            // keep 1 GB (or half of what is left, if less) for the other buffers of this and later calls
-            const size_t keep = have / 2 < ((size_t)1 << 30) ? have / 2 : ((size_t)1 << 30);
-            size_t fit = (have - keep) / per_proof;
-            if (getenv("DOT_RING_B200_DEBUG"))
-                fprintf(stderr, "[dot_ring_b200] prove: free %.2f GB (+%.2f GB held), %.2f MB per proof -> up to %zu proofs per pass\n", free_b / 1e9,
-                        (double)(have - free_b) / 1e9, per_proof / 1e6, fit);
-            if (fit < chunk_cap) chunk_cap = fit < 64 ? 64 : fit;
-        }
+int dr_ring_prove_multi(dr_ctx* c, dr_ring* const* rs, size_t n_rings, const uint32_t* ring_index, size_t n, const uint8_t* blob, const uint32_t* alpha_off,
+                        const uint32_t* alpha_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* secret_keys32, const uint32_t* producer_index,
+                        const uint8_t* zk_rows, uint8_t* proofs784, uint32_t* status) {
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || (n_rings && !rs) || n_rings > UINT32_MAX ||
+        (n && (!ring_index || !alpha_off || !alpha_len || !ad_off || !ad_len || !secret_keys32 || !producer_index || !proofs784 || !status)))
+        throw Error(DR_EINVAL, "bad argument");
+    if (n && !n_rings) throw Error(DR_EINVAL, "at least one ring is required");
+    Ring* const* rings = (Ring* const*)rs;
+    for (size_t k = 0; k < n_rings; k++) {
+        const Ring* ring = rings[k];
+        const Ring* first = rings[0];
+        if (!ring) throw Error(DR_EINVAL, "bad argument");
+        if (ring->ctx != ctx) throw Error(DR_EINVAL, "ring belongs to another context");
+        if (ring->srs != first->srs) throw Error(DR_EINVAL, "rings of one call must share the SRS handle");
+        if (!same_suite(ring->suite, first->suite) || !(ring->dev.seed == first->dev.seed) || !(ring->padding == first->padding))
+            throw Error(DR_EINVAL, "rings of one call must share the suite");
     }
-#endif
-    // equal passes: n proofs in ceil(n / cap) passes of the same width (a short last pass would pay the latency-bound kernels again
-    // for little work)
-    const size_t passes = (n + chunk_cap - 1) / chunk_cap;
-    const size_t pass_width = (n + passes - 1) / passes;
-    ProveScratch& sc = scratch_for(ctx);
-    sc.ensure(pass_width, N);
-    sc.blob.ensure(blob_len ? blob_len : 1);
-    h2d(ctx->stream, sc.blob.p, blob, blob_len);
-    PhaseTimer& pt = ctx->phases;
-    pt.reset();
-    pt.active = true;
-    struct Deactivate {
-        PhaseTimer& p;
-        ~Deactivate() { p.active = false; }
-    } deactivate{pt};
-    const uint32_t nthr = ntt_threads(N);
-    const size_t ntt_smem = ntt_smem_bytes(N);
-    const bool large = N > 4096 || ctx->generic_ntt_path;  // two-pass transforms + element-wise twists instead of the fused single-CTA kernels
-    const NttPlan* big_plan = large ? &ctx->plan(N, rg.omega) : nullptr;
-    std::vector<ProveInput> hin;
-
-    for (size_t base = 0; base < n; base += pass_width) {
-        const uint32_t m = (uint32_t)((n - base < pass_width) ? n - base : pass_width);
-        pt.mark(ctx, 7);
-        hin.assign(m, ProveInput{});
-        for (uint32_t i = 0; i < m; i++) {
-            ProveInput& pi = hin[i];
-            pi.alpha_off = alpha_off[base + i];
-            pi.alpha_len = alpha_len[base + i];
-            pi.ad_off = ad_off[base + i];
-            pi.ad_len = ad_len[base + i];
-            pi.k = producer_index[base + i];
-            memcpy(pi.sk, secret_keys32 + 32 * (base + i), 32);
-        }
-        h2d(ctx->stream, sc.in.p, hin.data(), m * sizeof(ProveInput));
-        const uint32_t tb = 64, pb = (m + tb - 1) / tb;
-
-        pt.mark(ctx, 0);
-        // zk rows (Montgomery) into the state, then Pedersen + witness
-        if (zk_rows) {
-            h2d(ctx->stream, sc.zraw.p, zk_rows + (size_t)base * 12 * 32, (size_t)m * 12 * 32);
-            launch(ctx->stream, Dim3((m * 12 + 127) / 128), 128, 0, ZkRowsBody(), (const uint8_t*)sc.zraw.p, sc.st.p, m);
-        } else {
-            launch(ctx->stream, Dim3((m * 12 + 127) / 128), 128, 0, ZkRowsBody(), (const uint8_t*)nullptr, sc.st.p, m);
-        }
-        // Pedersen part: the half the ring proof needs (blinding factor, blinded key) on the main stream, eight lanes per proof; the
-        // rest (nonces, R, Ok, responses) on the side stream, joined before the proofs are assembled
-        {
-            const uint32_t per_block = tb / COOP_LANES;  // eight lanes per proof
-            launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, pedersen_start_smem(tb), PedersenStartBody(), rg, (const ProveInput*)sc.in.p, (const uint8_t*)sc.blob.p,
-                   sc.st.p, m);
-        }
-        ctx->fork_side();
-        launch(ctx->side, Dim3((m + 31) / 32), 32, 0, PedersenFinishBody(), rg, (const ProveInput*)sc.in.p, sc.st.p, m);
-        {
-            const uint32_t wt = 4 * WIT_LANES;  // four proofs per block, a warp each
-            launch(ctx->stream, Dim3((m + 3) / 4), wt, witness_coop_smem(wt), WitnessBody(), rg, sc.st.p, m, (const Shake128*)ring->prefix.p);
-        }
-        pt.mark(ctx, 1);
-        // The coefficient form of the witness columns is first needed by the low-degree extension, the commitments by the transcript:
-        // on the fused path the interpolation runs on a second side stream next to the (sparse) commitments.
-        const bool overlap_intt = !large && !ctx->dense_witness_commit;
-        if (!large) {
-            if (overlap_intt) ctx->fork_side2();
-            launch(overlap_intt ? ctx->side2 : ctx->stream, Dim3(4, m), nthr, ntt_smem, WitnessInttBody(), rg, (const ProofState*)sc.st.p, sc.wit_coef.p);
-        } else {
-            launch(ctx->stream, Dim3((N + 127) / 128, 4, m), 128, 0, WitnessEvalBody(), rg, (const ProofState*)sc.st.p, sc.wit_coef.p);
-            ntt_device(ctx, *big_plan, sc.wit_coef.p, sc.wit_coef.p, 4 * (size_t)m, true, sc.ntt_tmp);
-        }
-        pt.mark(ctx, 2);
-        if (ctx->dense_witness_commit || large) {
-            commit_device(ctx, ring->srs, sc.wit_coef.p, N, N, 4 * m, sc.res.p);
-        } else {
-            if (!ring->lag) ring->lag = &ring->srs->lagrange_table(N, rg.logN, rg.omega, rg.tw_inv, rg.n_inv);
-            ctx->partials.ensure((size_t)4 * m);
-            launch_lb<64, 8>(ctx->stream, Dim3(4, m), 64, witness_commit_smem(ring->lag->geom.W, 64), WitnessCommitBody(), (const G1Affine*)ring->lag->table.p, ring->lag->geom, rg, (const ProofState*)sc.st.p,
-                   ctx->partials.p);
-            launch_commit_finish(ctx->stream, (const G1*)ctx->partials.p, 1u, 4 * m, sc.res.p);
-        }
-        // column order (b, accx, accy, accip) -> payload slots (0, 2, 3, 1)
-        launch(ctx->stream, Dim3((4 * m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)sc.res.p, 4u, 0x01030200u, sc.st.p, m);
-        pt.mark(ctx, 5);
-        launch(ctx->stream, Dim3(pb), tb, 0, Transcript1Body(), sc.st.p, m);
-        if (overlap_intt) ctx->join_side2();
-        pt.mark(ctx, 3);
-        if (!large) {
-            launch(ctx->stream, Dim3(16, m), nthr, ntt_smem, WitnessLdeBody(), rg, (const ProofState*)sc.st.p, (const Fr*)sc.wit_coef.p, sc.lde.p);
-        } else {
-            launch(ctx->stream, Dim3((N + 127) / 128, 4, 4 * m), 128, 0, CosetTwistBody(), N, rg.w4, (const Fr*)sc.wit_coef.p, sc.lde.p);
-            ntt_device(ctx, *big_plan, sc.lde.p, sc.lde.p, 16 * (size_t)m, false, sc.ntt_tmp);
-        }
-        launch(ctx->stream, Dim3((4 * N + 127) / 128, m), 128, 0, ConstraintBody(), rg, (const ProofState*)sc.st.p, (const Fr*)sc.lde.p, sc.agg.p);
-        if (!large) {
-            launch(ctx->stream, Dim3(4, m), nthr, ntt_smem, QuotientInttBody(), rg, sc.agg.p);
-        } else {
-            ntt_device(ctx, *big_plan, sc.agg.p, sc.agg.p, 4 * (size_t)m, true, sc.ntt_tmp);
-            launch(ctx->stream, Dim3((N + 127) / 128, 4, m), 128, 0, CosetUntwistBody(), N, rg.w4inv, sc.agg.p);
-        }
-        launch(ctx->stream, Dim3((N + 127) / 128, m), 128, 0, QuotientCombineBody(), rg, (const Fr*)sc.agg.p, sc.cagg.p);
-        launch(ctx->stream, Dim3((qlen + 127) / 128, m), 128, 0, QuotientFoldBody(), rg, (const Fr*)sc.cagg.p, sc.quot.p, qlen);
-        pt.mark(ctx, 2);
-        commit_device(ctx, ring->srs, sc.quot.p, qlen, qlen, m, sc.res.p);
-        launch(ctx->stream, Dim3((m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)sc.res.p, 1u, 0x04u, sc.st.p, m);
-        pt.mark(ctx, 5);
-        launch(ctx->stream, Dim3(pb), tb, 0, Transcript2Body(), sc.st.p, m);
-        pt.mark(ctx, 4);
-        launch(ctx->stream, Dim3(7, m), 128, 128 * sizeof(Fr), EvalBody(), rg, sc.st.p, (const Fr*)sc.wit_coef.p);
-        launch(ctx->stream, Dim3((N + 127) / 128, m), 128, 0, LinPolyBody(), rg, (const ProofState*)sc.st.p, (const Fr*)sc.wit_coef.p, sc.lin.p);
-        launch(ctx->stream, Dim3(1, m), 128, 128 * sizeof(Fr), LinEvalBody(), rg, sc.st.p, (const Fr*)sc.lin.p);
-        pt.mark(ctx, 5);
-        launch(ctx->stream, Dim3(pb), tb, 0, Transcript3Body(), sc.st.p, m);
-        pt.mark(ctx, 4);
-        launch(ctx->stream, Dim3((qlen + 127) / 128, m), 128, 0, AggOpenBody(), rg, (const ProofState*)sc.st.p, (const Fr*)sc.wit_coef.p, (const Fr*)sc.quot.p, qlen, sc.aggopen.p);
-        launch(ctx->stream, Dim3(2, m), 256, synthetic_div_smem(256), OpenQuotientsBody(), rg, (const ProofState*)sc.st.p, sc.aggopen.p, qlen, sc.lin.p);
-        pt.mark(ctx, 2);
-        commit_device_pair(ctx, ring->srs, sc.aggopen.p, qlen, 3 * N, sc.lin.p, N, N - 1, m, sc.res.p);
-        launch(ctx->stream, Dim3((m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)sc.res.p, 1u, 0x05u, sc.st.p, m);
-        launch(ctx->stream, Dim3((m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)(sc.res.p + m), 1u, 0x06u, sc.st.p, m);
-        pt.mark(ctx, 5);
-        ctx->join_side();
-        launch(ctx->stream, Dim3(pb), tb, 0, FinalizeBody(), (const ProofState*)sc.st.p, m, sc.out.p, sc.status.p);
-        pt.mark(ctx, 8);
-        dev_zero(ctx->stream, sc.in.p, m * sizeof(ProveInput));  // secret keys do not outlive the pass on the device
-        d2h(ctx->stream, proofs784 + 784 * base, sc.out.p, (size_t)m * 784);
-        d2h(ctx->stream, status + base, sc.status.p, (size_t)m * sizeof(uint32_t));
-        pt.mark(ctx, -1);
-        stream_sync(ctx->stream);
-        pt.collect(ctx);
-    }
-    {  // ... nor in the host staging buffer (volatile: the stores must not be optimised away)
-        volatile uint8_t* w = (volatile uint8_t*)hin.data();
-        for (size_t i = 0; i < hin.size() * sizeof(ProveInput); i++) w[i] = 0;
-    }
+    // rings of one domain size share its roots of unity: a pass takes the twiddles and coset powers from one of them
+    for (size_t k = 0; k < n_rings; k++)
+        for (size_t j = 0; j < k; j++)
+            if (rings[j]->dev.N == rings[k]->dev.N && (rings[j]->dev.omega != rings[k]->dev.omega || rings[j]->radix_omega != rings[k]->radix_omega))
+                throw Error(DR_EINVAL, "rings of one domain size must share omega and radix_omega");
+    for (size_t i = 0; i < n; i++)
+        if (ring_index[i] >= n_rings) throw Error(DR_EINVAL, "ring index out of range");
+    ctx->activate();
+    if (!n) return DR_OK;
+    std::vector<RingTab> table(n_rings);
+    for (size_t k = 0; k < n_rings; k++) table[k] = rings[k]->tab;
+    DevBuf<RingTab> dtable(n_rings);
+    h2d(ctx->stream, dtable.p, table.data(), n_rings * sizeof(RingTab));
+    ring_prove(ctx, rings, dtable.p, ring_index, n, blob, alpha_off, alpha_len, ad_off, ad_len, secret_keys32, producer_index, zk_rows, proofs784, status);
     DR_API_END
 }
 

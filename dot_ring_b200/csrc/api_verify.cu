@@ -306,11 +306,6 @@ struct RingVerifier {
     uint8_t g1_0_be96[96];
 };
 
-static bool same_suite(const SuiteDev& a, const SuiteDev& b) {
-    return a.suite_id_len == b.suite_id_len && !memcmp(a.suite_id, b.suite_id, a.suite_id_len) && a.dst_len == b.dst_len && !memcmp(a.dst, b.dst, a.dst_len) &&
-           a.hash_kind == b.hash_kind && a.generator == b.generator && a.blinding_base == b.blinding_base;
-}
-
 }  // namespace dr
 
 using namespace dr;

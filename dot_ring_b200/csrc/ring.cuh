@@ -25,12 +25,10 @@ namespace dr {
 
 constexpr uint32_t SCALAR_BITS = 253;
 
-// Per-ring constants and device tables, passed to kernels by value.
+// What a pass reads that depends only on the domain size N or on the suite, passed to kernels by value.  The ring's own data
+// (keys, fixed columns, transcript prefix) is in RingTab, so that one pass can prove items of several rings.
 struct RingDev {
-    uint32_t N, logN, max_ring, last;  // last = N - 4 (last accumulator row)
-    const TEAffine* nm;                // [N]   PK || padding || 2^i B || 4 x (0,0)
-    const Fr* fixed_coef;              // [3][N]   px, py, s  coefficients
-    const Fr* fixed_lde;               // [6][4N]  px, py, s, L_0, L_last, (x - w^last): coset layout
+    uint32_t N, logN, last;            // last = N - 4 (last accumulator row)
     const Fr* tw_fwd;                  // [N/2] w^k
     const Fr* tw_inv;                  // [N/2] w^-k
     const Fr* w4;                      // [4N]  w4^k
@@ -48,6 +46,16 @@ struct RingDev {
     uint32_t dst_len;
     uint8_t dst[64];  // hash-to-curve DST (without the trailing length byte)
     uint32_t hash_kind;  // 0: SHA-512 suite (XMD h2c, counter-mode squeeze), 1: SHAKE128 suite (XOF h2c, direct squeeze)
+};
+
+// One ring's device tables: an array of these is indexed by ProofState::ring.  The kernels that read them run one proof per
+// block or per warp and resolve the entry there, before any branch on per-thread data.
+struct RingTab {
+    const TEAffine* nm;      // [N]   PK || padding || 2^i B || 4 x (0,0)
+    const Fr* fixed_coef;    // [3][N]   px, py, s  coefficients
+    const Fr* fixed_lde;     // [6][4N]  px, py, s, L_0, L_last, (x - w^last): coset layout
+    const Shake128* prefix;  // ring transcript after the verifier key (root.py:54-71)
+    uint32_t max_ring;
 };
 
 // The suite's transcript hash (primitives.py:26-55).  Absorb-only until squeezed; squeezing never disturbs the state, so a
@@ -95,6 +103,7 @@ struct VrfHash {
 struct ProofState {
     uint32_t k;         // producer index
     uint32_t status;    // 0 ok; 1 = producer key does not match secret key / ring row
+    uint32_t ring;      // entry of the call's RingTab array
     uint32_t t[8];      // Pedersen blinding factor, raw limbs
     Fr zk[12];          // blinding rows: b, accx, accy, accip (3 each), Montgomery
     TEAffine a0;        // seed + PK_k
@@ -115,7 +124,7 @@ struct ProofState {
 struct ProveInput {  // host-packed per proof
     uint32_t alpha_off, alpha_len, ad_off, ad_len;
     uint32_t k;
-    uint32_t pad;
+    uint32_t ring;  // entry of the call's RingTab array
     uint8_t sk[32];
 };
 
@@ -353,7 +362,7 @@ struct TeFixedTableBody {
 // table windows.  What remains on one lane: the affine conversions, the SHA-512 / SHAKE transcripts and the point encodings.
 DR_HD size_t pedersen_start_smem(uint32_t threads) { return (threads / COOP_LANES) * (sizeof(TeCoopState) + 2 * sizeof(TEAffine)); }
 struct PedersenStartBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const ProveInput* in, const uint8_t* blob, ProofState* st, uint32_t count) const {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProveInput* in, const uint8_t* blob, ProofState* st, uint32_t count) const {
         const uint32_t items = ctx.nthreads / COOP_LANES;
         TeCoopState* cs = (TeCoopState*)ctx.smem;
         TEAffine* maps = (TEAffine*)(cs + items);  // [items][2]
@@ -423,9 +432,12 @@ struct PedersenStartBody {
             if (s.live) te_mul_fixed_coop_partial(t % COOP_LANES, rg.b_tab, s.k, s.part);
         }
         DR_BLOCK_SYNC();
-        // F. blinded key; ring-membership check of the producer key
+        // F. blinded key; ring-membership check of the producer key against the item's ring
         DR_THREAD_LOOP(t, ctx) {
             const uint32_t item = t / COOP_LANES, lane = t % COOP_LANES, p = ctx.bx * items + item;
+            const uint32_t ring = p < count ? in[p].ring : 0u;
+            const TEAffine* nm = tab[ring].nm;
+            const uint32_t max_ring = tab[ring].max_ring;
             if (p < count && lane == 0) {
                 TeCoopState& s = cs[item];
                 ProofState& ps = st[p];
@@ -434,9 +446,10 @@ struct PedersenStartBody {
                 TEAffine blinded;
                 pedersen_begin_blind(pk, te_fold_fixed_coop(s.part), ps.pedersen, blinded, ps.vrf_tr);
                 ps.k = pi.k;
+                ps.ring = ring;
                 ps.relation = blinded;
                 // producer_key must be pk(sk) and sit at row k of the ring (vrf/ring/vrf.py:196-197, members.py:71-81)
-                ps.status = (pi.k < rg.max_ring && rg.nm[pi.k] == pk) ? 0u : 1u;
+                ps.status = (pi.k < max_ring && nm[pi.k] == pk) ? 0u : 1u;
             }
         }
     }
@@ -464,20 +477,25 @@ constexpr uint32_t WIT_LANES = 32, WIT_ROWS = 8;
 static_assert(WIT_LANES * WIT_ROWS >= SCALAR_BITS, "every bit row needs a lane");
 DR_HD size_t witness_coop_smem(uint32_t threads) { return (size_t)2 * threads * sizeof(TEExt); }
 struct WitnessBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, ProofState* st, uint32_t count, const Shake128* prefix) const {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, ProofState* st, uint32_t count) const {
         TEExt* sm = (TEExt*)ctx.smem;  // two scan buffers of nthreads entries
         const uint32_t T = ctx.nthreads, ppb = T / WIT_LANES;
         auto bit_of = [](const ProofState& ps, uint32_t j) { return (ps.t[j >> 5] >> (j & 31)) & 1u; };
+        // the proof's ring, resolved per warp (one proof per warp) before any branch on lane data
+        auto ring_of = [&](uint32_t p) -> const RingTab& { return tab[p < count ? st[p].ring : 0u]; };
         // 1. lane totals (lane 0 starts from a0 = seed + PK_k)
         DR_THREAD_LOOP(t, ctx) {
             const uint32_t lane = t % WIT_LANES, p = ctx.bx * ppb + t / WIT_LANES;
+            const RingTab& rt = ring_of(p);
+            const TEAffine* nm = rt.nm;
+            const uint32_t max_ring = rt.max_ring;
             TEExt acc = TEExt::identity();
             if (p < count) {
                 const ProofState& ps = st[p];
-                if (lane == 0) acc = te_add(TEExt::from_affine(rg.seed), TEExt::from_affine(rg.nm[ps.k < rg.max_ring ? ps.k : 0]));
+                if (lane == 0) acc = te_add(TEExt::from_affine(rg.seed), TEExt::from_affine(nm[ps.k < max_ring ? ps.k : 0]));
 #pragma unroll 1
                 for (uint32_t j = lane * WIT_ROWS; j < (lane + 1) * WIT_ROWS && j < SCALAR_BITS; j++)
-                    if (bit_of(ps, j)) acc = te_add(acc, TEExt::from_affine(rg.nm[rg.max_ring + j]));
+                    if (bit_of(ps, j)) acc = te_add(acc, TEExt::from_affine(nm[max_ring + j]));
             }
             sm[t] = acc;
         }
@@ -497,16 +515,19 @@ struct WitnessBody {
         // 3. walk the lane's rows from the sum of everything before them; affine through one inversion per lane
         DR_THREAD_LOOP(t, ctx) {
             const uint32_t lane = t % WIT_LANES, p = ctx.bx * ppb + t / WIT_LANES;
+            const RingTab& rt = ring_of(p);
+            const TEAffine* nm = rt.nm;
+            const uint32_t max_ring = rt.max_ring;
             if (p < count) {
                 ProofState& ps = st[p];
-                const TEExt a0 = te_add(TEExt::from_affine(rg.seed), TEExt::from_affine(rg.nm[ps.k < rg.max_ring ? ps.k : 0]));
+                const TEExt a0 = te_add(TEExt::from_affine(rg.seed), TEExt::from_affine(nm[ps.k < max_ring ? ps.k : 0]));
                 TEExt acc = lane ? sm[cur * T + t - 1] : a0;
                 Fr zs[WIT_ROWS], pre[WIT_ROWS];
                 Fr run = lane ? Fr::one() : a0.Z;
                 uint32_t rows = 0;
 #pragma unroll 1
                 for (uint32_t j = lane * WIT_ROWS; j < (lane + 1) * WIT_ROWS && j < SCALAR_BITS; j++, rows++) {
-                    if (bit_of(ps, j)) acc = te_add(acc, TEExt::from_affine(rg.nm[rg.max_ring + j]));
+                    if (bit_of(ps, j)) acc = te_add(acc, TEExt::from_affine(nm[max_ring + j]));
                     ps.s[j] = {acc.X, acc.Y};  // projective for now
                     zs[rows] = acc.Z;
                     pre[rows] = run;
@@ -527,6 +548,7 @@ struct WitnessBody {
         // 4. consistency check and transcript start, one lane per proof
         DR_THREAD_LOOP(t, ctx) {
             const uint32_t lane = t % WIT_LANES, p = ctx.bx * ppb + t / WIT_LANES;
+            const Shake128* prefix = ring_of(p).prefix;
             if (p < count && lane == 0) {
                 ProofState& ps = st[p];
                 // the accumulator must end at seed + relation (proof_builder.py:66-69)
@@ -544,13 +566,14 @@ struct WitnessBody {
     }
 };
 
-// Column synthesis (columns.py:111-146 + 43-53): value of witness column `col` at row `row`.
-DR_HD Fr witness_eval(const RingDev& rg, const ProofState& ps, uint32_t col, uint32_t row) {
+// Column synthesis (columns.py:111-146 + 43-53): value of witness column `col` at row `row`.  `max_ring` is the proof's ring's
+// (RingTab::max_ring), which the caller resolves once per block.
+DR_HD Fr witness_eval(const RingDev& rg, uint32_t max_ring, const ProofState& ps, uint32_t col, uint32_t row) {
     const uint32_t N = rg.N;
     if (row >= N - 3) return ps.zk[3 * col + (row - (N - 3))];
     if (col == COL_B) {
-        if (row < rg.max_ring) return row == ps.k ? Fr::one() : Fr::zero();
-        uint32_t j = row - rg.max_ring;
+        if (row < max_ring) return row == ps.k ? Fr::one() : Fr::zero();
+        uint32_t j = row - max_ring;
         if (j < SCALAR_BITS && ((ps.t[j >> 5] >> (j & 31)) & 1)) return Fr::one();
         return Fr::zero();
     }
@@ -558,12 +581,12 @@ DR_HD Fr witness_eval(const RingDev& rg, const ProofState& ps, uint32_t col, uin
     const TEAffine* pt;
     if (row <= ps.k)
         pt = &rg.seed;
-    else if (row <= rg.max_ring)
+    else if (row <= max_ring)
         pt = &ps.a0;
     else {
         // max_ring_size below the domain's capacity leaves more than 253 blinding-base rows (members.py:46-51); the b column
         // is zero there (columns.py:111-124), so the accumulator keeps its final value
-        uint32_t j = row - rg.max_ring - 1;
+        uint32_t j = row - max_ring - 1;
         pt = &ps.s[j < SCALAR_BITS ? j : SCALAR_BITS - 1];
     }
     return col == COL_ACCX ? pt->x : pt->y;
@@ -571,13 +594,14 @@ DR_HD Fr witness_eval(const RingDev& rg, const ProofState& ps, uint32_t col, uin
 
 // ---- C. witness interpolation: grid (4 columns, proofs) ------------------------------------------------
 struct WitnessInttBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const ProofState* st, Fr* wit_coef) const {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProofState* st, Fr* wit_coef) const {
         const ProofState& ps = st[ctx.by];
+        const uint32_t max_ring = tab[ps.ring].max_ring;
         uint32_t col = ctx.bx;
         Fr* dst = wit_coef + ((size_t)ctx.by * 4 + col) * rg.N;
         Fr ninv = rg.n_inv;
         ntt_block(
-            ctx, rg.N, rg.logN, rg.tw_inv, [&](uint32_t r) { return witness_eval(rg, ps, col, r); }, [&](uint32_t k, const Fr& v) { dst[k] = v * ninv; });
+            ctx, rg.N, rg.logN, rg.tw_inv, [&](uint32_t r) { return witness_eval(rg, max_ring, ps, col, r); }, [&](uint32_t k, const Fr& v) { dst[k] = v * ninv; });
     }
 };
 
@@ -596,7 +620,7 @@ constexpr uint32_t WC_MAX_STEPS = 272;  // <= 1 (row k) + 253 (bit rows) + 3 bli
 DR_HD size_t witness_commit_steps_bytes(uint32_t W) { return (((size_t)WC_MAX_STEPS * (2 + W + 1 + 2) * sizeof(int16_t) + 16 + 15) / 16) * 16; }
 DR_HD size_t witness_commit_smem(uint32_t W, uint32_t threads) { return witness_commit_steps_bytes(W) + threads * sizeof(G1); }
 struct WitnessCommitBody {
-    DR_HD void operator()(const BlockCtx& ctx, const G1Affine* table, TableGeom g, RingDev rg, const ProofState* st, G1* out) const {
+    DR_HD void operator()(const BlockCtx& ctx, const G1Affine* table, TableGeom g, RingDev rg, const RingTab* tab, const ProofState* st, G1* out) const {
         int16_t* steps = (int16_t*)ctx.smem;
         const uint32_t stride = 2 + g.W;
         int16_t* rows = steps + (size_t)WC_MAX_STEPS * stride;
@@ -604,6 +628,7 @@ struct WitnessCommitBody {
         uint32_t* counters = (uint32_t*)(units + 2 * WC_MAX_STEPS);  // rows found, full steps, unit steps
         G1* sm = (G1*)(ctx.smem + witness_commit_steps_bytes(g.W));
         const ProofState& ps = st[ctx.by];
+        const uint32_t max_ring = tab[ps.ring].max_ring;
         const uint32_t col = ctx.bx, N = rg.N;
         DR_THREAD_LOOP(t, ctx) {
             if (t < 3) counters[t] = 0;
@@ -613,8 +638,8 @@ struct WitnessCommitBody {
         DR_THREAD_LOOP(t, ctx) {
 #pragma unroll 1
             for (uint32_t j = 1 + t; j <= N; j += ctx.nthreads) {
-                Fr d = witness_eval(rg, ps, col, j - 1);
-                if (j < N) d = d - witness_eval(rg, ps, col, j);
+                Fr d = witness_eval(rg, max_ring, ps, col, j - 1);
+                if (j < N) d = d - witness_eval(rg, max_ring, ps, col, j);
                 if (d.is_zero()) continue;
                 uint32_t slot = atomic_add_u32(&counters[0], 1u);
                 if (slot < WC_MAX_STEPS) rows[slot] = (int16_t)j;  // base S_j is table point j - 1 (N <= 4096)
@@ -628,8 +653,8 @@ struct WitnessCommitBody {
 #pragma unroll 1
             for (uint32_t slot = t; slot < found; slot += ctx.nthreads) {
                 const uint32_t j = (uint32_t)(uint16_t)rows[slot];
-                Fr d = witness_eval(rg, ps, col, j - 1);
-                if (j < N) d = d - witness_eval(rg, ps, col, j);
+                Fr d = witness_eval(rg, max_ring, ps, col, j - 1);
+                if (j < N) d = d - witness_eval(rg, max_ring, ps, col, j);
                 Fr kc = d.from_mont(), nk = d.neg().from_mont();
                 bool flip = (nk.v[1] | nk.v[2] | nk.v[3] | nk.v[4] | nk.v[5] | nk.v[6] | nk.v[7]) == 0;  // use the shorter of d, -d
                 if (flip) kc = nk;
@@ -722,14 +747,15 @@ struct Transcript1Body {
 
 // ---- F. 4x low-degree extension of the witness columns: grid (16 = 4 cosets x 4 columns, proofs) ---------
 struct WitnessLdeBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const ProofState* st, const Fr* wit_coef, Fr* lde) const {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProofState* st, const Fr* wit_coef, Fr* lde) const {
         uint32_t col = ctx.bx & 3, j = ctx.bx >> 2;
         const Fr* src = wit_coef + ((size_t)ctx.by * 4 + col) * rg.N;
         Fr* dst = lde + (((size_t)ctx.by * 4 + col) * 4 + j) * rg.N;
         const uint32_t mask = 4 * rg.N - 1;
         if (j == 0) {  // coset 0 is the N-domain itself: the column's own evaluations, no transform needed
             const ProofState& ps = st[ctx.by];
-            DR_STRIDE_LOOP(i, rg.N, ctx) { dst[i] = witness_eval(rg, ps, col, i); }
+            const uint32_t max_ring = tab[ps.ring].max_ring;
+            DR_STRIDE_LOOP(i, rg.N, ctx) { dst[i] = witness_eval(rg, max_ring, ps, col, i); }
             return;
         }
         ntt_block(
@@ -753,11 +779,12 @@ struct PlainLdeBody {
 // The transform no longer fits one CTA, so the fused loaders / storers above become element-wise passes around the
 // two-pass NTT of ntt.cuh: materialise the witness evaluations, pre-twist the cosets, untwist after the inverse transform.
 struct WitnessEvalBody {  // grid (ceil(N / threads), 4 columns, proofs): out[(p*4 + col)*N + r] = column value at row r
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const ProofState* st, Fr* out) const {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProofState* st, Fr* out) const {
         const ProofState& ps = st[ctx.bz];
+        const uint32_t max_ring = tab[ps.ring].max_ring;
         DR_THREAD_LOOP(t, ctx) {
             uint32_t r = ctx.bx * ctx.nthreads + t;
-            if (r < rg.N) out[((size_t)ctx.bz * 4 + ctx.by) * rg.N + r] = witness_eval(rg, ps, ctx.by, r);
+            if (r < rg.N) out[((size_t)ctx.bz * 4 + ctx.by) * rg.N + r] = witness_eval(rg, max_ring, ps, ctx.by, r);
         }
     }
 };
@@ -789,13 +816,13 @@ struct CosetUntwistBody {  // grid (ceil(N / threads), 4 cosets, vectors): buf[(
 // ---- G. constraints c1..c7 and their alpha-aggregation on the 4N domain (constraints.py:64-151,
 //         proof_builder.py:165-179): grid (ceil(4N / threads), proofs) ----------------------------------------
 struct ConstraintBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const ProofState* st, const Fr* lde, Fr* agg) const {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProofState* st, const Fr* lde, Fr* agg) const {
         const ProofState& ps = st[ctx.by];
         const uint32_t N = rg.N, N4 = 4 * rg.N;
         const Fr* w = lde + (size_t)ctx.by * 4 * N4;
         const Fr *b4 = w + COL_B * N4, *ax4 = w + COL_ACCX * N4, *ay4 = w + COL_ACCY * N4, *aip4 = w + COL_ACCIP * N4;
-        const Fr *px4 = rg.fixed_lde, *py4 = rg.fixed_lde + N4, *s4 = rg.fixed_lde + 2 * N4, *l0 = rg.fixed_lde + 3 * N4, *ln = rg.fixed_lde + 4 * N4,
-                 *nl = rg.fixed_lde + 5 * N4;
+        const Fr* fl = tab[ps.ring].fixed_lde;
+        const Fr *px4 = fl, *py4 = fl + N4, *s4 = fl + 2 * N4, *l0 = fl + 3 * N4, *ln = fl + 4 * N4, *nl = fl + 5 * N4;
         Fr* out = agg + (size_t)ctx.by * N4;
         const TEAffine rps = ps.s[SCALAR_BITS - 1];  // result + seed
         DR_THREAD_LOOP(t, ctx) {
@@ -952,15 +979,16 @@ DR_HD Fr block_poly_eval(const BlockCtx& ctx, const Fr* poly, uint32_t n, const 
 // ---- K. evaluations at zeta (proof_builder.py:243-267): grid (7, proofs) ----------------------------------------
 // slot order = payload order: px, py, s, b, accip, accx, accy
 struct EvalBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, ProofState* st, const Fr* wit_coef) const {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, ProofState* st, const Fr* wit_coef) const {
         ProofState& ps = st[ctx.by];
         uint32_t slot = ctx.bx;
         const Fr* poly;
         const Fr* wc = wit_coef + (size_t)ctx.by * 4 * rg.N;
+        const Fr* fc = tab[ps.ring].fixed_coef;
         switch (slot) {
-            case 0: poly = rg.fixed_coef; break;
-            case 1: poly = rg.fixed_coef + rg.N; break;
-            case 2: poly = rg.fixed_coef + 2 * rg.N; break;
+            case 0: poly = fc; break;
+            case 1: poly = fc + rg.N; break;
+            case 2: poly = fc + 2 * rg.N; break;
             case 3: poly = wc + COL_B * rg.N; break;
             case 4: poly = wc + COL_ACCIP * rg.N; break;
             case 5: poly = wc + COL_ACCX * rg.N; break;
@@ -1035,8 +1063,10 @@ struct Transcript3Body {
 
 // ---- M. aggregated opening polynomial (proof_builder.py:288-315): grid (ceil((3N+1)/threads), proofs) ------------
 struct AggOpenBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const ProofState* st, const Fr* wit_coef, const Fr* quot, uint32_t qstride, Fr* aggopen) const {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProofState* st, const Fr* wit_coef, const Fr* quot, uint32_t qstride,
+                          Fr* aggopen) const {
         const ProofState& ps = st[ctx.by];
+        const Fr* fc = tab[ps.ring].fixed_coef;
         const uint32_t N = rg.N;
         const Fr* wc = wit_coef + (size_t)ctx.by * 4 * N;
         const Fr* q = quot + (size_t)ctx.by * qstride;
@@ -1046,7 +1076,7 @@ struct AggOpenBody {
             if (k < 3 * N + 1) {
                 Fr acc = q[k] * ps.nu[7];
                 if (k < N) {
-                    acc = acc + rg.fixed_coef[k] * ps.nu[0] + rg.fixed_coef[N + k] * ps.nu[1] + rg.fixed_coef[2 * N + k] * ps.nu[2] +
+                    acc = acc + fc[k] * ps.nu[0] + fc[N + k] * ps.nu[1] + fc[2 * N + k] * ps.nu[2] +
                           wc[COL_B * N + k] * ps.nu[3] + wc[COL_ACCIP * N + k] * ps.nu[4] + wc[COL_ACCX * N + k] * ps.nu[5] + wc[COL_ACCY * N + k] * ps.nu[6];
                 }
                 dst[k] = acc;

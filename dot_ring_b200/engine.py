@@ -250,6 +250,22 @@ class PooledRingNative:
         self.pool.map(lambda i: self.replicas[i].prove_packed(pk, bounds[i][0], bounds[i][1]), range(len(bounds)))
         return _native.NativeRing.unpack_proofs(pk)
 
+    @staticmethod
+    def prove_multi(rings: list["PooledRingNative"], index, alphas, ads, secret_keys, producer_index, zk_rows=None):
+        """Item i against rings[index[i]] (`NativeRing.prove_multi`): the batch is packed once and sharded contiguously; device d
+        proves its shard against its own replicas of the rings.  Every ring must be built on the same pool."""
+        if not rings:
+            if len(alphas):
+                raise ValueError("at least one ring is required")
+            return [], []
+        pool = rings[0].pool
+        if any(not isinstance(r, PooledRingNative) or r.pool is not pool for r in rings):
+            raise ValueError("rings of one call must be built on the same EnginePool")
+        pk = _native.NativeRing.pack_prove_inputs(alphas, ads, secret_keys, producer_index, zk_rows, ring_index=index)
+        bounds = pool.shard_bounds(pk["n"], len(pool))
+        pool.map(lambda i: _native.NativeRing.prove_multi_packed([r.replicas[i] for r in rings], pk, bounds[i][0], bounds[i][1]), range(len(bounds)))
+        return _native.NativeRing.unpack_proofs(pk)
+
     def verify_batch(self, inputs, ads, proofs, coeffs, aggregate: bool = False):
         """Per-item mode: shards are independent.  Aggregated mode (`RingVRF.batch_verify`): every device folds its shard into
         its own random-linear-combination check (its slice of the caller's coefficients) and the batch is accepted iff every

@@ -397,6 +397,22 @@ class RingVRF(VRF):
         return cls.prove_batch([alpha], [additional_data], secret_key, producer_key, ring, ring_root, salt=salt, zk_rows=zk_rows)[0]
 
     @classmethod
+    def _signer_rows(cls, ring: Ring, pairs) -> dict[bytes, int]:
+        """{producer key: its row in `ring`} for a set of (secret key, producer key) pairs.  vrf.py:196-197: producer_key must be
+        pk(sk) -- one device scalar multiplication per distinct key pair, remembered per ring under a digest of the pair (no secret
+        key outlives the call in the cache); ValueError on a pair that does not match or a key that is not in the ring."""
+        cache = ring.__dict__.setdefault("_signer_rows", {})
+        tag = lambda sk, pk: hashlib.blake2b(sk + pk, digest_size=16).digest()  # noqa: E731
+        distinct = sorted(p for p in pairs if tag(*p) not in cache)
+        if distinct:
+            derived = cls.cv.public_keys_from_secrets([sk for sk, _ in distinct])
+            for (sk, pk), got in zip(distinct, derived):
+                if pk != got:
+                    raise ValueError("producer_key does not match secret_key")
+                cache[tag(sk, pk)] = ring.index_of(pk)
+        return {pk: cache[tag(sk, pk)] for sk, pk in pairs}
+
+    @classmethod
     def prove_batch(
         cls,
         alphas: Sequence[bytes],
@@ -417,21 +433,9 @@ class RingVRF(VRF):
         pks = [bytes(producer_key)] * n if isinstance(producer_key, (bytes, bytearray)) else [bytes(p) for p in producer_key]
         if len(sks) != n or len(pks) != n:
             raise ValueError("secret_key / producer_key must be single values or one per item")
-        # vrf.py:196-197: producer_key must be pk(sk) -- one device scalar multiplication per distinct key pair, remembered per ring
-        # under a digest of the pair (no secret key outlives the call in the cache)
-        cache = ring.__dict__.setdefault("_signer_rows", {})
-        tag = lambda sk, pk: hashlib.blake2b(sk + pk, digest_size=16).digest()  # noqa: E731
-        pairs = set(zip(sks, pks))
-        distinct = sorted(p for p in pairs if tag(*p) not in cache)
-        if distinct:
-            derived = cls.cv.public_keys_from_secrets([sk for sk, _ in distinct])
-            for (sk, pk), got in zip(distinct, derived):
-                if pk != got:
-                    raise ValueError("producer_key does not match secret_key")
-                cache[tag(sk, pk)] = ring.index_of(pk)
+        index = cls._signer_rows(ring, set(zip(sks, pks)))
         if ring_root is not None and ring_root.encode() != RingRoot.from_ring(ring).encode():
             raise ValueError("ring_root does not match ring")
-        index = {pk: cache[tag(sk, pk)] for sk, pk in pairs}
         if zk_rows is None and not ring.params.test_vectors:
             prime = ring.params.prime
             zk_rows = [secrets.randbelow(prime) for _ in range(12 * n)]
@@ -439,6 +443,71 @@ class RingVRF(VRF):
             zk_rows = None
         msgs = [bytes(salt) + bytes(a) for a in alphas]
         proofs, status = ring.native.prove_batch(msgs, [bytes(a) for a in additional_data], sks, [index[pk] for pk in pks], zk_rows)
+        if any(status):
+            raise ValueError("producer_key does not match secret_key")
+        if as_bytes:
+            return proofs
+        return [cls._from_bytes_trusted(p) for p in proofs]
+
+    @classmethod
+    def prove_multi(
+        cls,
+        alphas: Sequence[bytes],
+        additional_data: Sequence[bytes],
+        secret_keys: Sequence[bytes],
+        producer_keys: Sequence[bytes],
+        rings: Sequence[Ring],
+        ring_index: Sequence[int],
+        salt: bytes = b"",
+        zk_rows: Sequence[int] | bytes | None = None,
+        as_bytes: bool = False,
+    ):
+        """Prove item i against ``rings[ring_index[i]]``, every ring in one device pass; semantically a loop over ``prove``.
+
+        The rings share the suite and the engine (one :class:`Engine`, or one :class:`EnginePool` whose devices each take a
+        contiguous shard); their domain sizes may differ.  Blinding rows as in ``prove_batch``: 12 per item, drawn fresh unless
+        ``zk_rows`` gives them, and zeros for items whose ring has ``test_vectors=True``."""
+        from . import _native
+        from .engine import PooledRingNative
+
+        n = len(alphas)
+        rings = list(rings)
+        index = [int(k) for k in ring_index]
+        sks, pks = [bytes(s) for s in secret_keys], [bytes(p) for p in producer_keys]
+        if not (len(additional_data) == len(sks) == len(pks) == len(index) == n):
+            raise ValueError("alphas, additional_data, secret_keys, producer_keys and ring_index must have the same length")
+        if any(not 0 <= k < len(rings) for k in index):
+            raise ValueError("ring index out of range")
+        if n == 0:
+            return []
+        rows = [0] * n
+        for k in sorted(set(index)):
+            items = [i for i in range(n) if index[i] == k]
+            found = cls._signer_rows(rings[k], {(sks[i], pks[i]) for i in items})
+            for i in items:
+                rows[i] = found[pks[i]]
+        zeroed = [rings[k].params.test_vectors for k in index]
+        if all(zeroed):
+            zk = None
+        else:
+            if zk_rows is None:
+                prime = rings[index[zeroed.index(False)]].params.prime
+                zk = [0 if z else secrets.randbelow(prime) for z in zeroed for _ in range(12)]
+            else:
+                if isinstance(zk_rows, (bytes, bytearray)):
+                    if len(zk_rows) != 12 * 32 * n:
+                        raise ValueError("zk_rows must hold 12 field elements per proof")
+                    zk_rows = [int.from_bytes(zk_rows[32 * j : 32 * j + 32], "little") for j in range(12 * n)]
+                if len(zk_rows) != 12 * n:
+                    raise ValueError("zk_rows must hold 12 field elements per proof")
+                zk = [0 if zeroed[j // 12] else int(v) for j, v in enumerate(zk_rows)]
+        natives = [r.native for r in rings]
+        pooled = [isinstance(x, PooledRingNative) for x in natives]
+        if any(pooled) and not all(pooled):
+            raise ValueError("rings of one call must be built on the same engine")
+        prove = PooledRingNative.prove_multi if all(pooled) else _native.NativeRing.prove_multi
+        msgs = [bytes(salt) + bytes(a) for a in alphas]
+        proofs, status = prove(natives, index, msgs, [bytes(a) for a in additional_data], sks, rows, zk)
         if any(status):
             raise ValueError("producer_key does not match secret_key")
         if as_bytes:

@@ -175,11 +175,25 @@ int dr_ring_points(dr_ring* ring, uint8_t* out_xy64, size_t n_points);
 int dr_ring_prove_batch(dr_ctx* ctx, dr_ring* ring, size_t n, const uint8_t* blob, const uint32_t* alpha_off, const uint32_t* alpha_len,
                         const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* secret_keys32, const uint32_t* producer_index,
                         const uint8_t* zk_rows, uint8_t* proofs784, uint32_t* status);
-/* Per-phase device time of the last dr_ring_prove_batch on this ctx (ms): [0] pedersen+witness, [1] interpolate,
- * [2] commits (all MSMs), [3] LDE+constraints+quotient, [4] evaluations+openings polys, [5] transcripts+assembly. */
+/* ---- Ring VRF prove, one batch over several rings ------------------------------------------------------------
+ * Batches `RingVRF[Bandersnatch].prove` (dot_ring/vrf/ring/vrf.py:185-209) over items that belong to different rings: item i is
+ * proved against rings[ring_index[i]], and producer_index[i] is a row of that ring.  blob / offsets, secret_keys32, zk_rows (NULL:
+ * zeros), proofs784 and status[i] (non-zero when sk_i does not own that row of that ring) are as in dr_ring_prove_batch, and each
+ * proof equals dr_ring_prove_batch of its own ring on the same item.  Domain sizes may differ: items are grouped by domain size,
+ * every group runs its own equal-width passes, and the results land in the caller's order.  The rings share one pass, so a batch
+ * spread over K rings costs one call's fixed latency instead of K.  n == 0 returns DR_OK.  DR_EINVAL when a ring belongs to another
+ * context, when the rings use different dr_srs handles, differ in suite (id, DST, hash, generator, blinding base, accumulator seed,
+ * padding point) or, at one domain size, in omega / radix_omega, when an index is out of range, or when n > 0 and n_rings == 0. */
+int dr_ring_prove_multi(dr_ctx* ctx, dr_ring* const* rings, size_t n_rings, const uint32_t* ring_index, size_t n, const uint8_t* blob,
+                        const uint32_t* alpha_off, const uint32_t* alpha_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* secret_keys32,
+                        const uint32_t* producer_index, const uint8_t* zk_rows, uint8_t* proofs784, uint32_t* status);
+/* Per-phase device time of the last dr_ring_prove_batch / dr_ring_prove_multi on this ctx (ms, the whole call, summed over its
+ * domain groups): [0] pedersen+witness, [1] interpolate, [2] commits (all MSMs), [3] LDE+constraints+quotient, [4] evaluations+openings
+ * polys, [5] transcripts+assembly. */
 int dr_ring_prove_phase_ms(dr_ctx* ctx, float out[6]);
 /* Device time (CUDA events on the ctx stream, around the launches only) and launch count of the dominant kernel, the dense fixed-base
- * commit `CommitBodyT`, within the last dr_ring_prove_batch on this ctx: 3 launches per pass (quotient + two openings). */
+ * commit `CommitBodyT`, within the last dr_ring_prove_batch / dr_ring_prove_multi on this ctx (summed over its domain groups): 3
+ * launches per pass (quotient + two openings). */
 int dr_ring_prove_commit_kernel_ms(dr_ctx* ctx, float* ms, uint32_t* launches);
 /* Window width of the table the sparse witness commitments of this ring read (built at the first proof; 0 before that). */
 uint32_t dr_ring_witness_table_bits(const dr_ring* ring);
