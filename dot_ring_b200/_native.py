@@ -115,6 +115,8 @@ class Library:
         L.dr_ring_proof_verify_batch.argtypes = [c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_int, c_void_p, POINTER(c_int)]
         L.dr_ring_verify_batch.argtypes = [c_void_p, c_void_p, c_size_t] + [c_void_p] * 7 + [c_int, c_void_p, POINTER(c_int)]
         L.dr_ring_verify_set_msm_threshold.argtypes = [c_size_t]
+        L.dr_ring_roots_from_keys.argtypes = [c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]
+        L.dr_ring_root_update.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]
         L.dr_ring_verifier_create.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, POINTER(c_void_p)]
         L.dr_ring_verifier_destroy.argtypes = [c_void_p]
         L.dr_ring_verifier_destroy.restype = None
@@ -617,6 +619,40 @@ def make_ring_params(*, domain_size: int, omega: int, seed, blinding_base, gener
 
 def _xy(pt) -> bytes:
     return int(pt[0]).to_bytes(32, "little") + int(pt[1]).to_bytes(32, "little")
+
+
+def ring_roots_from_keys(srs: NativeSrs, params: RingParamsStruct, key_sets: list[list[bytes]]) -> list[bytes]:
+    """dr_ring_roots_from_keys: the 144-byte root of every key set (32-byte keys), all under one params, in one call."""
+    if any(len(k) != 32 for keys in key_sets for k in keys):
+        raise ValueError("ring keys must be 32 bytes")
+    n = len(key_sets)
+    counts = np.array([len(keys) for keys in key_sets] or [0], dtype=np.int64)
+    if counts.max() >> 32:
+        raise ValueError("ring size exceeds max supported size")
+    blob = b"".join(k for keys in key_sets for k in keys)
+    out = ctypes.create_string_buffer(144 * max(n, 1))
+    lib = srs.ctx.library
+    lib.check(lib.lib.dr_ring_roots_from_keys(srs.ctx.handle, srs.handle, ctypes.byref(params), n, blob or None, np.ctypeslib.as_ctypes(counts.astype(np.uint32)), out))
+    return [out.raw[144 * i : 144 * i + 144] for i in range(n)]
+
+
+def ring_root_update(srs: NativeSrs, params: RingParamsStruct, root144: bytes, rows: list[int], new_keys: list[bytes], old_keys: list[bytes] | None = None) -> bytes:
+    """dr_ring_root_update: the root after row rows[j] went from old_keys[j] (None: padding everywhere) to new_keys[j]."""
+    n = len(rows)
+    if len(root144) != 144:
+        raise ValueError(f"invalid ring root length: ring root must be exactly 144 bytes, got {len(root144)}")
+    if len(new_keys) != n or (old_keys is not None and len(old_keys) != n):
+        raise ValueError("one new key (and one old key, when given) per row is required")
+    if any(len(k) != 32 for k in list(new_keys) + list(old_keys or [])):
+        raise ValueError("ring keys must be 32 bytes")
+    if any(not 0 <= int(r) < 1 << 32 for r in rows):
+        raise ValueError("row out of range")
+    out = ctypes.create_string_buffer(144)
+    idx = np.ctypeslib.as_ctypes(np.array([int(r) for r in rows] or [0], dtype=np.uint32))
+    lib = srs.ctx.library
+    lib.check(lib.lib.dr_ring_root_update(srs.ctx.handle, srs.handle, ctypes.byref(params), bytes(root144), n, idx, b"".join(old_keys) if old_keys is not None else None,
+                                          b"".join(new_keys) or None, out))
+    return out.raw
 
 
 class NativeRing:

@@ -21,6 +21,36 @@ static TEAffine te_from_param(const uint8_t* xy) {
     return p;
 }
 
+// The ring's row layout: N, padding rows, and room for the 253 bit rows next to max_ring_size keys.
+static void check_ring_shape(const dr_ring_params* prm) {
+    const uint32_t N = prm->domain_size;
+    // the reference stops at 4096 (params.py:172-173); larger domains (to 2^16) run the same pipeline over the two-pass NTT
+    if (N < 512 || N > 65536 || (N & (N - 1))) throw Error(DR_EINVAL, "domain_size must be a power of two in [512, 65536]");
+    if (prm->padding_rows != 4) throw Error(DR_EINVAL, "padding_rows must be 4 to match the 3 hidden rows");
+    if (prm->max_ring_size + SCALAR_BITS + 4 > N) throw Error(DR_EINVAL, "max_ring_size exceeds supported size for this domain");
+}
+
+// omega^N == 1, omega^(N/2) != 1
+static void check_primitive_root(const Fr& omega, uint32_t logN) {
+    Fr t = omega;
+    for (uint32_t i = 0; i + 1 < logN; i++) t = t.sqr();
+    if (t == Fr::one() || t.sqr() != Fr::one()) throw Error(DR_EINVAL, "omega is not a primitive N-th root of unity");
+}
+
+// The rows of the public vector PK || padding || 2^i B || zeros (members.py:36-53) that no key sets: padding below max_ring (a key
+// overwrites its row), then the blinding-base doublings, then four zero rows.
+static std::vector<TEAffine> public_vector_rows(uint32_t N, uint32_t max_ring, const TEAffine& padding, const TEAffine& blinding_base) {
+    std::vector<TEAffine> host(N);
+    for (uint32_t i = 0; i < max_ring; i++) host[i] = padding;
+    TEExt cur = TEExt::from_affine(blinding_base);
+    for (uint32_t i = max_ring; i < N - 4; i++) {
+        host[i] = te_to_affine(cur);
+        cur = te_dbl(cur);
+    }
+    for (uint32_t i = N - 4; i < N; i++) host[i] = TEAffine{Fr::zero(), Fr::zero()};
+    return host;
+}
+
 // Per-pass device scratch.  Buffers with disjoint lifetimes share storage: the 16N-element low-degree extensions are dead once
 // the constraints are evaluated, so the combined quotient coefficients (cagg), the aggregated opening polynomial (aggopen) and
 // the linearisation polynomial (lin), all born later, live inside that block: 27 N + 1 field elements per proof instead of 35 N.
@@ -306,6 +336,120 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
     }
 }
 
+// ---- ring roots without a ring ----------------------------------------------------------------------------------------------
+// What dr_ring_roots_from_keys / dr_ring_root_update read of the params, checked as dr_ring_create checks it, and of the SRS.
+struct RootSetup {
+    uint32_t N = 0, logN = 0, max_ring = 0;
+    Fr omega;
+    TEAffine padding, blinding_base;
+};
+
+static RootSetup root_setup(Ctx* ctx, Srs* srs, const dr_ring_params* prm) {
+    check_ring_shape(prm);
+    RootSetup s;
+    s.N = prm->domain_size;
+    while ((1u << s.logN) < s.N) s.logN++;
+    s.max_ring = prm->max_ring_size;
+    s.omega = fr_from_param(prm->omega);
+    check_primitive_root(s.omega, s.logN);
+    s.padding = te_from_param(prm->padding_point);
+    s.blinding_base = te_from_param(prm->blinding_base);
+    if (srs->ctx != ctx) throw Error(DR_EINVAL, "SRS belongs to another context");
+    if (srs->n < s.N) throw Error(DR_EINVAL, "SRS too small for this domain (needs N G1 points)");
+    return s;
+}
+
+// `batch` evaluation vectors of N elements (in place: -> coefficients) -> their KZG commitments, affine, on the device
+static void commit_columns(Ctx* ctx, Srs* srs, const RootSetup& s, Fr* cols, uint32_t batch, G1Affine* out) {
+    DevBuf<Fr> ntt_tmp;
+    ntt_device(ctx, ctx->plan(s.N, s.omega), cols, cols, batch, true, ntt_tmp);
+    commit_device(ctx, srs, cols, s.N, s.N, batch, out);
+}
+
+// The root half of dr_ring_create for n_rings key vectors: every ring's px, py and the shared s in one column buffer, one batched
+// inverse NTT and one batched commitment per pass.  C_s is committed once, in the first pass.
+static void ring_roots(Ctx* ctx, Srs* srs, const RootSetup& s, size_t n_rings, const uint8_t* keys32, const std::vector<uint32_t>& key_off, uint8_t* roots144) {
+    const uint32_t N = s.N;
+    const size_t total = key_off[n_rings];
+    const std::vector<TEAffine> rows = public_vector_rows(N, s.max_ring, s.padding, s.blinding_base);
+    DevBuf<TEAffine> drows(N);
+    DevBuf<uint8_t> dkeys(total * 32);
+    DevBuf<uint32_t> doff(n_rings + 1);
+    h2d(ctx->stream, drows.p, rows.data(), N * sizeof(TEAffine));
+    h2d(ctx->stream, dkeys.p, keys32, total * 32);
+    h2d(ctx->stream, doff.p, key_off.data(), (n_rings + 1) * sizeof(uint32_t));
+    // rings per pass: two columns of N elements each, at most 1 GB of columns and 1024 rings (grid rows) at a time
+    const size_t by_memory = ((size_t)1 << 30) / (2 * (size_t)N * sizeof(Fr));
+    const size_t per_pass = std::min(n_rings, std::min<size_t>(1024, by_memory));
+    const uint32_t cap = (uint32_t)(2 * per_pass + 1);
+    DevBuf<Fr> cols((size_t)cap * N);
+    DevBuf<G1Affine> cm(cap);
+    DevBuf<uint8_t> enc(48 * (size_t)cap);
+    std::vector<uint8_t> host(48 * (size_t)cap);
+    uint8_t c_s[48];
+    for (size_t r0 = 0; r0 < n_rings; r0 += per_pass) {
+        const uint32_t m = (uint32_t)std::min(per_pass, n_rings - r0);
+        const uint32_t with_s = r0 == 0 ? 1 : 0;
+        const uint32_t batch = 2 * m + with_s;
+        launch(ctx->stream, Dim3((N + 127) / 128, m + with_s), 128, 0, RingRootColumnsBody(), (const TEAffine*)drows.p, (const uint8_t*)dkeys.p,
+               (const uint32_t*)(doff.p + r0), m, N, s.max_ring, s.padding, cols.p);
+        commit_columns(ctx, srs, s, cols.p, batch, cm.p);
+        launch(ctx->stream, Dim3((batch + 63) / 64), 64, 0, G1EncodeBody(), (const G1Affine*)cm.p, batch, (uint8_t*)nullptr, enc.p);
+        d2h(ctx->stream, host.data(), enc.p, 48 * (size_t)batch);
+        stream_sync(ctx->stream);
+        if (with_s) memcpy(c_s, host.data() + 96 * (size_t)m, 48);
+        for (uint32_t k = 0; k < m; k++) {
+            uint8_t* out = roots144 + 144 * (r0 + k);
+            memcpy(out, host.data() + 96 * (size_t)k, 96);
+            memcpy(out + 96, c_s, 48);
+        }
+    }
+}
+
+// The root is linear in the column evaluations: C_px' = C_px + commit(iNTT(dx)), dx non-zero on the changed rows only (and py
+// alike).  The selector column is committed next to the two differences: the root's C_s must equal it.
+static void ring_root_update(Ctx* ctx, Srs* srs, const RootSetup& s, const uint8_t* root144, size_t n, const uint32_t* rows, const uint8_t* old_keys32,
+                             const uint8_t* new_keys32, uint8_t* out144) {
+    G1Affine in[3];
+    for (int i = 0; i < 3; i++)
+        if (!g1_decode(in[i], root144 + 48 * i, 48)) throw Error(DR_EINVAL, "invalid BLS12-381 G1 encoding in ring root");
+    std::vector<uint8_t> seen(s.max_ring, 0);
+    for (size_t j = 0; j < n; j++) {
+        if (rows[j] >= s.max_ring) throw Error(DR_EINVAL, "row out of range: key rows lie below max_ring_size");
+        if (seen[rows[j]]++) throw Error(DR_EINVAL, "a row appears twice in one update");
+    }
+    const uint32_t N = s.N;
+    DevBuf<Fr> cols(3 * (size_t)N);  // dx | dy | s
+    DevBuf<uint8_t> dkeys(2 * n * 32);
+    DevBuf<uint32_t> drows(n);
+    dev_zero(ctx->stream, cols.p, 2 * (size_t)N * sizeof(Fr));
+    if (n) {
+        if (old_keys32) h2d(ctx->stream, dkeys.p, old_keys32, n * 32);
+        h2d(ctx->stream, dkeys.p + n * 32, new_keys32, n * 32);
+        h2d(ctx->stream, drows.p, rows, n * sizeof(uint32_t));
+        launch(ctx->stream, Dim3((uint32_t)((n + 63) / 64)), 64, 0, RootDeltaBody(), old_keys32 ? (const uint8_t*)dkeys.p : (const uint8_t*)nullptr,
+               (const uint8_t*)(dkeys.p + n * 32), (const uint32_t*)drows.p, (uint32_t)n, N, s.padding, cols.p);
+    }
+    launch(ctx->stream, Dim3((N + 127) / 128, 1), 128, 0, RingRootColumnsBody(), (const TEAffine*)nullptr, (const uint8_t*)nullptr, (const uint32_t*)nullptr, 0u, N,
+           s.max_ring, s.padding, cols.p + 2 * (size_t)N);
+    DevBuf<G1Affine> cm(3);
+    commit_columns(ctx, srs, s, cols.p, 3, cm.p);
+    G1Affine delta[3];
+    d2h(ctx->stream, delta, cm.p, sizeof(delta));
+    stream_sync(ctx->stream);
+    uint8_t c_s[48];
+    g1_compress(c_s, delta[2]);
+    if (memcmp(c_s, root144 + 96, 48)) throw Error(DR_EINVAL, "ring root does not belong to these params and this SRS (its C_s differs)");
+    uint8_t out[144];
+    for (int i = 0; i < 2; i++) {
+        G1 sum = G1::from_affine(in[i]);
+        g1_add(sum, G1::from_affine(delta[i]));
+        g1_compress(out + 48 * i, g1_to_affine(sum));
+    }
+    memcpy(out + 96, c_s, 48);
+    memcpy(out144, out, 144);
+}
+
 }  // namespace dr
 
 using namespace dr;
@@ -330,10 +474,7 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     if (!ctx || !srs || !prm || !out || (n_keys && !keys32)) throw Error(DR_EINVAL, "bad argument");
     ctx->activate();
     const uint32_t N = prm->domain_size;
-    // the reference stops at 4096 (params.py:172-173); larger domains (to 2^16) run the same pipeline over the two-pass NTT
-    if (N < 512 || N > 65536 || (N & (N - 1))) throw Error(DR_EINVAL, "domain_size must be a power of two in [512, 65536]");
-    if (prm->padding_rows != 4) throw Error(DR_EINVAL, "padding_rows must be 4 to match the 3 hidden rows");
-    if (prm->max_ring_size + SCALAR_BITS + 4 > N) throw Error(DR_EINVAL, "max_ring_size exceeds supported size for this domain");
+    check_ring_shape(prm);
     if (n_keys > prm->max_ring_size) throw Error(DR_EINVAL, "ring size exceeds max supported size");
     if (3 * (size_t)N + 1 > srs->n) throw Error(DR_EINVAL, "SRS too small for this domain (needs 3N+1 G1 points)");
     if (prm->suite_id_len > 32 || prm->h2c_dst_len > 64) throw Error(DR_EINVAL, "suite id / DST too long");
@@ -353,11 +494,7 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     ring->radix_omega = w4;
     // sanity: w4^4 == omega, omega^N == 1, omega^(N/2) != 1
     if (w4.sqr().sqr() != d.omega) throw Error(DR_EINVAL, "radix_omega^4 != omega");
-    {
-        Fr t = d.omega;
-        for (uint32_t i = 0; i + 1 < d.logN; i++) t = t.sqr();
-        if (t == Fr::one() || t.sqr() != Fr::one()) throw Error(DR_EINVAL, "omega is not a primitive N-th root of unity");
-    }
+    check_primitive_root(d.omega, d.logN);
     d.seed = te_from_param(prm->seed);
     d.blinding_base = te_from_param(prm->blinding_base);
     d.generator = te_from_param(prm->generator);
@@ -409,14 +546,7 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     // ---- public vector PK || padding || 2^i B || zeros (members.py:36-53) ----
     ring->nm.alloc(N);
     {
-        std::vector<TEAffine> host(N);
-        for (uint32_t i = 0; i < max_ring; i++) host[i] = ring->padding;
-        TEExt cur = TEExt::from_affine(d.blinding_base);
-        for (uint32_t i = max_ring; i < N - 4; i++) {
-            host[i] = te_to_affine(cur);
-            cur = te_dbl(cur);
-        }
-        for (uint32_t i = N - 4; i < N; i++) host[i] = TEAffine{Fr::zero(), Fr::zero()};
+        std::vector<TEAffine> host = public_vector_rows(N, max_ring, ring->padding, d.blinding_base);
         h2d(ctx->stream, ring->nm.p, host.data(), N * sizeof(TEAffine));
         if (n_keys) {
             DevBuf<uint8_t> kraw(n_keys * 32);
@@ -536,6 +666,38 @@ int dr_ring_points(dr_ring* r, uint8_t* out_xy64, size_t n_points) {
         fr_to_le_bytes_raw(out_xy64 + 64 * i, host[i].x.from_mont());
         fr_to_le_bytes_raw(out_xy64 + 64 * i + 32, host[i].y.from_mont());
     }
+    DR_API_END
+}
+
+int dr_ring_roots_from_keys(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, size_t n_rings, const uint8_t* keys32, const uint32_t* key_counts, uint8_t* roots144) {
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    Srs* srs = (Srs*)s;
+    if (!ctx || !srs || !prm || (n_rings && (!key_counts || !roots144))) throw Error(DR_EINVAL, "bad argument");
+    ctx->activate();
+    const RootSetup st = root_setup(ctx, srs, prm);
+    std::vector<uint32_t> key_off(n_rings + 1, 0);
+    for (size_t k = 0; k < n_rings; k++) {
+        if (key_counts[k] > st.max_ring) throw Error(DR_EINVAL, "ring size exceeds max supported size");
+        const uint64_t end = (uint64_t)key_off[k] + key_counts[k];
+        if (end > UINT32_MAX) throw Error(DR_EINVAL, "more than 2^32 - 1 keys in one call");
+        key_off[k + 1] = (uint32_t)end;
+    }
+    if (key_off[n_rings] && !keys32) throw Error(DR_EINVAL, "bad argument");
+    if (!n_rings) return DR_OK;
+    ring_roots(ctx, srs, st, n_rings, keys32, key_off, roots144);
+    DR_API_END
+}
+
+int dr_ring_root_update(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_t root144[144], size_t n, const uint32_t* rows, const uint8_t* old_keys32,
+                        const uint8_t* new_keys32, uint8_t out_root144[144]) {
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    Srs* srs = (Srs*)s;
+    if (!ctx || !srs || !prm || !root144 || !out_root144 || (n && (!rows || !new_keys32))) throw Error(DR_EINVAL, "bad argument");
+    ctx->activate();
+    const RootSetup st = root_setup(ctx, srs, prm);
+    ring_root_update(ctx, srs, st, root144, n, rows, old_keys32, new_keys32, out_root144);
     DR_API_END
 }
 

@@ -1253,16 +1253,57 @@ struct ZkRowsBody {
 };
 
 // ---- ring set-up helpers ----------------------------------------------------------------------------------------
-// keys (32 bytes each) -> nm[i]; undecodable / identity / out-of-subgroup keys become the padding point
+// The public-vector row of one 32-byte key: undecodable / identity / out-of-subgroup keys become the padding point
 // (members.py:36-41,61-69).
+DR_HD TEAffine ring_key_point(const uint8_t* key, const TEAffine& padding) {
+    TEAffine p;
+    if (!te_decode_checked(p, key)) p = padding;
+    return p;
+}
+// keys (32 bytes each) -> nm[i]
 struct KeyDecodeBody {
     DR_HD void operator()(const BlockCtx& ctx, const uint8_t* keys, uint32_t n_keys, TEAffine padding, TEAffine* nm) const {
         DR_THREAD_LOOP(t, ctx) {
             uint32_t i = ctx.bx * ctx.nthreads + t;
-            if (i < n_keys) {
-                TEAffine p;
-                if (!te_decode_checked(p, keys + 32 * (size_t)i)) p = padding;
-                nm[i] = p;
+            if (i < n_keys) nm[i] = ring_key_point(keys + 32 * (size_t)i, padding);
+        }
+    }
+};
+// Evaluations of the fixed columns of several rings at once (dr_ring_roots_from_keys): block row k < n_rings writes ring k's px and
+// py at out[2kN ..) and out[(2k+1)N ..), row i being its key key_off[k] + i while i < key_off[k+1] - key_off[k] and the
+// key-independent row tail[i] (padding, 2^j B, zeros) after that; block row n_rings, when launched, writes the selector s
+// (i < max_ring) at out[2 n_rings N ..).
+struct RingRootColumnsBody {
+    DR_HD void operator()(const BlockCtx& ctx, const TEAffine* tail, const uint8_t* keys, const uint32_t* key_off, uint32_t n_rings, uint32_t N, uint32_t max_ring,
+                          TEAffine padding, Fr* out) const {
+        const uint32_t k = ctx.by;
+        DR_THREAD_LOOP(t, ctx) {
+            uint32_t i = ctx.bx * ctx.nthreads + t;
+            if (i < N) {
+                if (k == n_rings) {
+                    out[2 * (size_t)n_rings * N + i] = i < max_ring ? Fr::one() : Fr::zero();
+                } else {
+                    const uint32_t first = key_off[k], count = key_off[k + 1] - first;
+                    const TEAffine p = i < count ? ring_key_point(keys + 32 * ((size_t)first + i), padding) : tail[i];
+                    out[2 * (size_t)k * N + i] = p.x;
+                    out[(2 * (size_t)k + 1) * N + i] = p.y;
+                }
+            }
+        }
+    }
+};
+// Change of the px / py evaluations when row rows[j] goes from old_keys[j] (null: the padding point) to new_keys[j], keys mapped as in
+// ring_key_point: out[rows[j]] = dx, out[N + rows[j]] = dy; the other rows of out stay as they are (zero).  Rows are distinct.
+struct RootDeltaBody {
+    DR_HD void operator()(const BlockCtx& ctx, const uint8_t* old_keys, const uint8_t* new_keys, const uint32_t* rows, uint32_t n, uint32_t N, TEAffine padding,
+                          Fr* out) const {
+        DR_THREAD_LOOP(t, ctx) {
+            uint32_t j = ctx.bx * ctx.nthreads + t;
+            if (j < n) {
+                const TEAffine from = old_keys ? ring_key_point(old_keys + 32 * (size_t)j, padding) : padding;
+                const TEAffine to = ring_key_point(new_keys + 32 * (size_t)j, padding);
+                out[rows[j]] = to.x - from.x;
+                out[N + rows[j]] = to.y - from.y;
             }
         }
     }

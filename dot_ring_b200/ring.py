@@ -8,12 +8,15 @@ root) and their 4x low-degree extensions.  The reference recomputes the latter o
 
 ``RingVerifier(roots)`` verifies Ring VRF proofs against ring roots alone: the verifier needs neither the keys nor the SRS
 window table, and one batch may span several rings (one aggregated pairing check for all of them).
+
+``RingRoot.from_keys(keys, params)`` derives a root from keys without a ``Ring`` or that table, and ``root.update(rows, new_keys,
+old_keys)`` follows a change of a few rows from the root alone (the root is linear in the column evaluations).
 """
 
 from __future__ import annotations
 
 from collections.abc import Sequence
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 from functools import lru_cache
 from typing import Any
 
@@ -125,12 +128,83 @@ class Column:
         return self._commitment
 
 
+def _run_on(engine: "Engine | EnginePool | None", fn):
+    """fn(engine) (None: the default engine); for a pool, fn(its first engine) on that engine's worker thread: a root is a few
+    hundred thousand additions, not worth sharding."""
+    engine = engine or default_engine()
+    if isinstance(engine, EnginePool):
+        return engine.map(lambda i: fn(engine.engines[i]), [0])[0]
+    return fn(engine)
+
+
+def _root_params(params: RingProofParams) -> _native.RingParamsStruct:
+    """The dr_ring_params of `params` as the root functions read them."""
+    aux = params.cv.curve.params.auxiliary_points
+    if not aux.padding_point:
+        raise ValueError("padding point is not configured in curve parameters")
+    return _native.make_ring_params(domain_size=params.domain_size, max_ring_size=params.max_ring_size, padding_rows=params.padding_rows, omega=params.omega,
+                                    seed=aux.accumulator_base, blinding_base=aux.blinding_base, padding_point=aux.padding_point, generator=(0, 0), suite_id=b"",
+                                    h2c_dst=b"")  # fmt: skip
+
+
+def _ring_keys(keys: Sequence[bytes]) -> list[bytes]:
+    """Keys of the wrong length can never decode: as in Ring, they become keys that map to the padding point."""
+    return [bytes(k) if len(k) == 32 else b"\xff" * 32 for k in keys]
+
+
 @dataclass
 class RingRoot:
     px: Column
     py: Column
     s: Column
     params: RingProofParams | None = None
+    engine: Any = field(default=None, compare=False, repr=False)  # what `update` commits with (None: the default engine)
+
+    @classmethod
+    def _from_bytes(cls, data: bytes, params: RingProofParams, eng: Engine, owner) -> "RingRoot":
+        pts, _ = eng.ctx.g1_decompress(data)
+        n = params.domain_size
+        return cls(px=Column("px", pts[0:96], n), py=Column("py", pts[96:192], n), s=Column("s", pts[192:288], n), params=params, engine=owner)
+
+    @classmethod
+    def from_keys(cls, keys: Sequence[bytes], params: RingProofParams | None = None, engine: "Engine | EnginePool | None" = None) -> "RingRoot":
+        """`RingRoot.from_ring(Ring(keys, params))` without the ring: the keys' public vector committed on the device with the
+        engine's small root table (`Engine.root_srs`), never the prover's window table."""
+        if params is None:
+            params = RingProofParams.from_ring_size(len(keys))
+        return cls.from_key_sets([keys], params, engine)[0]
+
+    @classmethod
+    def from_key_sets(cls, key_sets: Sequence[Sequence[bytes]], params: RingProofParams, engine: "Engine | EnginePool | None" = None) -> list["RingRoot"]:
+        """`from_keys` of every key set under one params, in one device call."""
+        sets = [_ring_keys(keys) for keys in key_sets]
+        for keys in sets:
+            if len(keys) > params.max_ring_size:
+                raise ValueError(f"ring size {len(keys)} exceeds max supported size {params.max_ring_size}")
+        struct = _root_params(params)
+
+        def run(eng: Engine):
+            roots = _native.ring_roots_from_keys(eng.root_srs(params.domain_size), struct, sets)
+            return [cls._from_bytes(r, params, eng, engine) for r in roots]
+
+        return _run_on(engine, run)
+
+    def update(self, rows: Sequence[int], new_keys: Sequence[bytes], old_keys: Sequence[bytes] | None = None) -> "RingRoot":
+        """The root after row rows[j] went from old_keys[j] to new_keys[j] (old_keys None: the rows held padding, an append); a
+        new key that does not decode nulls its row.  Needs only this root, not the other keys; `self` is left as it is."""
+        if self.params is None:
+            raise ValueError("updating a ring root requires its ring proof parameters")
+        params = self.params
+        struct = _root_params(params)
+        new = _ring_keys(new_keys)
+        old = None if old_keys is None else _ring_keys(old_keys)
+
+        def run(eng: Engine):
+            data = eng.ctx.g1_compress(b"".join(self.fixed_commitments()))
+            out = _native.ring_root_update(eng.root_srs(params.domain_size), struct, data, list(rows), new, old)
+            return RingRoot._from_bytes(out, params, eng, self.engine)
+
+        return _run_on(self.engine, run)
 
     @classmethod
     def from_ring(cls, ring: Ring, params: RingProofParams | None = None) -> "RingRoot":

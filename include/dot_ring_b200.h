@@ -306,6 +306,27 @@ int dr_ring_verify_multi(dr_ctx* ctx, dr_ring_verifier* const* verifiers, size_t
                          const uint32_t* in_off, const uint32_t* in_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* proofs784,
                          const uint8_t* coeffs_le32, int aggregate, uint8_t* verdict, int* all_ok);
 
+/* ---- ring roots from keys, and their updates -------------------------------------------------------------------------
+ * The 144-byte ring root of a key vector without a dr_ring: `RingRoot.from_ring(Ring(keys))` (dot_ring/vrf/ring/members.py:22-55,
+ * root.py:21-44,133-173) = compress(C_px) | compress(C_py) | compress(C_s) of the public vector PK || padding || 2^i B || 4 zero rows,
+ * keys mapped as dr_ring_create maps them (undecodable / identity / out-of-subgroup -> padding point).  Equal to dr_ring_root of
+ * dr_ring_create on the same keys, params and SRS G1 points, but `srs` needs only N points (not 3N + 1), may have any window geometry,
+ * and its G2 points are not used; nothing of the prover's ring (LDEs, verifier key, transcript) is built.
+ * params: domain_size, max_ring_size, padding_rows, omega, blinding_base, padding_point are read; the rest is ignored.
+ * dr_ring_roots_from_keys: ring k's keys are the next key_counts[k] 32-byte keys of keys32 after those of the rings before it; all rings
+ * share `params`; roots144 receives n_rings roots.  One call decodes every key, transforms and commits every ring's columns in batches.
+ * dr_ring_root_update: the root of the key vector in which row rows[j] held old_keys32[j] (NULL: every listed row held padding, an
+ * append) and now holds new_keys32[j], from root144 alone.  Old and new keys are mapped by the same rule (a new key that does not
+ * decode nulls the row); C_s does not change.  n == 0 copies the input root after the checks.  out_root144 may alias root144.
+ * DR_EINVAL: a check of dr_ring_create on N, padding_rows, max_ring_size or omega fails; key_counts[k] > max_ring_size; the SRS has
+ * fewer than N points or belongs to another context; a row >= max_ring_size or a row listed twice; root144 does not decode (as
+ * RingRoot.decode); the root's C_s is not the C_s of these params and this SRS (a root built for other params or another SRS).
+ * A commitment that sums to infinity is encoded as dr_g1_compress encodes infinity. */
+int dr_ring_roots_from_keys(dr_ctx* ctx, dr_srs* srs, const dr_ring_params* params, size_t n_rings, const uint8_t* keys32, const uint32_t* key_counts,
+                            uint8_t* roots144);
+int dr_ring_root_update(dr_ctx* ctx, dr_srs* srs, const dr_ring_params* params, const uint8_t root144[144], size_t n, const uint32_t* rows,
+                        const uint8_t* old_keys32, const uint8_t* new_keys32, uint8_t out_root144[144]);
+
 /* Aggregated batches of at least `n` proofs fold the two sides with two variable-base MSMs instead of 13 scalar multiplications
  * per proof (default 8192; same verdicts, tests lower it to exercise the path on small batches). */
 int dr_ring_verify_set_msm_threshold(size_t n);
