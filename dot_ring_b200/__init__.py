@@ -11,7 +11,8 @@ from .curve import Bandersnatch, Bandersnatch_SHAKE128
 from .kzg import KZG
 from .params import RingProofParams
 from .ring import Ring, RingRoot, RingVerifier
+from .ring_proof import RingProof
 from .vrf import PedersenVRF, RingVRF, ThinVRF, TinyVRF
 
-__all__ = ["Bandersnatch", "Bandersnatch_SHAKE128", "KZG", "RingProofParams", "Ring", "RingRoot", "RingVerifier", "RingVRF", "PedersenVRF", "TinyVRF", "ThinVRF", "__version__"]
+__all__ = ["Bandersnatch", "Bandersnatch_SHAKE128", "KZG", "RingProofParams", "Ring", "RingRoot", "RingVerifier", "RingProof", "RingVRF", "PedersenVRF", "TinyVRF", "ThinVRF", "__version__"]
 __version__ = "0.1.0"

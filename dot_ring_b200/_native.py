@@ -96,6 +96,7 @@ class Library:
         L.dr_ring_points.argtypes = [c_void_p, c_void_p, c_size_t]
         L.dr_ring_prove_batch.argtypes = [c_void_p, c_void_p, c_size_t] + [c_void_p] * 10
         L.dr_ring_prove_multi.argtypes = [c_void_p, c_void_p, c_size_t, c_void_p, c_size_t] + [c_void_p] * 10
+        L.dr_ring_proof_prove_multi.argtypes = [c_void_p, c_void_p, c_size_t, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p]
         L.dr_ring_prove_phase_ms.argtypes = [c_void_p, POINTER(c_float * 6)]
         L.dr_ring_prove_commit_kernel_ms.argtypes = [c_void_p, POINTER(c_float), POINTER(c_uint32)]
         L.dr_ring_witness_table_bits.argtypes = [c_void_p]
@@ -712,23 +713,30 @@ class NativeRing:
             raise ValueError("batch inputs must have equal length")
         blob, a_off, a_len, d_off, d_len = pack_items(alphas, ads)
         rows = np.ctypeslib.as_ctypes(np.array(producer_index if n else [0], dtype=np.uint32))
-        ring = None
-        if ring_index is not None:
-            idx = np.array(ring_index if n else [0], dtype=np.int64)
-            if idx.min() < 0 or idx.max() >> 32:
-                raise ValueError("ring index out of range")
-            ring = np.ctypeslib.as_ctypes(idx.astype(np.uint32))
-        zk = None
+        ring = None if ring_index is None else NativeRing._pack_ring_index(ring_index, n)
+        return {"n": n, "blob": blob, "a_off": a_off, "a_len": a_len, "d_off": d_off, "d_len": d_len, "sk": b"".join(secret_keys), "rows": rows,
+                "zk": NativeRing._pack_zk_rows(zk_rows, n), "ring": ring, "proofs": ctypes.create_string_buffer(784 * max(n, 1)),
+                "status": (ctypes.c_uint32 * max(n, 1))()}
+
+    @staticmethod
+    def _pack_zk_rows(zk_rows, n: int) -> bytes | None:
+        """12 blinding rows per proof as 32-byte little-endian values (None: zeros)."""
         if isinstance(zk_rows, (bytes, bytearray)):  # already 12 x 32-byte little-endian values per proof
             if len(zk_rows) != 12 * 32 * n:
                 raise ValueError("zk_rows must hold 12 field elements per proof")
-            zk = bytes(zk_rows)
-        elif zk_rows is not None:
+            return bytes(zk_rows)
+        if zk_rows is not None:
             if len(zk_rows) != 12 * n:
                 raise ValueError("zk_rows must hold 12 field elements per proof")
-            zk = b"".join(int(v).to_bytes(32, "little") for v in zk_rows)
-        return {"n": n, "blob": blob, "a_off": a_off, "a_len": a_len, "d_off": d_off, "d_len": d_len, "sk": b"".join(secret_keys), "rows": rows, "zk": zk,
-                "ring": ring, "proofs": ctypes.create_string_buffer(784 * max(n, 1)), "status": (ctypes.c_uint32 * max(n, 1))()}
+            return b"".join(int(v).to_bytes(32, "little") for v in zk_rows)
+        return None
+
+    @staticmethod
+    def _pack_ring_index(ring_index, n: int):
+        idx = np.array(ring_index if n else [0], dtype=np.int64)
+        if idx.min() < 0 or idx.max() >> 32:
+            raise ValueError("ring index out of range")
+        return np.ctypeslib.as_ctypes(idx.astype(np.uint32))
 
     @staticmethod
     def _packed_args(pk: dict, lo: int, hi: int) -> list:
@@ -771,6 +779,58 @@ class NativeRing:
         pk = NativeRing.pack_prove_inputs(alphas, ads, secret_keys, producer_index, zk_rows, ring_index=index)
         NativeRing.prove_multi_packed(rings, pk)
         return NativeRing.unpack_proofs(pk)
+
+    @staticmethod
+    def pack_ring_proof_inputs(index: list[int], producer_index: list[int], blindings: list[int], zk_rows=None, label: bytes | None = None) -> dict:
+        """Host-side packing of a bare ring-proof batch (dr_ring_proof_prove_multi), once per batch: a shard is a sub-range of every array."""
+        n = len(index)
+        if not (len(producer_index) == len(blindings) == n):
+            raise ValueError("batch inputs must have equal length")
+        if any(int(t) < 0 or int(t) >> 256 for t in blindings):
+            raise ValueError("blinding factor out of range")
+        rows = np.array(producer_index if n else [0], dtype=np.int64)
+        if rows.min() < 0 or rows.max() >> 32:
+            raise ValueError("producer row out of range")
+        label = b"" if label is None else bytes(label)
+        return {"n": n, "ring": NativeRing._pack_ring_index(index, n), "rows": np.ctypeslib.as_ctypes(rows.astype(np.uint32)),
+                "t": b"".join(int(t).to_bytes(32, "little") for t in blindings), "zk": NativeRing._pack_zk_rows(zk_rows, n), "label": label,
+                "relations": ctypes.create_string_buffer(64 * max(n, 1)), "payloads": ctypes.create_string_buffer(592 * max(n, 1))}
+
+    @staticmethod
+    def proof_prove_multi_packed(rings: list["NativeRing"], pk: dict, lo: int = 0, hi: int | None = None) -> None:
+        """dr_ring_proof_prove_multi over items [lo, hi) of a packed bare ring-proof batch."""
+        hi = pk["n"] if hi is None else hi
+        if hi <= lo:
+            return
+        if not rings:
+            raise ValueError("at least one ring is required")
+        ctx = rings[0].ctx
+        handles = (c_void_p * len(rings))(*[r.handle for r in rings])
+        t = (ctypes.c_char * (32 * (hi - lo))).from_buffer_copy(pk["t"], 32 * lo)
+        zk = None if pk["zk"] is None else (ctypes.c_char * (384 * (hi - lo))).from_buffer_copy(pk["zk"], 384 * lo)
+        label = pk["label"]
+        ctx.library.check(
+            ctx.library.lib.dr_ring_proof_prove_multi(
+                ctx.handle, handles, len(rings), ctypes.byref(pk["ring"], 4 * lo), hi - lo, ctypes.byref(pk["rows"], 4 * lo), t, zk, label or None, len(label),
+                ctypes.byref(pk["relations"], 64 * lo), ctypes.byref(pk["payloads"], 592 * lo),
+            )
+        )
+        ctypes.memset(t, 0, ctypes.sizeof(t))
+
+    @staticmethod
+    def unpack_ring_proofs(pk: dict):
+        """-> (relations as (x, y), 592-byte payloads)."""
+        n, rel, pay = pk["n"], pk["relations"].raw, pk["payloads"].raw
+        relations = [(int.from_bytes(rel[64 * i : 64 * i + 32], "little"), int.from_bytes(rel[64 * i + 32 : 64 * i + 64], "little")) for i in range(n)]
+        return relations, [pay[592 * i : 592 * i + 592] for i in range(n)]
+
+    @staticmethod
+    def proof_prove_multi(rings: list["NativeRing"], index: list[int], producer_index: list[int], blindings: list[int], zk_rows=None, label: bytes | None = None):
+        """Bare ring proofs (RingProofBuilder.build): item i proves row producer_index[i] of rings[index[i]] with blinding factor blindings[i],
+        under `label` (None: the suite id) -> (relations PK_k + t * B as (x, y), 592-byte payloads)."""
+        pk = NativeRing.pack_ring_proof_inputs(index, producer_index, blindings, zk_rows, label)
+        NativeRing.proof_prove_multi_packed(rings, pk)
+        return NativeRing.unpack_ring_proofs(pk)
 
     @staticmethod
     def unpack_proofs(pk: dict):

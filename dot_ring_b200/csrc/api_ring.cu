@@ -96,20 +96,34 @@ static ProveScratch& scratch_for(Ctx* ctx) {
     return *(ProveScratch*)ctx->prove_scratch.get();
 }
 
+// What a prove call produces.  Ring VRF (dr_ring_prove_batch / _multi): `secrets32` are secret keys, each item gets its Pedersen part
+// and a 784-byte proof with a status word.  Bare ring proof (dr_ring_proof_prove_multi): `secrets32` are blinding factors, the inputs
+// (blob and offsets) are unused, and each item gets its relation (64 bytes) and 592-byte payload.
+struct ProveOutputs {
+    bool bare = false;
+    uint8_t* proofs784 = nullptr;
+    uint32_t* status = nullptr;
+    uint8_t* relations_xy64 = nullptr;
+    uint8_t* payloads592 = nullptr;
+};
+
 // One prove call: item i against rings[ring_index[i]] (ring_index null: every item against rings[0]).  The callers have checked
 // that the rings share the context, the SRS and the suite; `dtab` holds their RingTab entries on the device, in the same order.
 // Items are grouped by domain size (ascending), in the caller's order within a group, and every group runs its own equal-width
-// passes over one scratch sized for the largest domain of the call.  Proofs and status words land at the caller's positions.
+// passes over one scratch sized for the largest domain of the call.  Outputs land at the caller's positions.
 static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const uint32_t* ring_index, size_t n, const uint8_t* blob, const uint32_t* alpha_off,
-                       const uint32_t* alpha_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* secret_keys32, const uint32_t* producer_index,
-                       const uint8_t* zk_rows, uint8_t* proofs784, uint32_t* status) {
+                       const uint32_t* alpha_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* secrets32, const uint32_t* producer_index,
+                       const uint8_t* zk_rows, const ProveOutputs& res) {
     auto ring_of = [&](size_t i) { return ring_index ? ring_index[i] : 0u; };
+    const bool bare = res.bare;
     size_t blob_len = 0;
     std::vector<uint32_t> domains;  // distinct domain sizes of the items' rings
     for (size_t i = 0; i < n; i++) {
-        size_t e1 = (size_t)alpha_off[i] + alpha_len[i], e2 = (size_t)ad_off[i] + ad_len[i];
-        if (e1 > blob_len) blob_len = e1;
-        if (e2 > blob_len) blob_len = e2;
+        if (!bare) {
+            size_t e1 = (size_t)alpha_off[i] + alpha_len[i], e2 = (size_t)ad_off[i] + ad_len[i];
+            if (e1 > blob_len) blob_len = e1;
+            if (e2 > blob_len) blob_len = e2;
+        }
         const uint32_t N = rings[ring_of(i)]->dev.N;
         if (std::find(domains.begin(), domains.end(), N) == domains.end()) domains.push_back(N);
     }
@@ -203,13 +217,15 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
             for (uint32_t i = 0; i < m; i++) {
                 const size_t it = item(base + i);
                 ProveInput& pi = hin[i];
-                pi.alpha_off = alpha_off[it];
-                pi.alpha_len = alpha_len[it];
-                pi.ad_off = ad_off[it];
-                pi.ad_len = ad_len[it];
+                if (!bare) {
+                    pi.alpha_off = alpha_off[it];
+                    pi.alpha_len = alpha_len[it];
+                    pi.ad_off = ad_off[it];
+                    pi.ad_len = ad_len[it];
+                }
                 pi.k = producer_index[it];
                 pi.ring = ring_of(it);
-                memcpy(pi.sk, secret_keys32 + 32 * it, 32);
+                memcpy(pi.sk, secrets32 + 32 * it, 32);
             }
             h2d(ctx->stream, sc.in.p, hin.data(), m * sizeof(ProveInput));
             const uint32_t tb = 64, pb = (m + tb - 1) / tb;
@@ -229,14 +245,20 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
                 launch(ctx->stream, Dim3((m * 12 + 127) / 128), 128, 0, ZkRowsBody(), (const uint8_t*)nullptr, sc.st.p, m);
             }
             // Pedersen part: the half the ring proof needs (blinding factor, blinded key) on the main stream, eight lanes per proof; the
-            // rest (nonces, R, Ok, responses) on the side stream, joined before the proofs are assembled
+            // rest (nonces, R, Ok, responses) on the side stream, joined before the proofs are assembled.  A bare ring proof starts from
+            // the caller's blinding factor instead and has no Pedersen part.
             {
                 const uint32_t per_block = tb / COOP_LANES;  // eight lanes per proof
-                launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, pedersen_start_smem(tb), PedersenStartBody(), rg, dtab, (const ProveInput*)sc.in.p,
-                       (const uint8_t*)sc.blob.p, sc.st.p, m);
+                if (bare) {
+                    launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, ring_proof_start_smem(tb), RingProofStartBody(), rg, dtab, (const ProveInput*)sc.in.p,
+                           sc.st.p, m);
+                } else {
+                    launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, pedersen_start_smem(tb), PedersenStartBody(), rg, dtab, (const ProveInput*)sc.in.p,
+                           (const uint8_t*)sc.blob.p, sc.st.p, m);
+                    ctx->fork_side();
+                    launch(ctx->side, Dim3((m + 31) / 32), 32, 0, PedersenFinishBody(), rg, (const ProveInput*)sc.in.p, sc.st.p, m);
+                }
             }
-            ctx->fork_side();
-            launch(ctx->side, Dim3((m + 31) / 32), 32, 0, PedersenFinishBody(), rg, (const ProveInput*)sc.in.p, sc.st.p, m);
             {
                 const uint32_t wt = 4 * WIT_LANES;  // four proofs per block, a warp each
                 launch(ctx->stream, Dim3((m + 3) / 4), wt, witness_coop_smem(wt), WitnessBody(), rg, dtab, sc.st.p, m);
@@ -305,18 +327,27 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
             launch(ctx->stream, Dim3((m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)sc.res.p, 1u, 0x05u, sc.st.p, m);
             launch(ctx->stream, Dim3((m + 127) / 128), 128, 0, StoreCommitBody(), (const G1Affine*)(sc.res.p + m), 1u, 0x06u, sc.st.p, m);
             pt.mark(ctx, 5);
-            ctx->join_side();
-            launch(ctx->stream, Dim3(pb), tb, 0, FinalizeBody(), (const ProofState*)sc.st.p, m, sc.out.p, sc.status.p);
+            if (bare) {
+                launch(ctx->stream, Dim3(pb), tb, 0, RingProofFinalizeBody(), sc.st.p, m, sc.out.p);
+            } else {
+                ctx->join_side();
+                launch(ctx->stream, Dim3(pb), tb, 0, FinalizeBody(), (const ProofState*)sc.st.p, m, sc.out.p, sc.status.p);
+            }
             pt.mark(ctx, 8);
-            dev_zero(ctx->stream, sc.in.p, m * sizeof(ProveInput));  // secret keys do not outlive the pass on the device
-            if (direct) {
-                d2h(ctx->stream, proofs784 + 784 * base, sc.out.p, (size_t)m * 784);
-                d2h(ctx->stream, status + base, sc.status.p, (size_t)m * sizeof(uint32_t));
+            dev_zero(ctx->stream, sc.in.p, m * sizeof(ProveInput));  // secret keys / blinding factors do not outlive the pass on the device
+            if (bare && direct) {
+                d2h(ctx->stream, res.relations_xy64 + 64 * base, sc.out.p, (size_t)m * 64);
+                d2h(ctx->stream, res.payloads592 + 592 * base, sc.out.p + (size_t)m * 64, (size_t)m * 592);
+            } else if (direct) {
+                d2h(ctx->stream, res.proofs784 + 784 * base, sc.out.p, (size_t)m * 784);
+                d2h(ctx->stream, res.status + base, sc.status.p, (size_t)m * sizeof(uint32_t));
             } else {
                 hout.resize((size_t)m * 784);
-                hstatus.resize(m);
-                d2h(ctx->stream, hout.data(), sc.out.p, (size_t)m * 784);
-                d2h(ctx->stream, hstatus.data(), sc.status.p, (size_t)m * sizeof(uint32_t));
+                d2h(ctx->stream, hout.data(), sc.out.p, (size_t)m * (bare ? 656 : 784));
+                if (!bare) {
+                    hstatus.resize(m);
+                    d2h(ctx->stream, hstatus.data(), sc.status.p, (size_t)m * sizeof(uint32_t));
+                }
             }
             pt.mark(ctx, -1);
             stream_sync(ctx->stream);
@@ -324,8 +355,13 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
             if (!direct) {
                 for (uint32_t i = 0; i < m; i++) {
                     const size_t it = item(base + i);
-                    memcpy(proofs784 + 784 * it, hout.data() + (size_t)784 * i, 784);
-                    status[it] = hstatus[i];
+                    if (bare) {
+                        memcpy(res.relations_xy64 + 64 * it, hout.data() + (size_t)64 * i, 64);
+                        memcpy(res.payloads592 + 592 * it, hout.data() + (size_t)64 * m + (size_t)592 * i, 592);
+                    } else {
+                        memcpy(res.proofs784 + 784 * it, hout.data() + (size_t)784 * i, 784);
+                        res.status[it] = hstatus[i];
+                    }
                 }
             }
         }
@@ -334,6 +370,42 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
         volatile uint8_t* w = (volatile uint8_t*)hin.data();
         for (size_t i = 0; i < hin.size() * sizeof(ProveInput); i++) w[i] = 0;
     }
+}
+
+// The ring transcript after the verifier key (root.py:54-71, phases.py:72-74) under `label`: what dr_ring_create keeps with the ring
+// under the suite id, and dr_ring_proof_prove_multi builds per call for another label.
+static Shake128 ring_transcript_prefix(const uint8_t* label, uint32_t label_len, const Srs* srs, const uint8_t* commit_be96) {
+    Shake128 tr;
+    tr.init();
+    tr.absorb(label, label_len);
+    tr.absorb_be32(label_len);
+    shake_absorb_label(tr, "vk", 2);
+    tr.absorb(srs->g1_0_be96, 96);
+    tr.absorb(srs->g2_be192, 384);
+    tr.absorb(commit_be96, 288);
+    tr.absorb_be32(96 + 384 + 288);
+    return tr;
+}
+
+// The argument checks dr_ring_prove_multi and dr_ring_proof_prove_multi share: the rings and the ring index.
+static void check_prove_rings(Ctx* ctx, Ring* const* rings, size_t n_rings, const uint32_t* ring_index, size_t n) {
+    if (n && !n_rings) throw Error(DR_EINVAL, "at least one ring is required");
+    for (size_t k = 0; k < n_rings; k++) {
+        const Ring* ring = rings[k];
+        const Ring* first = rings[0];
+        if (!ring) throw Error(DR_EINVAL, "bad argument");
+        if (ring->ctx != ctx) throw Error(DR_EINVAL, "ring belongs to another context");
+        if (ring->srs != first->srs) throw Error(DR_EINVAL, "rings of one call must share the SRS handle");
+        if (!same_suite(ring->suite, first->suite) || !(ring->dev.seed == first->dev.seed) || !(ring->padding == first->padding))
+            throw Error(DR_EINVAL, "rings of one call must share the suite");
+    }
+    // rings of one domain size share its roots of unity: a pass takes the twiddles and coset powers from one of them
+    for (size_t k = 0; k < n_rings; k++)
+        for (size_t j = 0; j < k; j++)
+            if (rings[j]->dev.N == rings[k]->dev.N && (rings[j]->dev.omega != rings[k]->dev.omega || rings[j]->radix_omega != rings[k]->radix_omega))
+                throw Error(DR_EINVAL, "rings of one domain size must share omega and radix_omega");
+    for (size_t i = 0; i < n; i++)
+        if (ring_index[i] >= n_rings) throw Error(DR_EINVAL, "ring index out of range");
 }
 
 // ---- ring roots without a ring ----------------------------------------------------------------------------------------------
@@ -600,15 +672,7 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
 
     // ---- verifier-key transcript prefix (root.py:54-71, phases.py:72-74) ----
     {
-        Shake128 tr;
-        tr.init();
-        tr.absorb(d.suite_id, d.suite_id_len);
-        tr.absorb_be32(d.suite_id_len);
-        shake_absorb_label(tr, "vk", 2);
-        tr.absorb(srs->g1_0_be96, 96);
-        tr.absorb(srs->g2_be192, 384);
-        tr.absorb(ring->commit_be96, 288);
-        tr.absorb_be32(96 + 384 + 288);
+        const Shake128 tr = ring_transcript_prefix(d.suite_id, d.suite_id_len, srs, ring->commit_be96);
         ring->prefix.alloc(1);
         h2d(ctx->stream, ring->prefix.p, &tr, sizeof(Shake128));
         ring->tab.prefix = ring->prefix.p;
@@ -711,7 +775,10 @@ int dr_ring_prove_batch(dr_ctx* c, dr_ring* r, size_t n, const uint8_t* blob, co
         throw Error(DR_EINVAL, "bad argument");
     ctx->activate();
     if (!n) return DR_OK;
-    ring_prove(ctx, &ring, ring->tab_dev.p, nullptr, n, blob, alpha_off, alpha_len, ad_off, ad_len, secret_keys32, producer_index, zk_rows, proofs784, status);
+    ProveOutputs res;
+    res.proofs784 = proofs784;
+    res.status = status;
+    ring_prove(ctx, &ring, ring->tab_dev.p, nullptr, n, blob, alpha_off, alpha_len, ad_off, ad_len, secret_keys32, producer_index, zk_rows, res);
     DR_API_END
 }
 
@@ -723,31 +790,62 @@ int dr_ring_prove_multi(dr_ctx* c, dr_ring* const* rs, size_t n_rings, const uin
     if (!ctx || (n_rings && !rs) || n_rings > UINT32_MAX ||
         (n && (!ring_index || !alpha_off || !alpha_len || !ad_off || !ad_len || !secret_keys32 || !producer_index || !proofs784 || !status)))
         throw Error(DR_EINVAL, "bad argument");
-    if (n && !n_rings) throw Error(DR_EINVAL, "at least one ring is required");
     Ring* const* rings = (Ring* const*)rs;
-    for (size_t k = 0; k < n_rings; k++) {
-        const Ring* ring = rings[k];
-        const Ring* first = rings[0];
-        if (!ring) throw Error(DR_EINVAL, "bad argument");
-        if (ring->ctx != ctx) throw Error(DR_EINVAL, "ring belongs to another context");
-        if (ring->srs != first->srs) throw Error(DR_EINVAL, "rings of one call must share the SRS handle");
-        if (!same_suite(ring->suite, first->suite) || !(ring->dev.seed == first->dev.seed) || !(ring->padding == first->padding))
-            throw Error(DR_EINVAL, "rings of one call must share the suite");
-    }
-    // rings of one domain size share its roots of unity: a pass takes the twiddles and coset powers from one of them
-    for (size_t k = 0; k < n_rings; k++)
-        for (size_t j = 0; j < k; j++)
-            if (rings[j]->dev.N == rings[k]->dev.N && (rings[j]->dev.omega != rings[k]->dev.omega || rings[j]->radix_omega != rings[k]->radix_omega))
-                throw Error(DR_EINVAL, "rings of one domain size must share omega and radix_omega");
-    for (size_t i = 0; i < n; i++)
-        if (ring_index[i] >= n_rings) throw Error(DR_EINVAL, "ring index out of range");
+    check_prove_rings(ctx, rings, n_rings, ring_index, n);
     ctx->activate();
     if (!n) return DR_OK;
     std::vector<RingTab> table(n_rings);
     for (size_t k = 0; k < n_rings; k++) table[k] = rings[k]->tab;
     DevBuf<RingTab> dtable(n_rings);
     h2d(ctx->stream, dtable.p, table.data(), n_rings * sizeof(RingTab));
-    ring_prove(ctx, rings, dtable.p, ring_index, n, blob, alpha_off, alpha_len, ad_off, ad_len, secret_keys32, producer_index, zk_rows, proofs784, status);
+    ProveOutputs res;
+    res.proofs784 = proofs784;
+    res.status = status;
+    ring_prove(ctx, rings, dtable.p, ring_index, n, blob, alpha_off, alpha_len, ad_off, ad_len, secret_keys32, producer_index, zk_rows, res);
+    DR_API_END
+}
+
+int dr_ring_proof_prove_multi(dr_ctx* c, dr_ring* const* rs, size_t n_rings, const uint32_t* ring_index, size_t n, const uint32_t* producer_index,
+                              const uint8_t* blinding_le32, const uint8_t* zk_rows, const uint8_t* label, size_t label_len, uint8_t* relations_xy64,
+                              uint8_t* payloads592) {
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || (n_rings && !rs) || n_rings > UINT32_MAX || (label_len && !label) ||
+        (n && (!ring_index || !producer_index || !blinding_le32 || !relations_xy64 || !payloads592)))
+        throw Error(DR_EINVAL, "bad argument");
+    if (label_len > 32) throw Error(DR_EINVAL, "transcript label longer than 32 bytes");
+    Ring* const* rings = (Ring* const*)rs;
+    check_prove_rings(ctx, rings, n_rings, ring_index, n);
+    for (size_t i = 0; i < n; i++) {
+        if (producer_index[i] >= rings[ring_index[i]]->tab.max_ring) throw Error(DR_EINVAL, "producer row out of range: rows lie below max_ring_size");
+        Fn t;
+        for (int j = 0; j < 8; j++) {
+            const uint8_t* b = blinding_le32 + 32 * i + 4 * j;
+            t.v[j] = (uint32_t)b[0] | (uint32_t)b[1] << 8 | (uint32_t)b[2] << 16 | (uint32_t)b[3] << 24;
+        }
+        if (!t.is_canonical_raw()) throw Error(DR_EINVAL, "blinding factor is not below the group order");
+    }
+    ctx->activate();
+    if (!n) return DR_OK;
+    std::vector<RingTab> table(n_rings);
+    for (size_t k = 0; k < n_rings; k++) table[k] = rings[k]->tab;
+    // another label than the suite id: one transcript prefix per ring of the call, pointed at by this call's copy of the table
+    DevBuf<Shake128> prefixes;
+    const RingDev& lead = rings[0]->dev;
+    if (label_len && !(label_len == lead.suite_id_len && !memcmp(label, lead.suite_id, label_len))) {
+        std::vector<Shake128> host(n_rings);
+        for (size_t k = 0; k < n_rings; k++) host[k] = ring_transcript_prefix(label, (uint32_t)label_len, rings[k]->srs, rings[k]->commit_be96);
+        prefixes.alloc(n_rings);
+        h2d(ctx->stream, prefixes.p, host.data(), n_rings * sizeof(Shake128));
+        for (size_t k = 0; k < n_rings; k++) table[k].prefix = prefixes.p + k;
+    }
+    DevBuf<RingTab> dtable(n_rings);
+    h2d(ctx->stream, dtable.p, table.data(), n_rings * sizeof(RingTab));
+    ProveOutputs res;
+    res.bare = true;
+    res.relations_xy64 = relations_xy64;
+    res.payloads592 = payloads592;
+    ring_prove(ctx, rings, dtable.p, ring_index, n, nullptr, nullptr, nullptr, nullptr, nullptr, blinding_le32, producer_index, zk_rows, res);
     DR_API_END
 }
 

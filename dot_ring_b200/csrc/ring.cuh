@@ -125,7 +125,7 @@ struct ProveInput {  // host-packed per proof
     uint32_t alpha_off, alpha_len, ad_off, ad_len;
     uint32_t k;
     uint32_t ring;  // entry of the call's RingTab array
-    uint8_t sk[32];
+    uint8_t sk[32];  // Ring VRF: the secret key; bare ring proof: the blinding factor t (both little-endian, below the group order)
 };
 
 // column index convention inside the prover buffers
@@ -454,6 +454,44 @@ struct PedersenStartBody {
         }
     }
 };
+// The start of a bare ring proof (RingProofBuilder.build, proof_builder.py:38-69) from a caller's blinding factor t, in place of
+// PedersenStartBody: relation = PK_k + t * B, with t * B split by table windows over eight lanes per proof as in step E above.  No
+// hash-to-curve, no sk * G, no Pedersen transcript; the host has checked t < order and k < max_ring.
+DR_HD size_t ring_proof_start_smem(uint32_t threads) { return (size_t)threads * sizeof(TEExt); }
+struct RingProofStartBody {
+    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProveInput* in, ProofState* st, uint32_t count) const {
+        const uint32_t items = ctx.nthreads / COOP_LANES;
+        TEExt* part = (TEExt*)ctx.smem;  // [items][COOP_LANES]
+        auto limbs = [](uint32_t* out, const uint8_t* le32) {
+            for (int i = 0; i < 8; i++)
+                out[i] = (uint32_t)le32[4 * i] | (uint32_t)le32[4 * i + 1] << 8 | (uint32_t)le32[4 * i + 2] << 16 | (uint32_t)le32[4 * i + 3] << 24;
+        };
+        DR_THREAD_LOOP(t, ctx) {
+            const uint32_t item = t / COOP_LANES, p = ctx.bx * items + item;
+            if (p < count) {
+                uint32_t tr[8];
+                limbs(tr, in[p].sk);
+                te_mul_fixed_coop_partial(t % COOP_LANES, rg.b_tab, tr, part + COOP_LANES * item);
+            }
+        }
+        DR_BLOCK_SYNC();
+        DR_THREAD_LOOP(t, ctx) {
+            const uint32_t item = t / COOP_LANES, lane = t % COOP_LANES, p = ctx.bx * items + item;
+            const uint32_t ring = p < count ? in[p].ring : 0u;
+            const TEAffine* nm = tab[ring].nm;
+            if (p < count && lane == 0) {
+                ProofState& ps = st[p];
+                const ProveInput& pi = in[p];
+                ps.k = pi.k;
+                ps.ring = ring;
+                limbs(ps.t, pi.sk);
+                ps.relation = te_to_affine(te_add(TEExt::from_affine(nm[pi.k]), te_fold_fixed_coop(part + COOP_LANES * item)));
+                ps.status = 0;
+            }
+        }
+    }
+};
+
 // Second half, one thread per proof; nothing of the ring proof depends on it, so it runs on the side stream.
 struct PedersenFinishBody {
     DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const ProveInput* in, ProofState* st, uint32_t count) const {
@@ -1197,6 +1235,17 @@ struct OpenQuotientsBody {
 };
 
 // ---- P. proof assembly (vrf/ring/vrf.py:51-58, proof_payload.py:68-91): 784 bytes per proof ----------------------
+// the 592-byte ring-proof payload (proof_payload.py:68-91)
+DR_HD void encode_ring_payload(uint8_t* o, const ProofState& ps) {
+    for (int i = 0; i < 4; i++) g1_compress(o + 48 * i, ps.commits[i]);
+    o += 192;
+    for (int i = 0; i < 7; i++) fr_to_le_bytes_raw(o + 32 * i, ps.evals[i].from_mont());
+    o += 224;
+    g1_compress(o, ps.commits[4]);
+    fr_to_le_bytes_raw(o + 48, ps.lzw.from_mont());
+    g1_compress(o + 80, ps.commits[5]);
+    g1_compress(o + 128, ps.commits[6]);
+}
 struct FinalizeBody {
     DR_HD void operator()(const BlockCtx& ctx, const ProofState* st, uint32_t count, uint8_t* out, uint32_t* status) const {
         DR_THREAD_LOOP(t, ctx) {
@@ -1205,16 +1254,24 @@ struct FinalizeBody {
                 const ProofState& ps = st[p];
                 uint8_t* o = out + 784 * (size_t)p;
                 for (int i = 0; i < 192; i++) o[i] = ps.pedersen[i];
-                o += 192;
-                for (int i = 0; i < 4; i++) g1_compress(o + 48 * i, ps.commits[i]);
-                o += 192;
-                for (int i = 0; i < 7; i++) fr_to_le_bytes_raw(o + 32 * i, ps.evals[i].from_mont());
-                o += 224;
-                g1_compress(o, ps.commits[4]);
-                fr_to_le_bytes_raw(o + 48, ps.lzw.from_mont());
-                g1_compress(o + 80, ps.commits[5]);
-                g1_compress(o + 128, ps.commits[6]);
+                encode_ring_payload(o + 192, ps);
                 status[p] = ps.status;
+            }
+        }
+    }
+};
+// Bare ring proofs: relations (x | y, 32-byte little-endian each) at out[64 p ..), payloads at out[64 count + 592 p ..).  The
+// blinding factor is the last thing of the proof state that identifies the signer (relation - t * B = PK_k): it is cleared here.
+struct RingProofFinalizeBody {
+    DR_HD void operator()(const BlockCtx& ctx, ProofState* st, uint32_t count, uint8_t* out) const {
+        DR_THREAD_LOOP(t, ctx) {
+            uint32_t p = ctx.bx * ctx.nthreads + t;
+            if (p < count) {
+                ProofState& ps = st[p];
+                fr_to_le_bytes_raw(out + 64 * (size_t)p, ps.relation.x.from_mont());
+                fr_to_le_bytes_raw(out + 64 * (size_t)p + 32, ps.relation.y.from_mont());
+                encode_ring_payload(out + 64 * (size_t)count + 592 * (size_t)p, ps);
+                for (int i = 0; i < 8; i++) ps.t[i] = 0;
             }
         }
     }

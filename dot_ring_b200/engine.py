@@ -281,6 +281,22 @@ class PooledRingNative:
         pool.map(lambda i: _native.NativeRing.prove_multi_packed([r.replicas[i] for r in rings], pk, bounds[i][0], bounds[i][1]), range(len(bounds)))
         return _native.NativeRing.unpack_proofs(pk)
 
+    @staticmethod
+    def proof_prove_multi(rings: list["PooledRingNative"], index, producer_index, blindings, zk_rows=None, label=None):
+        """Bare ring proofs (`NativeRing.proof_prove_multi`) sharded as `prove_multi`: packed once, device d proves a contiguous shard
+        against its own replicas of the rings."""
+        if not rings:
+            if len(index):
+                raise ValueError("at least one ring is required")
+            return [], []
+        pool = rings[0].pool
+        if any(not isinstance(r, PooledRingNative) or r.pool is not pool for r in rings):
+            raise ValueError("rings of one call must be built on the same EnginePool")
+        pk = _native.NativeRing.pack_ring_proof_inputs(index, producer_index, blindings, zk_rows, label)
+        bounds = pool.shard_bounds(pk["n"], len(pool))
+        pool.map(lambda i: _native.NativeRing.proof_prove_multi_packed([r.replicas[i] for r in rings], pk, bounds[i][0], bounds[i][1]), range(len(bounds)))
+        return _native.NativeRing.unpack_ring_proofs(pk)
+
     def verify_batch(self, inputs, ads, proofs, coeffs, aggregate: bool = False):
         """Per-item mode: shards are independent.  Aggregated mode (`RingVRF.batch_verify`): every device folds its shard into
         its own random-linear-combination check (its slice of the caller's coefficients) and the batch is accepted iff every

@@ -486,21 +486,7 @@ class RingVRF(VRF):
             found = cls._signer_rows(rings[k], {(sks[i], pks[i]) for i in items})
             for i in items:
                 rows[i] = found[pks[i]]
-        zeroed = [rings[k].params.test_vectors for k in index]
-        if all(zeroed):
-            zk = None
-        else:
-            if zk_rows is None:
-                prime = rings[index[zeroed.index(False)]].params.prime
-                zk = [0 if z else secrets.randbelow(prime) for z in zeroed for _ in range(12)]
-            else:
-                if isinstance(zk_rows, (bytes, bytearray)):
-                    if len(zk_rows) != 12 * 32 * n:
-                        raise ValueError("zk_rows must hold 12 field elements per proof")
-                    zk_rows = [int.from_bytes(zk_rows[32 * j : 32 * j + 32], "little") for j in range(12 * n)]
-                if len(zk_rows) != 12 * n:
-                    raise ValueError("zk_rows must hold 12 field elements per proof")
-                zk = [0 if zeroed[j // 12] else int(v) for j, v in enumerate(zk_rows)]
+        zk = _blinding_rows([rings[k] for k in index], zk_rows)
         natives = [r.native for r in rings]
         pooled = [isinstance(x, PooledRingNative) for x in natives]
         if any(pooled) and not all(pooled):
@@ -553,6 +539,25 @@ class RingVRF(VRF):
     @classmethod
     def proof_to_hash(cls, gamma: bytes, mul_cofactor: bool = False) -> bytes:
         return PedersenVRF[cls.cv].proof_to_hash(gamma, mul_cofactor)
+
+
+def _blinding_rows(item_rings: Sequence[Ring], zk_rows):
+    """The 12 blinding rows of every item, for the item's ring: zeros where the ring has ``test_vectors=True``, else the given
+    ``zk_rows`` (ints, or 32-byte little-endian values) or fresh ``secrets.randbelow`` draws; None when every item is zeroed."""
+    n = len(item_rings)
+    zeroed = [r.params.test_vectors for r in item_rings]
+    if all(zeroed):
+        return None
+    if zk_rows is None:
+        prime = item_rings[zeroed.index(False)].params.prime
+        return [0 if z else secrets.randbelow(prime) for z in zeroed for _ in range(12)]
+    if isinstance(zk_rows, (bytes, bytearray)):
+        if len(zk_rows) != 12 * 32 * n:
+            raise ValueError("zk_rows must hold 12 field elements per proof")
+        zk_rows = [int.from_bytes(zk_rows[32 * j : 32 * j + 32], "little") for j in range(12 * n)]
+    if len(zk_rows) != 12 * n:
+        raise ValueError("zk_rows must hold 12 field elements per proof")
+    return [0 if zeroed[j // 12] else int(v) for j, v in enumerate(zk_rows)]
 
 
 class _LazyRingVRF:

@@ -187,6 +187,24 @@ int dr_ring_prove_batch(dr_ctx* ctx, dr_ring* ring, size_t n, const uint8_t* blo
 int dr_ring_prove_multi(dr_ctx* ctx, dr_ring* const* rings, size_t n_rings, const uint32_t* ring_index, size_t n, const uint8_t* blob,
                         const uint32_t* alpha_off, const uint32_t* alpha_len, const uint32_t* ad_off, const uint32_t* ad_len, const uint8_t* secret_keys32,
                         const uint32_t* producer_index, const uint8_t* zk_rows, uint8_t* proofs784, uint32_t* status);
+/* ---- bare ring proofs from a caller's blinding factor ---------------------------------------------------------------
+ * Replaces `RingProofBuilder(...).build()` (dot_ring/ring_proof/proof_builder.py:38-142) alone, without `PedersenVRF.prove`: item i proves
+ * that relation_i = PK_k + t_i * B for row k = producer_index[i] of rings[ring_index[i]], with the caller's blinding factor
+ * t_i = blinding_le32[i] (e.g. what dr_pedersen_prove_batch_ex returns, or a fresh one for a plain anonymous-membership proof).
+ *   relations_xy64[i]: PK_k + t_i * B, affine x | y, 32-byte little-endian each (the layout dr_ring_proof_verify_batch reads);
+ *   payloads592[i]: the 592-byte ring-proof payload (proof_payload.py:68-91);
+ *   zk_rows: 12 x 32 bytes per item as in dr_ring_prove_batch, NULL for zeros;
+ *   label: the transcript label; NULL or label_len == 0 means the rings' suite id (what dr_ring_prove_batch absorbs), otherwise the
+ *          transcript starts as RingRoot.verifier_transcript_prefix(label) does: label, "vk", [1]_1, [1]_2 | [tau]_2 and the three fixed
+ *          commitments (e.g. "w3f-ring-proof-test" for w3f ring-proof verifiers).  label_len <= 32, as in dr_verifier_key.
+ * The ring, SRS and suite rules of dr_ring_prove_multi apply unchanged, and results land in the caller's order.  Any row below
+ * max_ring_size is proved against the point that row holds (there is no secret key to check it against, so no status word).
+ * n == 0 returns DR_OK.  DR_EINVAL when a blinding factor is not below the Bandersnatch subgroup order, producer_index[i] >=
+ * max_ring_size of its ring, label_len > 32, or a check of dr_ring_prove_multi fails.  dr_ring_prove_phase_ms and
+ * dr_ring_prove_commit_kernel_ms report this call as they report dr_ring_prove_multi. */
+int dr_ring_proof_prove_multi(dr_ctx* ctx, dr_ring* const* rings, size_t n_rings, const uint32_t* ring_index, size_t n, const uint32_t* producer_index,
+                              const uint8_t* blinding_le32, const uint8_t* zk_rows, const uint8_t* label, size_t label_len, uint8_t* relations_xy64,
+                              uint8_t* payloads592);
 /* Per-phase device time of the last dr_ring_prove_batch / dr_ring_prove_multi on this ctx (ms, the whole call, summed over its
  * domain groups): [0] pedersen+witness, [1] interpolate, [2] commits (all MSMs), [3] LDE+constraints+quotient, [4] evaluations+openings
  * polys, [5] transcripts+assembly. */
