@@ -197,6 +197,7 @@ class VerifierKeyStruct(ctypes.Structure):
 
 
 def _put(arr, data: bytes) -> None:
+    data = bytes(data)
     if len(data) > ctypes.sizeof(arr):
         raise ValueError(f"value of {len(data)} bytes does not fit a {ctypes.sizeof(arr)}-byte field")
     ctypes.memmove(arr, data, len(data))
@@ -597,29 +598,21 @@ class RingParamsStruct(ctypes.Structure):
     ]
 
 
-def _fill(arr, data: bytes) -> None:
-    _put(arr, bytes(data))
-
-
 def make_ring_params(*, domain_size: int, omega: int, seed, blinding_base, generator, suite_id: bytes, h2c_dst: bytes, hash_name: str = "sha512", max_ring_size: int = 0,
                      padding_rows: int = 0, radix_omega: int = 0, padding_point=(0, 0)) -> RingParamsStruct:
     p = RingParamsStruct()
     p.domain_size, p.max_ring_size, p.padding_rows = domain_size, max_ring_size, padding_rows
     p.suite_id_len, p.h2c_dst_len = len(suite_id), len(h2c_dst)
     p.hash_id = HASH_IDS[hash_name]
-    _fill(p.omega, int(omega).to_bytes(32, "little"))
-    _fill(p.radix_omega, int(radix_omega).to_bytes(32, "little"))
-    _fill(p.seed, _xy(seed))
-    _fill(p.blinding_base, _xy(blinding_base))
-    _fill(p.padding_point, _xy(padding_point))
-    _fill(p.generator, _xy(generator))
-    _fill(p.suite_id, suite_id)
-    _fill(p.h2c_dst, h2c_dst)
+    _put(p.omega, int(omega).to_bytes(32, "little"))
+    _put(p.radix_omega, int(radix_omega).to_bytes(32, "little"))
+    _put(p.seed, _xy64(seed))
+    _put(p.blinding_base, _xy64(blinding_base))
+    _put(p.padding_point, _xy64(padding_point))
+    _put(p.generator, _xy64(generator))
+    _put(p.suite_id, suite_id)
+    _put(p.h2c_dst, h2c_dst)
     return p
-
-
-def _xy(pt) -> bytes:
-    return int(pt[0]).to_bytes(32, "little") + int(pt[1]).to_bytes(32, "little")
 
 
 def ring_roots_from_keys(srs: NativeSrs, params: RingParamsStruct, key_sets: list[list[bytes]]) -> list[bytes]:

@@ -283,17 +283,6 @@ void commit_device_pair(Ctx* ctx, Srs* srs, const Fr* scalars_a, size_t stride_a
 
 using namespace dr;
 
-#define DR_API_BEGIN try {
-#define DR_API_END                                   \
-    }                                                \
-    catch (const Error& e) {                         \
-        return set_error(e.code, e.what());          \
-    }                                                \
-    catch (const std::exception& e) {                \
-        return set_error(DR_ECUDA, e.what());        \
-    }                                                \
-    return DR_OK;
-
 extern "C" {
 
 const char* dr_last_error(void) { return g_last_error.c_str(); }

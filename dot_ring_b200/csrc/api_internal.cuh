@@ -263,6 +263,76 @@ inline bool same_suite(const SuiteDev& a, const SuiteDev& b) {
            a.hash_kind == b.hash_kind && a.generator == b.generator && a.blinding_base == b.blinding_base;
 }
 
+// ---- decoding of the parameter structs (dr_ring_params, dr_vrf_suite, dr_verifier_key) ----
+inline Fr fr_param(const uint8_t* b) {
+    Fr r;
+    fr_from_le_bytes_raw(r, b);
+    if (!r.is_canonical_raw()) throw Error(DR_EINVAL, "field element is not canonical");
+    return r.to_mont();
+}
+inline TEAffine te_param(const uint8_t* xy) {
+    TEAffine p{fr_param(xy), fr_param(xy + 32)};
+    if (!te_on_curve(p)) throw Error(DR_EINVAL, "point is not on the curve");
+    return p;
+}
+// The suite as dr_ring_params and dr_vrf_suite both carry it; the window tables are left to the caller.
+inline SuiteDev suite_param(uint32_t suite_id_len, const uint8_t* suite_id, uint32_t dst_len, const uint8_t* dst, uint32_t hash_id, const uint8_t* generator,
+                            const uint8_t* blinding_base) {
+    if (suite_id_len > 32 || dst_len > 64) throw Error(DR_EINVAL, "suite id / DST too long");
+    if (hash_id > 1) throw Error(DR_EINVAL, "unknown suite hash");
+    SuiteDev d{};
+    d.generator = te_param(generator);
+    d.blinding_base = te_param(blinding_base);
+    d.suite_id_len = suite_id_len;
+    memcpy(d.suite_id, suite_id, 32);
+    d.dst_len = dst_len;
+    memcpy(d.dst, dst, 64);
+    d.hash_kind = hash_id;
+    return d;
+}
+inline SuiteDev suite_param(const dr_ring_params& p) {
+    return suite_param(p.suite_id_len, p.suite_id, p.h2c_dst_len, p.h2c_dst, p.hash_id, p.generator, p.blinding_base);
+}
+inline SuiteDev suite_param(const dr_vrf_suite* s) {
+    if (!s) throw Error(DR_EINVAL, "bad suite");
+    return suite_param(s->suite_id_len, s->suite_id, s->h2c_dst_len, s->h2c_dst, s->hash_id, s->generator, s->blinding_base);
+}
+// The domain sizes a ring supports: the reference stops at 4096 (params.py:172-173); larger domains (to 2^16) run the same pipeline
+// over the two-pass NTT.
+inline void check_domain_size(uint32_t N) {
+    if (N < 512 || N > 65536 || (N & (N - 1))) throw Error(DR_EINVAL, "domain_size must be a power of two in [512, 65536]");
+}
+// omega^N == 1, omega^(N/2) != 1
+inline void check_primitive_root(const Fr& omega, uint32_t logN) {
+    Fr t = omega;
+    for (uint32_t i = 0; i + 1 < logN; i++) t = t.sqr();
+    if (t == Fr::one() || t.sqr() != Fr::one()) throw Error(DR_EINVAL, "omega is not a primitive N-th root of unity");
+}
+// w^(N-4) and the coefficients of (X - w^(N-1))(X - w^(N-2))(X - w^(N-3)), from w^-1 (omega^N == 1)
+inline void domain_tail(const Fr& omega, Fr tail[4], Fr& w_last) {
+    const Fr winv = omega.inv();
+    const Fr r1 = winv, r2 = winv * winv, r3 = r2 * winv;
+    w_last = r3 * winv;
+    tail[3] = Fr::one();
+    tail[2] = (r1 + r2 + r3).neg();
+    tail[1] = r1 * r2 + r1 * r3 + r2 * r3;
+    tail[0] = (r1 * r2 * r3).neg();
+}
+// The ring transcript after the verifier key under `label` (root.py:54-71, phases.py:72-74): label | "vk" | G1[0] | G2[0..1] | the
+// three fixed commitments, uncompressed.
+inline Shake128 ring_transcript_prefix(const uint8_t* label, uint32_t label_len, const uint8_t* g1_0_be96, const uint8_t* g2_be192, const uint8_t* fixed_be96) {
+    Shake128 tr;
+    tr.init();
+    tr.absorb(label, label_len);
+    tr.absorb_be32(label_len);
+    shake_absorb_label(tr, "vk", 2);
+    tr.absorb(g1_0_be96, 96);
+    tr.absorb(g2_be192, 384);
+    tr.absorb(fixed_be96, 288);
+    tr.absorb_be32(96 + 384 + 288);
+    return tr;
+}
+
 
 VerifierKeyDev make_verifier_key(Ctx* ctx, uint32_t N, const Fr& omega, const TEAffine& seed, const uint8_t* label, uint32_t label_len, const uint8_t* g1_0_be96,
                                  const uint8_t* g2_be192, const uint8_t* fixed_be96, std::shared_ptr<Ctx::G2Lines>& lines);
@@ -280,3 +350,15 @@ void commit_device_pair(Ctx* ctx, Srs* srs, const Fr* scalars_a, size_t stride_a
                         G1Affine* out_affine);
 
 }  // namespace dr
+
+// Body of a C ABI entry point: an exception becomes its error code (DR_ECUDA for anything but dr::Error) and dr_last_error's text.
+#define DR_API_BEGIN try {
+#define DR_API_END                                \
+    }                                             \
+    catch (const dr::Error& e) {                  \
+        return dr::set_error(e.code, e.what());   \
+    }                                             \
+    catch (const std::exception& e) {             \
+        return dr::set_error(DR_ECUDA, e.what()); \
+    }                                             \
+    return DR_OK;

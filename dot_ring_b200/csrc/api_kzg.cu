@@ -120,17 +120,6 @@ static void side_sum(Ctx* ctx, const uint8_t* pts_be96, const uint8_t* scalars_l
 
 using namespace dr;
 
-#define DR_API_BEGIN try {
-#define DR_API_END                            \
-    }                                         \
-    catch (const Error& e) {                  \
-        return set_error(e.code, e.what());   \
-    }                                         \
-    catch (const std::exception& e) {         \
-        return set_error(DR_ECUDA, e.what()); \
-    }                                         \
-    return DR_OK;
-
 extern "C" {
 
 int dr_kzg_open(dr_ctx* c, dr_srs* s, const uint8_t* coeffs_le32, size_t n, size_t batch, const uint8_t* points_le32, uint8_t* proofs_be96, uint8_t* values_le32) {

@@ -92,17 +92,6 @@ void msm_points_device(Ctx* ctx, const G1Affine* points, const uint8_t* scalars_
 
 using namespace dr;
 
-#define DR_API_BEGIN try {
-#define DR_API_END                            \
-    }                                         \
-    catch (const Error& e) {                  \
-        return set_error(e.code, e.what());   \
-    }                                         \
-    catch (const std::exception& e) {         \
-        return set_error(DR_ECUDA, e.what()); \
-    }                                         \
-    return DR_OK;
-
 static const uint8_t G1_GENERATOR_BE96[96] = {
     0x17, 0xf1, 0xd3, 0xa7, 0x31, 0x97, 0xd7, 0x94, 0x26, 0x95, 0x63, 0x8c, 0x4f, 0xa9, 0xac, 0x0f, 0xc3, 0x68, 0x8c, 0x4f, 0x97, 0x74, 0xb9, 0x05,
     0xa1, 0x4e, 0x3a, 0x3f, 0x17, 0x1b, 0xac, 0x58, 0x6c, 0x55, 0xe8, 0x3f, 0xf9, 0x7a, 0x1a, 0xef, 0xfb, 0x3a, 0xf0, 0x0a, 0xdb, 0x22, 0xc6, 0xbb,

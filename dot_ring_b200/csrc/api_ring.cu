@@ -9,32 +9,11 @@
 
 namespace dr {
 
-static Fr fr_from_param(const uint8_t* b) {
-    Fr r;
-    fr_from_le_bytes_raw(r, b);
-    if (!r.is_canonical_raw()) throw Error(DR_EINVAL, "field element is not canonical");
-    return r.to_mont();
-}
-static TEAffine te_from_param(const uint8_t* xy) {
-    TEAffine p{fr_from_param(xy), fr_from_param(xy + 32)};
-    if (!te_on_curve(p)) throw Error(DR_EINVAL, "auxiliary point is not on the curve");
-    return p;
-}
-
 // The ring's row layout: N, padding rows, and room for the 253 bit rows next to max_ring_size keys.
 static void check_ring_shape(const dr_ring_params* prm) {
-    const uint32_t N = prm->domain_size;
-    // the reference stops at 4096 (params.py:172-173); larger domains (to 2^16) run the same pipeline over the two-pass NTT
-    if (N < 512 || N > 65536 || (N & (N - 1))) throw Error(DR_EINVAL, "domain_size must be a power of two in [512, 65536]");
+    check_domain_size(prm->domain_size);
     if (prm->padding_rows != 4) throw Error(DR_EINVAL, "padding_rows must be 4 to match the 3 hidden rows");
-    if (prm->max_ring_size + SCALAR_BITS + 4 > N) throw Error(DR_EINVAL, "max_ring_size exceeds supported size for this domain");
-}
-
-// omega^N == 1, omega^(N/2) != 1
-static void check_primitive_root(const Fr& omega, uint32_t logN) {
-    Fr t = omega;
-    for (uint32_t i = 0; i + 1 < logN; i++) t = t.sqr();
-    if (t == Fr::one() || t.sqr() != Fr::one()) throw Error(DR_EINVAL, "omega is not a primitive N-th root of unity");
+    if (prm->max_ring_size + SCALAR_BITS + 4 > prm->domain_size) throw Error(DR_EINVAL, "max_ring_size exceeds supported size for this domain");
 }
 
 // The rows of the public vector PK || padding || 2^i B || zeros (members.py:36-53) that no key sets: padding below max_ring (a key
@@ -116,6 +95,7 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
                        const uint8_t* zk_rows, const ProveOutputs& res) {
     auto ring_of = [&](size_t i) { return ring_index ? ring_index[i] : 0u; };
     const bool bare = res.bare;
+    const SuiteDev& suite = rings[0]->suite;
     size_t blob_len = 0;
     std::vector<uint32_t> domains;  // distinct domain sizes of the items' rings
     for (size_t i = 0; i < n; i++) {
@@ -199,7 +179,7 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
     for (size_t g = 0, group_begin = 0; g < group_end.size(); group_begin = group_end[g++]) {
         const size_t group_n = group_end[g] - group_begin;
         auto item = [&](size_t j) -> size_t { return direct ? j : order[group_begin + j]; };
-        // everything of a pass that depends only on N or on the suite comes from the group's first ring
+        // everything of a pass that depends only on N comes from the group's first ring
         Ring* lead = rings[ring_of(item(0))];
         const RingDev& rg = lead->dev;
         const uint32_t N = rg.N;
@@ -250,13 +230,13 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
             {
                 const uint32_t per_block = tb / COOP_LANES;  // eight lanes per proof
                 if (bare) {
-                    launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, ring_proof_start_smem(tb), RingProofStartBody(), rg, dtab, (const ProveInput*)sc.in.p,
+                    launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, ring_proof_start_smem(tb), RingProofStartBody(), suite, dtab, (const ProveInput*)sc.in.p,
                            sc.st.p, m);
                 } else {
-                    launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, pedersen_start_smem(tb), PedersenStartBody(), rg, dtab, (const ProveInput*)sc.in.p,
+                    launch(ctx->stream, Dim3((m + per_block - 1) / per_block), tb, pedersen_start_smem(tb), PedersenStartBody(), suite, dtab, (const ProveInput*)sc.in.p,
                            (const uint8_t*)sc.blob.p, sc.st.p, m);
                     ctx->fork_side();
-                    launch(ctx->side, Dim3((m + 31) / 32), 32, 0, PedersenFinishBody(), rg, (const ProveInput*)sc.in.p, sc.st.p, m);
+                    launch(ctx->side, Dim3((m + 31) / 32), 32, 0, PedersenFinishBody(), suite, (const ProveInput*)sc.in.p, sc.st.p, m);
                 }
             }
             {
@@ -372,21 +352,6 @@ static void ring_prove(Ctx* ctx, Ring* const* rings, const RingTab* dtab, const 
     }
 }
 
-// The ring transcript after the verifier key (root.py:54-71, phases.py:72-74) under `label`: what dr_ring_create keeps with the ring
-// under the suite id, and dr_ring_proof_prove_multi builds per call for another label.
-static Shake128 ring_transcript_prefix(const uint8_t* label, uint32_t label_len, const Srs* srs, const uint8_t* commit_be96) {
-    Shake128 tr;
-    tr.init();
-    tr.absorb(label, label_len);
-    tr.absorb_be32(label_len);
-    shake_absorb_label(tr, "vk", 2);
-    tr.absorb(srs->g1_0_be96, 96);
-    tr.absorb(srs->g2_be192, 384);
-    tr.absorb(commit_be96, 288);
-    tr.absorb_be32(96 + 384 + 288);
-    return tr;
-}
-
 // The argument checks dr_ring_prove_multi and dr_ring_proof_prove_multi share: the rings and the ring index.
 static void check_prove_rings(Ctx* ctx, Ring* const* rings, size_t n_rings, const uint32_t* ring_index, size_t n) {
     if (n && !n_rings) throw Error(DR_EINVAL, "at least one ring is required");
@@ -422,10 +387,10 @@ static RootSetup root_setup(Ctx* ctx, Srs* srs, const dr_ring_params* prm) {
     s.N = prm->domain_size;
     while ((1u << s.logN) < s.N) s.logN++;
     s.max_ring = prm->max_ring_size;
-    s.omega = fr_from_param(prm->omega);
+    s.omega = fr_param(prm->omega);
     check_primitive_root(s.omega, s.logN);
-    s.padding = te_from_param(prm->padding_point);
-    s.blinding_base = te_from_param(prm->blinding_base);
+    s.padding = te_param(prm->padding_point);
+    s.blinding_base = te_param(prm->blinding_base);
     if (srs->ctx != ctx) throw Error(DR_EINVAL, "SRS belongs to another context");
     if (srs->n < s.N) throw Error(DR_EINVAL, "SRS too small for this domain (needs N G1 points)");
     return s;
@@ -526,17 +491,6 @@ static void ring_root_update(Ctx* ctx, Srs* srs, const RootSetup& s, const uint8
 
 using namespace dr;
 
-#define DR_API_BEGIN try {
-#define DR_API_END                            \
-    }                                         \
-    catch (const Error& e) {                  \
-        return set_error(e.code, e.what());   \
-    }                                         \
-    catch (const std::exception& e) {         \
-        return set_error(DR_ECUDA, e.what()); \
-    }                                         \
-    return DR_OK;
-
 extern "C" {
 
 int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_t* keys32, size_t n_keys, dr_ring** out) {
@@ -549,11 +503,12 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     check_ring_shape(prm);
     if (n_keys > prm->max_ring_size) throw Error(DR_EINVAL, "ring size exceeds max supported size");
     if (3 * (size_t)N + 1 > srs->n) throw Error(DR_EINVAL, "SRS too small for this domain (needs 3N+1 G1 points)");
-    if (prm->suite_id_len > 32 || prm->h2c_dst_len > 64) throw Error(DR_EINVAL, "suite id / DST too long");
 
     auto ring = std::make_unique<Ring>();
     ring->ctx = ctx;
     ring->srs = srs;
+    SuiteDev& su = ring->suite;
+    su = suite_param(*prm);
     RingDev& d = ring->dev;
     d.N = N;
     d.logN = 0;
@@ -561,26 +516,18 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     const uint32_t max_ring = prm->max_ring_size;
     ring->tab.max_ring = max_ring;
     d.last = N - 4;
-    d.omega = fr_from_param(prm->omega);
-    Fr w4 = fr_from_param(prm->radix_omega);
+    d.omega = fr_param(prm->omega);
+    Fr w4 = fr_param(prm->radix_omega);
     ring->radix_omega = w4;
     // sanity: w4^4 == omega, omega^N == 1, omega^(N/2) != 1
     if (w4.sqr().sqr() != d.omega) throw Error(DR_EINVAL, "radix_omega^4 != omega");
     check_primitive_root(d.omega, d.logN);
-    d.seed = te_from_param(prm->seed);
-    d.blinding_base = te_from_param(prm->blinding_base);
-    d.generator = te_from_param(prm->generator);
-    ring->g_table = ctx->fixed_table(d.generator);
-    ring->b_table = ctx->fixed_table(d.blinding_base);
-    d.g_tab = ring->g_table->tab.p;
-    d.b_tab = ring->b_table->tab.p;
-    ring->padding = te_from_param(prm->padding_point);
-    d.suite_id_len = prm->suite_id_len;
-    memcpy(d.suite_id, prm->suite_id, 32);
-    d.dst_len = prm->h2c_dst_len;
-    memcpy(d.dst, prm->h2c_dst, 64);
-    if (prm->hash_id > 1) throw Error(DR_EINVAL, "unknown suite hash");
-    d.hash_kind = prm->hash_id;
+    d.seed = te_param(prm->seed);
+    ring->g_table = ctx->fixed_table(su.generator);
+    ring->b_table = ctx->fixed_table(su.blinding_base);
+    su.g_tab = ring->g_table->tab.p;
+    su.b_tab = ring->b_table->tab.p;
+    ring->padding = te_param(prm->padding_point);
     d.n_inv = Fr::from_u32(N).inv();
     d.quarter = Fr::from_u32(4).inv();
 
@@ -605,20 +552,12 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     h2d(ctx->stream, ring->w4inv.p, hw4i.data(), 4 * N * sizeof(Fr));
     d.w4 = ring->w4.p;
     d.w4inv = ring->w4inv.p;
-    d.w_last = hw4[4 * (N - 4)];
-    {
-        // (X - w^(N-1))(X - w^(N-2))(X - w^(N-3))
-        Fr r1 = hw4[4 * (N - 1)], r2 = hw4[4 * (N - 2)], r3 = hw4[4 * (N - 3)];
-        d.tail[3] = Fr::one();
-        d.tail[2] = (r1 + r2 + r3).neg();
-        d.tail[1] = r1 * r2 + r1 * r3 + r2 * r3;
-        d.tail[0] = (r1 * r2 * r3).neg();
-    }
+    domain_tail(d.omega, d.tail, d.w_last);
 
     // ---- public vector PK || padding || 2^i B || zeros (members.py:36-53) ----
     ring->nm.alloc(N);
     {
-        std::vector<TEAffine> host = public_vector_rows(N, max_ring, ring->padding, d.blinding_base);
+        std::vector<TEAffine> host = public_vector_rows(N, max_ring, ring->padding, su.blinding_base);
         h2d(ctx->stream, ring->nm.p, host.data(), N * sizeof(TEAffine));
         if (n_keys) {
             DevBuf<uint8_t> kraw(n_keys * 32);
@@ -670,29 +609,16 @@ int dr_ring_create(dr_ctx* c, dr_srs* s, const dr_ring_params* prm, const uint8_
     }
     ring->tab.fixed_lde = ring->fixed_lde.p;
 
-    // ---- verifier-key transcript prefix (root.py:54-71, phases.py:72-74) ----
-    {
-        const Shake128 tr = ring_transcript_prefix(d.suite_id, d.suite_id_len, srs, ring->commit_be96);
-        ring->prefix.alloc(1);
-        h2d(ctx->stream, ring->prefix.p, &tr, sizeof(Shake128));
-        ring->tab.prefix = ring->prefix.p;
-        ring->tab_dev.alloc(1);
-        h2d(ctx->stream, ring->tab_dev.p, &ring->tab, sizeof(RingTab));
-        stream_sync(ctx->stream);
-    }
-    ring->vk = make_verifier_key(ctx, N, d.omega, d.seed, d.suite_id, d.suite_id_len, srs->g1_0_be96, srs->g2_be192, ring->commit_be96, ring->vk_lines);
+    // ---- verifier key; the prover starts from its transcript prefix under the suite id ----
+    ring->vk = make_verifier_key(ctx, N, d.omega, d.seed, su.suite_id, su.suite_id_len, srs->g1_0_be96, srs->g2_be192, ring->commit_be96, ring->vk_lines);
     ring->vk_dev.alloc(1);
     h2d(ctx->stream, ring->vk_dev.p, &ring->vk, sizeof(VerifierKeyDev));
+    ring->prefix.alloc(1);
+    h2d(ctx->stream, ring->prefix.p, &ring->vk.prefix, sizeof(Shake128));
+    ring->tab.prefix = ring->prefix.p;
+    ring->tab_dev.alloc(1);
+    h2d(ctx->stream, ring->tab_dev.p, &ring->tab, sizeof(RingTab));
     stream_sync(ctx->stream);
-    ring->suite.generator = d.generator;
-    ring->suite.blinding_base = d.blinding_base;
-    ring->suite.g_tab = d.g_tab;
-    ring->suite.b_tab = d.b_tab;
-    ring->suite.suite_id_len = d.suite_id_len;
-    memcpy(ring->suite.suite_id, d.suite_id, 32);
-    ring->suite.dst_len = d.dst_len;
-    memcpy(ring->suite.dst, d.dst, 64);
-    ring->suite.hash_kind = d.hash_kind;
     *out = (dr_ring*)ring.release();
     DR_API_END
 }
@@ -831,10 +757,11 @@ int dr_ring_proof_prove_multi(dr_ctx* c, dr_ring* const* rs, size_t n_rings, con
     for (size_t k = 0; k < n_rings; k++) table[k] = rings[k]->tab;
     // another label than the suite id: one transcript prefix per ring of the call, pointed at by this call's copy of the table
     DevBuf<Shake128> prefixes;
-    const RingDev& lead = rings[0]->dev;
-    if (label_len && !(label_len == lead.suite_id_len && !memcmp(label, lead.suite_id, label_len))) {
+    const SuiteDev& suite = rings[0]->suite;
+    if (label_len && !(label_len == suite.suite_id_len && !memcmp(label, suite.suite_id, label_len))) {
         std::vector<Shake128> host(n_rings);
-        for (size_t k = 0; k < n_rings; k++) host[k] = ring_transcript_prefix(label, (uint32_t)label_len, rings[k]->srs, rings[k]->commit_be96);
+        for (size_t k = 0; k < n_rings; k++)
+            host[k] = ring_transcript_prefix(label, (uint32_t)label_len, rings[k]->srs->g1_0_be96, rings[k]->srs->g2_be192, rings[k]->commit_be96);
         prefixes.alloc(n_rings);
         h2d(ctx->stream, prefixes.p, host.data(), n_rings * sizeof(Shake128));
         for (size_t k = 0; k < n_rings; k++) table[k].prefix = prefixes.p + k;

@@ -191,49 +191,44 @@ extern "C" {
 // field: 0 = Fq (48-byte big-endian), 1 = Fr, 2 = Fn (32-byte little-endian).  op: 0 mul, 1 add, 2 sub,
 // 3 inv(a), 4 sqr(a), 5 neg(a).  Inputs must be canonical.
 int dr_field_op(dr_ctx* c, int field, int op, const uint8_t* a, const uint8_t* b, uint8_t* out, size_t count) {
-    try {
-        Ctx* ctx = (Ctx*)c;
-        if (!ctx || !a || !b || !out || field < 0 || field > 2 || op < 0 || op > 5) throw Error(DR_EINVAL, "bad argument");
-        ctx->activate();
-        if (!count) return DR_OK;
-        uint32_t blocks = (uint32_t)((count + 127) / 128);
-        if (field == 0) {
-            std::vector<Fq> ha(count), hb(count), ho(count);
-            for (size_t i = 0; i < count; i++) {
-                fq_from_be_bytes_raw(ha[i], a + 48 * i);
-                fq_from_be_bytes_raw(hb[i], b + 48 * i);
-                if (!ha[i].is_canonical_raw() || !hb[i].is_canonical_raw()) throw Error(DR_EINVAL, "operand is not canonical");
-            }
-            DevBuf<Fq> da(count), db(count), dout(count);
-            h2d(ctx->stream, da.p, ha.data(), count * sizeof(Fq));
-            h2d(ctx->stream, db.p, hb.data(), count * sizeof(Fq));
-            launch(ctx->stream, Dim3(blocks), 128, 0, FieldOpBody<Fq>(), op, (const Fq*)da.p, (const Fq*)db.p, dout.p, (uint32_t)count);
-            d2h(ctx->stream, ho.data(), dout.p, count * sizeof(Fq));
-            stream_sync(ctx->stream);
-            for (size_t i = 0; i < count; i++) fq_to_be_bytes_raw(out + 48 * i, ho[i]);
-        } else {
-            std::vector<Fr> ha(count), hb(count), ho(count);
-            for (size_t i = 0; i < count; i++) {
-                fr_from_le_bytes_raw(ha[i], a + 32 * i);
-                fr_from_le_bytes_raw(hb[i], b + 32 * i);
-            }
-            DevBuf<Fr> da(count), db(count), dout(count);
-            h2d(ctx->stream, da.p, ha.data(), count * sizeof(Fr));
-            h2d(ctx->stream, db.p, hb.data(), count * sizeof(Fr));
-            if (field == 1)
-                launch(ctx->stream, Dim3(blocks), 128, 0, FieldOpBody<Fr>(), op, (const Fr*)da.p, (const Fr*)db.p, dout.p, (uint32_t)count);
-            else
-                launch(ctx->stream, Dim3(blocks), 128, 0, FieldOpBody<Fn>(), op, (const Fn*)da.p, (const Fn*)db.p, (Fn*)dout.p, (uint32_t)count);
-            d2h(ctx->stream, ho.data(), dout.p, count * sizeof(Fr));
-            stream_sync(ctx->stream);
-            for (size_t i = 0; i < count; i++) fr_to_le_bytes_raw(out + 32 * i, ho[i]);
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || !a || !b || !out || field < 0 || field > 2 || op < 0 || op > 5) throw Error(DR_EINVAL, "bad argument");
+    ctx->activate();
+    if (!count) return DR_OK;
+    uint32_t blocks = (uint32_t)((count + 127) / 128);
+    if (field == 0) {
+        std::vector<Fq> ha(count), hb(count), ho(count);
+        for (size_t i = 0; i < count; i++) {
+            fq_from_be_bytes_raw(ha[i], a + 48 * i);
+            fq_from_be_bytes_raw(hb[i], b + 48 * i);
+            if (!ha[i].is_canonical_raw() || !hb[i].is_canonical_raw()) throw Error(DR_EINVAL, "operand is not canonical");
         }
-    } catch (const Error& e) {
-        return set_error(e.code, e.what());
-    } catch (const std::exception& e) {
-        return set_error(DR_ECUDA, e.what());
+        DevBuf<Fq> da(count), db(count), dout(count);
+        h2d(ctx->stream, da.p, ha.data(), count * sizeof(Fq));
+        h2d(ctx->stream, db.p, hb.data(), count * sizeof(Fq));
+        launch(ctx->stream, Dim3(blocks), 128, 0, FieldOpBody<Fq>(), op, (const Fq*)da.p, (const Fq*)db.p, dout.p, (uint32_t)count);
+        d2h(ctx->stream, ho.data(), dout.p, count * sizeof(Fq));
+        stream_sync(ctx->stream);
+        for (size_t i = 0; i < count; i++) fq_to_be_bytes_raw(out + 48 * i, ho[i]);
+    } else {
+        std::vector<Fr> ha(count), hb(count), ho(count);
+        for (size_t i = 0; i < count; i++) {
+            fr_from_le_bytes_raw(ha[i], a + 32 * i);
+            fr_from_le_bytes_raw(hb[i], b + 32 * i);
+        }
+        DevBuf<Fr> da(count), db(count), dout(count);
+        h2d(ctx->stream, da.p, ha.data(), count * sizeof(Fr));
+        h2d(ctx->stream, db.p, hb.data(), count * sizeof(Fr));
+        if (field == 1)
+            launch(ctx->stream, Dim3(blocks), 128, 0, FieldOpBody<Fr>(), op, (const Fr*)da.p, (const Fr*)db.p, dout.p, (uint32_t)count);
+        else
+            launch(ctx->stream, Dim3(blocks), 128, 0, FieldOpBody<Fn>(), op, (const Fn*)da.p, (const Fn*)db.p, (Fn*)dout.p, (uint32_t)count);
+        d2h(ctx->stream, ho.data(), dout.p, count * sizeof(Fr));
+        stream_sync(ctx->stream);
+        for (size_t i = 0; i < count; i++) fr_to_le_bytes_raw(out + 32 * i, ho[i]);
     }
-    return DR_OK;
+    DR_API_END
 }
 
 // kind: 0 IMAD (32-bit mad.lo), 1 IMAD.WIDE (32x32+64), 2 Fq mul, 3 Fr mul, 4 G1 mixed add, 5 DFMA, 6 IMAD + DFMA interleaved (2 : 1),
@@ -245,69 +240,64 @@ int dr_microbench(dr_ctx* c, int kind, int iters, double* ops_per_s, float* ms_o
     (void)c; (void)kind; (void)iters; (void)ops_per_s; (void)ms_out;
     return set_error(DR_ESTATE, "micro-benchmarks need the CUDA build");
 #else
-    try {
-        Ctx* ctx = (Ctx*)c;
-        if (!ctx || iters <= 0 || !ops_per_s) throw Error(DR_EINVAL, "bad argument");
-        ctx->activate();
-        cudaDeviceProp prop;
-        DR_CUDA(cudaGetDeviceProperties(&prop, ctx->device));
-        // kinds 7..10 measure latency: one warp per SM, so nothing hides the dependent chain
-        const bool latency = kind >= 7 && kind <= 10;
-        const int threads = latency ? 32 : 256;
-        const int blocks = prop.multiProcessorCount * (latency ? 1 : (kind >= 2 && kind <= 4) || kind >= 11 ? 2 : 8);
-        size_t nthreads = (size_t)blocks * threads;
-        DevBuf<uint8_t> out(nthreads * sizeof(G1));
-        DevBuf<G1Affine> pts;
-        if (kind == 4) {
-            // a few hundred distinct multiples of the generator as operands
-            std::vector<G1Affine> h(256);
-            uint8_t gen[96] = {0x17, 0xf1, 0xd3, 0xa7, 0x31, 0x97, 0xd7, 0x94, 0x26, 0x95, 0x63, 0x8c, 0x4f, 0xa9, 0xac, 0x0f, 0xc3, 0x68, 0x8c, 0x4f, 0x97, 0x74, 0xb9, 0x05,
-                               0xa1, 0x4e, 0x3a, 0x3f, 0x17, 0x1b, 0xac, 0x58, 0x6c, 0x55, 0xe8, 0x3f, 0xf9, 0x7a, 0x1a, 0xef, 0xfb, 0x3a, 0xf0, 0x0a, 0xdb, 0x22, 0xc6, 0xbb,
-                               0x08, 0xb3, 0xf4, 0x81, 0xe3, 0xaa, 0xa0, 0xf1, 0xa0, 0x9e, 0x30, 0xed, 0x74, 0x1d, 0x8a, 0xe4, 0xfc, 0xf5, 0xe0, 0x95, 0xd5, 0xd0, 0x0a, 0xf6,
-                               0x00, 0xdb, 0x18, 0xcb, 0x2c, 0x04, 0xb3, 0xed, 0xd0, 0x3c, 0xc7, 0x44, 0xa2, 0x88, 0x8a, 0xe4, 0x0c, 0xaa, 0x23, 0x29, 0x46, 0xc5, 0xe7, 0xe1};
-            G1Affine g;
-            if (!g1_decode(g, gen, 96)) throw Error(DR_ESTATE, "generator decode failed");
-            G1 acc = G1::from_affine(g);
-            for (auto& p : h) {
-                acc = g1_dbl(acc);
-                g1_madd(acc, g);
-                p = g1_to_affine(acc);
-            }
-            pts.alloc(h.size());
-            h2d(ctx->stream, pts.p, h.data(), h.size() * sizeof(G1Affine));
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || iters <= 0 || !ops_per_s) throw Error(DR_EINVAL, "bad argument");
+    ctx->activate();
+    cudaDeviceProp prop;
+    DR_CUDA(cudaGetDeviceProperties(&prop, ctx->device));
+    // kinds 7..10 measure latency: one warp per SM, so nothing hides the dependent chain
+    const bool latency = kind >= 7 && kind <= 10;
+    const int threads = latency ? 32 : 256;
+    const int blocks = prop.multiProcessorCount * (latency ? 1 : (kind >= 2 && kind <= 4) || kind >= 11 ? 2 : 8);
+    size_t nthreads = (size_t)blocks * threads;
+    DevBuf<uint8_t> out(nthreads * sizeof(G1));
+    DevBuf<G1Affine> pts;
+    if (kind == 4) {
+        // a few hundred distinct multiples of the generator as operands
+        std::vector<G1Affine> h(256);
+        uint8_t gen[96] = {0x17, 0xf1, 0xd3, 0xa7, 0x31, 0x97, 0xd7, 0x94, 0x26, 0x95, 0x63, 0x8c, 0x4f, 0xa9, 0xac, 0x0f, 0xc3, 0x68, 0x8c, 0x4f, 0x97, 0x74, 0xb9, 0x05,
+                           0xa1, 0x4e, 0x3a, 0x3f, 0x17, 0x1b, 0xac, 0x58, 0x6c, 0x55, 0xe8, 0x3f, 0xf9, 0x7a, 0x1a, 0xef, 0xfb, 0x3a, 0xf0, 0x0a, 0xdb, 0x22, 0xc6, 0xbb,
+                           0x08, 0xb3, 0xf4, 0x81, 0xe3, 0xaa, 0xa0, 0xf1, 0xa0, 0x9e, 0x30, 0xed, 0x74, 0x1d, 0x8a, 0xe4, 0xfc, 0xf5, 0xe0, 0x95, 0xd5, 0xd0, 0x0a, 0xf6,
+                           0x00, 0xdb, 0x18, 0xcb, 0x2c, 0x04, 0xb3, 0xed, 0xd0, 0x3c, 0xc7, 0x44, 0xa2, 0x88, 0x8a, 0xe4, 0x0c, 0xaa, 0x23, 0x29, 0x46, 0xc5, 0xe7, 0xe1};
+        G1Affine g;
+        if (!g1_decode(g, gen, 96)) throw Error(DR_ESTATE, "generator decode failed");
+        G1 acc = G1::from_affine(g);
+        for (auto& p : h) {
+            acc = g1_dbl(acc);
+            g1_madd(acc, g);
+            p = g1_to_affine(acc);
         }
-        double per_thread = 0;
-        for (int rep = 0; rep < 2; rep++) {  // first repetition warms up
-            dr_ctx_timer_start(c);
-            switch (kind) {
-                case 0: mb_imad32<<<blocks, threads, 0, ctx->stream>>>((uint32_t*)out.p, 12345u, iters); per_thread = 64.0 * iters; break;
-                case 1: mb_imad_wide<<<blocks, threads, 0, ctx->stream>>>((uint64_t*)out.p, 12345u, iters); per_thread = 64.0 * iters; break;
-                case 2: mb_field_mul<Fq><<<blocks, threads, 0, ctx->stream>>>((Fq*)out.p, 12345u, iters); per_thread = 4.0 * iters; break;
-                case 3: mb_field_mul<Fr><<<blocks, threads, 0, ctx->stream>>>((Fr*)out.p, 12345u, iters); per_thread = 4.0 * iters; break;
-                case 4: mb_g1_madd<<<blocks, threads, 0, ctx->stream>>>((G1*)out.p, pts.p, 256u, iters); per_thread = 1.0 * iters; break;
-                case 5: mb_dfma<<<blocks, threads, 0, ctx->stream>>>((double*)out.p, 12345u, iters); per_thread = 64.0 * iters; break;
-                case 6: mb_imad_dfma<<<blocks, threads, 0, ctx->stream>>>((double*)out.p, 12345u, iters); per_thread = 96.0 * iters; break;  // 64 IMAD + 32 DFMA
-                case 7: mb_field_chain<Fr><<<blocks, threads, 0, ctx->stream>>>((Fr*)out.p, 12345u, iters); per_thread = 1.0 * iters; break;
-                case 8: mb_field_chain<Fq><<<blocks, threads, 0, ctx->stream>>>((Fq*)out.p, 12345u, iters); per_thread = 1.0 * iters; break;
-                case 9: mb_field_inv<Fr><<<blocks, threads, 0, ctx->stream>>>((Fr*)out.p, 12345u, iters); per_thread = 1.0 * iters; break;
-                case 10: mb_field_inv<Fq><<<blocks, threads, 0, ctx->stream>>>((Fq*)out.p, 12345u, iters); per_thread = 1.0 * iters; break;
-                case 11: mb_field_sqr<Fq><<<blocks, threads, 0, ctx->stream>>>((Fq*)out.p, 12345u, iters); per_thread = 4.0 * iters; break;
-                case 12: mb_field_sqr<Fr><<<blocks, threads, 0, ctx->stream>>>((Fr*)out.p, 12345u, iters); per_thread = 4.0 * iters; break;
-                default: throw Error(DR_EINVAL, "unknown micro-benchmark");
-            }
-            DR_CUDA(cudaGetLastError());
-            launch_counter()++;
-            float ms = 0;
-            dr_ctx_timer_stop(c, &ms);
-            if (ms_out) *ms_out = ms;
-            *ops_per_s = per_thread * (double)nthreads / (ms * 1e-3);
-        }
-    } catch (const Error& e) {
-        return set_error(e.code, e.what());
-    } catch (const std::exception& e) {
-        return set_error(DR_ECUDA, e.what());
+        pts.alloc(h.size());
+        h2d(ctx->stream, pts.p, h.data(), h.size() * sizeof(G1Affine));
     }
-    return DR_OK;
+    double per_thread = 0;
+    for (int rep = 0; rep < 2; rep++) {  // first repetition warms up
+        dr_ctx_timer_start(c);
+        switch (kind) {
+            case 0: mb_imad32<<<blocks, threads, 0, ctx->stream>>>((uint32_t*)out.p, 12345u, iters); per_thread = 64.0 * iters; break;
+            case 1: mb_imad_wide<<<blocks, threads, 0, ctx->stream>>>((uint64_t*)out.p, 12345u, iters); per_thread = 64.0 * iters; break;
+            case 2: mb_field_mul<Fq><<<blocks, threads, 0, ctx->stream>>>((Fq*)out.p, 12345u, iters); per_thread = 4.0 * iters; break;
+            case 3: mb_field_mul<Fr><<<blocks, threads, 0, ctx->stream>>>((Fr*)out.p, 12345u, iters); per_thread = 4.0 * iters; break;
+            case 4: mb_g1_madd<<<blocks, threads, 0, ctx->stream>>>((G1*)out.p, pts.p, 256u, iters); per_thread = 1.0 * iters; break;
+            case 5: mb_dfma<<<blocks, threads, 0, ctx->stream>>>((double*)out.p, 12345u, iters); per_thread = 64.0 * iters; break;
+            case 6: mb_imad_dfma<<<blocks, threads, 0, ctx->stream>>>((double*)out.p, 12345u, iters); per_thread = 96.0 * iters; break;  // 64 IMAD + 32 DFMA
+            case 7: mb_field_chain<Fr><<<blocks, threads, 0, ctx->stream>>>((Fr*)out.p, 12345u, iters); per_thread = 1.0 * iters; break;
+            case 8: mb_field_chain<Fq><<<blocks, threads, 0, ctx->stream>>>((Fq*)out.p, 12345u, iters); per_thread = 1.0 * iters; break;
+            case 9: mb_field_inv<Fr><<<blocks, threads, 0, ctx->stream>>>((Fr*)out.p, 12345u, iters); per_thread = 1.0 * iters; break;
+            case 10: mb_field_inv<Fq><<<blocks, threads, 0, ctx->stream>>>((Fq*)out.p, 12345u, iters); per_thread = 1.0 * iters; break;
+            case 11: mb_field_sqr<Fq><<<blocks, threads, 0, ctx->stream>>>((Fq*)out.p, 12345u, iters); per_thread = 4.0 * iters; break;
+            case 12: mb_field_sqr<Fr><<<blocks, threads, 0, ctx->stream>>>((Fr*)out.p, 12345u, iters); per_thread = 4.0 * iters; break;
+            default: throw Error(DR_EINVAL, "unknown micro-benchmark");
+        }
+        DR_CUDA(cudaGetLastError());
+        launch_counter()++;
+        float ms = 0;
+        dr_ctx_timer_stop(c, &ms);
+        if (ms_out) *ms_out = ms;
+        *ops_per_s = per_thread * (double)nthreads / (ms * 1e-3);
+    }
+    DR_API_END
 #endif
 }
 }

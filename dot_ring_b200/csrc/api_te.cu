@@ -100,77 +100,62 @@ extern "C" {
 // for a batch: ok[i] = 0 <=> the reference raises ValueError.  checked != 0 adds the non-identity
 // prime-subgroup test of `Curve.valid_point` (curve/curve.py:56-67).
 int dr_te_decode_batch(dr_ctx* c, const uint8_t* in32, size_t n, int checked, uint8_t* out_xy64, uint8_t* ok) {
-    try {
-        Ctx* ctx = (Ctx*)c;
-        if (!ctx || (n && (!in32 || !out_xy64 || !ok))) throw Error(DR_EINVAL, "bad argument");
-        ctx->activate();
-        if (!n) return DR_OK;
-        DevBuf<uint8_t> din(n * 32), dout(n * 64), dok(n);
-        h2d(ctx->stream, din.p, in32, n * 32);
-        launch(ctx->stream, Dim3((uint32_t)((n + 63) / 64)), 64, 0, TeDecodeBody(), (const uint8_t*)din.p, (uint32_t)n, checked, dout.p, dok.p);
-        d2h(ctx->stream, out_xy64, dout.p, n * 64);
-        d2h(ctx->stream, ok, dok.p, n);
-        stream_sync(ctx->stream);
-    } catch (const Error& e) {
-        return set_error(e.code, e.what());
-    } catch (const std::exception& e) {
-        return set_error(DR_ECUDA, e.what());
-    }
-    return DR_OK;
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || (n && (!in32 || !out_xy64 || !ok))) throw Error(DR_EINVAL, "bad argument");
+    ctx->activate();
+    if (!n) return DR_OK;
+    DevBuf<uint8_t> din(n * 32), dout(n * 64), dok(n);
+    h2d(ctx->stream, din.p, in32, n * 32);
+    launch(ctx->stream, Dim3((uint32_t)((n + 63) / 64)), 64, 0, TeDecodeBody(), (const uint8_t*)din.p, (uint32_t)n, checked, dout.p, dok.p);
+    d2h(ctx->stream, out_xy64, dout.p, n * 64);
+    d2h(ctx->stream, ok, dok.p, n);
+    stream_sync(ctx->stream);
+    DR_API_END
 }
 
 // Replaces `BandersnatchPoint.__mul__` (dot_ring/curve/specs/bandersnatch.py:177-191) for a batch:
 // out[i] = (scalars[i] mod order) * points[i]  (or * points[0] when n_points == 1), 32-byte encodings.
 int dr_te_mul_batch(dr_ctx* c, const uint8_t* points32, size_t n_points, const uint8_t* scalars32, size_t n, uint8_t* out32, uint8_t* ok) {
-    try {
-        Ctx* ctx = (Ctx*)c;
-        if (!ctx || (n && (!points32 || !scalars32 || !out32 || !ok)) || (n_points != 1 && n_points != n)) throw Error(DR_EINVAL, "bad argument");
-        ctx->activate();
-        if (!n) return DR_OK;
-        DevBuf<uint8_t> dp(n_points * 32), dk(n * 32), dout(n * 32), dok(n);
-        h2d(ctx->stream, dp.p, points32, n_points * 32);
-        h2d(ctx->stream, dk.p, scalars32, n * 32);
-        launch(ctx->stream, Dim3((uint32_t)((n + 63) / 64)), 64, 0, TeMulBody(), (const uint8_t*)dp.p, (uint32_t)n_points, (const uint8_t*)dk.p, (uint32_t)n, dout.p, dok.p);
-        d2h(ctx->stream, out32, dout.p, n * 32);
-        d2h(ctx->stream, ok, dok.p, n);
-        dev_zero(ctx->stream, dk.p, n * 32);  // the scalars may be secret keys (public-key derivation); the block is recycled
-        stream_sync(ctx->stream);
-    } catch (const Error& e) {
-        return set_error(e.code, e.what());
-    } catch (const std::exception& e) {
-        return set_error(DR_ECUDA, e.what());
-    }
-    return DR_OK;
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || (n && (!points32 || !scalars32 || !out32 || !ok)) || (n_points != 1 && n_points != n)) throw Error(DR_EINVAL, "bad argument");
+    ctx->activate();
+    if (!n) return DR_OK;
+    DevBuf<uint8_t> dp(n_points * 32), dk(n * 32), dout(n * 32), dok(n);
+    h2d(ctx->stream, dp.p, points32, n_points * 32);
+    h2d(ctx->stream, dk.p, scalars32, n * 32);
+    launch(ctx->stream, Dim3((uint32_t)((n + 63) / 64)), 64, 0, TeMulBody(), (const uint8_t*)dp.p, (uint32_t)n_points, (const uint8_t*)dk.p, (uint32_t)n, dout.p, dok.p);
+    d2h(ctx->stream, out32, dout.p, n * 32);
+    d2h(ctx->stream, ok, dok.p, n);
+    dev_zero(ctx->stream, dk.p, n * 32);  // the scalars may be secret keys (public-key derivation); the block is recycled
+    stream_sync(ctx->stream);
+    DR_API_END
 }
 
 // Replaces `BandersnatchPoint.msm` (dot_ring/curve/specs/bandersnatch.py:194-286: GLV joint windows for n <= 3,
 // `msm_pippenger_signed_native_cy` above; native_field/bandersnatch_te.pyx:257-418): out = sum_i (scalars[i] mod order) * points[i].
 // Every point is one thread's windowed multiplication, the partial sums are tree-folded.  DR_EINVAL on an undecodable point.
 int dr_te_msm(dr_ctx* c, const uint8_t* points32, const uint8_t* scalars32, size_t n, uint8_t out32[32]) {
-    try {
-        Ctx* ctx = (Ctx*)c;
-        if (!ctx || !out32 || (n && (!points32 || !scalars32))) throw Error(DR_EINVAL, "bad argument");
-        ctx->activate();
-        const uint32_t threads = 64;
-        const uint32_t blocks = n ? (uint32_t)((n + threads - 1) / threads) : 1;
-        DevBuf<uint8_t> dp(n ? n * 32 : 32), dk(n ? n * 32 : 32), dout(32);
-        DevBuf<TEExt> partial(blocks);
-        DevBuf<uint32_t> bad(1);
-        dev_zero(ctx->stream, bad.p, 4);
-        h2d(ctx->stream, dp.p, points32, n * 32);
-        h2d(ctx->stream, dk.p, scalars32, n * 32);
-        launch(ctx->stream, Dim3(blocks), threads, threads * sizeof(TEExt), TeMsmBody(), (const uint8_t*)dp.p, (const uint8_t*)dk.p, (uint32_t)n, partial.p, bad.p);
-        launch(ctx->stream, Dim3(1), threads, threads * sizeof(TEExt), TeMsmFinishBody(), (const TEExt*)partial.p, blocks, dout.p);
-        uint32_t bad_h = 0;
-        d2h(ctx->stream, &bad_h, bad.p, 4);
-        d2h(ctx->stream, out32, dout.p, 32);
-        stream_sync(ctx->stream);
-        if (bad_h) throw Error(DR_EINVAL, "Invalid point encoding");
-    } catch (const Error& e) {
-        return set_error(e.code, e.what());
-    } catch (const std::exception& e) {
-        return set_error(DR_ECUDA, e.what());
-    }
-    return DR_OK;
+    DR_API_BEGIN
+    Ctx* ctx = (Ctx*)c;
+    if (!ctx || !out32 || (n && (!points32 || !scalars32))) throw Error(DR_EINVAL, "bad argument");
+    ctx->activate();
+    const uint32_t threads = 64;
+    const uint32_t blocks = n ? (uint32_t)((n + threads - 1) / threads) : 1;
+    DevBuf<uint8_t> dp(n ? n * 32 : 32), dk(n ? n * 32 : 32), dout(32);
+    DevBuf<TEExt> partial(blocks);
+    DevBuf<uint32_t> bad(1);
+    dev_zero(ctx->stream, bad.p, 4);
+    h2d(ctx->stream, dp.p, points32, n * 32);
+    h2d(ctx->stream, dk.p, scalars32, n * 32);
+    launch(ctx->stream, Dim3(blocks), threads, threads * sizeof(TEExt), TeMsmBody(), (const uint8_t*)dp.p, (const uint8_t*)dk.p, (uint32_t)n, partial.p, bad.p);
+    launch(ctx->stream, Dim3(1), threads, threads * sizeof(TEExt), TeMsmFinishBody(), (const TEExt*)partial.p, blocks, dout.p);
+    uint32_t bad_h = 0;
+    d2h(ctx->stream, &bad_h, bad.p, 4);
+    d2h(ctx->stream, out32, dout.p, 32);
+    stream_sync(ctx->stream);
+    if (bad_h) throw Error(DR_EINVAL, "Invalid point encoding");
+    DR_API_END
 }
 }

@@ -48,18 +48,8 @@ VerifierKeyDev make_verifier_key(Ctx* ctx, uint32_t N, const Fr& omega, const TE
     vk.logN = 0;
     while ((1u << vk.logN) < N) vk.logN++;
     vk.omega = omega;
-    {
-        Fr t = omega;
-        for (uint32_t i = 0; i + 1 < vk.logN; i++) t = t.sqr();
-        if (t == Fr::one() || t.sqr() != Fr::one()) throw Error(DR_EINVAL, "omega is not a primitive N-th root of unity");
-    }
-    Fr winv = omega.inv();
-    Fr r1 = winv, r2 = winv * winv, r3 = r2 * winv;  // w^(N-1), w^(N-2), w^(N-3)
-    vk.w_last = r3 * winv;
-    vk.tail[3] = Fr::one();
-    vk.tail[2] = (r1 + r2 + r3).neg();
-    vk.tail[1] = r1 * r2 + r1 * r3 + r2 * r3;
-    vk.tail[0] = (r1 * r2 * r3).neg();
+    check_primitive_root(omega, vk.logN);
+    domain_tail(omega, vk.tail, vk.w_last);
     vk.n_inv = Fr::from_u32(N).inv();
     vk.seed = seed;
     for (int i = 0; i < 3; i++)
@@ -70,42 +60,8 @@ VerifierKeyDev make_verifier_key(Ctx* ctx, uint32_t N, const Fr& omega, const TE
     vk.pc = ctx->pairing_consts();
     lines = ctx->pairing_lines(g2_be192, vk.g2);  // once per context and G2 pair
     vk.lines = lines->lines.p;
-    // transcript prefix (root.py:54-71, phases.py:72-74): label | "vk" | G1[0] | G2[0..1] | 3 fixed commitments
-    Shake128 tr;
-    tr.init();
-    tr.absorb(label, label_len);
-    tr.absorb_be32(label_len);
-    shake_absorb_label(tr, "vk", 2);
-    tr.absorb(g1_0_be96, 96);
-    tr.absorb(g2_be192, 384);
-    tr.absorb(fixed_be96, 288);
-    tr.absorb_be32(96 + 384 + 288);
-    vk.prefix = tr;
+    vk.prefix = ring_transcript_prefix(label, label_len, g1_0_be96, g2_be192, fixed_be96);
     return vk;
-}
-
-static Fr fr_param(const uint8_t* b) {
-    Fr r;
-    fr_from_le_bytes_raw(r, b);
-    if (!r.is_canonical_raw()) throw Error(DR_EINVAL, "field element is not canonical");
-    return r.to_mont();
-}
-static TEAffine te_param(const uint8_t* xy) {
-    TEAffine p{fr_param(xy), fr_param(xy + 32)};
-    if (!te_on_curve(p)) throw Error(DR_EINVAL, "point is not on the curve");
-    return p;
-}
-static SuiteDev suite_from_abi(const dr_vrf_suite* s) {
-    if (!s || s->suite_id_len > 32 || s->h2c_dst_len > 64 || s->hash_id > 1) throw Error(DR_EINVAL, "bad suite");
-    SuiteDev d{};
-    d.generator = te_param(s->generator);
-    d.blinding_base = te_param(s->blinding_base);
-    d.suite_id_len = s->suite_id_len;
-    memcpy(d.suite_id, s->suite_id, 32);
-    d.dst_len = s->h2c_dst_len;
-    memcpy(d.dst, s->h2c_dst, 64);
-    d.hash_kind = s->hash_id;
-    return d;
 }
 
 // cooperative verification kernels: eight lanes per item (te_coop.cuh), eight items per block.  They cut the latency of an item
@@ -310,17 +266,6 @@ struct RingVerifier {
 
 using namespace dr;
 
-#define DR_API_BEGIN try {
-#define DR_API_END                            \
-    }                                         \
-    catch (const Error& e) {                  \
-        return set_error(e.code, e.what());   \
-    }                                         \
-    catch (const std::exception& e) {         \
-        return set_error(DR_ECUDA, e.what()); \
-    }                                         \
-    return DR_OK;
-
 extern "C" {
 
 int dr_ring_verify_set_msm_threshold(size_t n) {
@@ -362,7 +307,7 @@ int dr_pedersen_verify_batch(dr_ctx* c, const dr_vrf_suite* suite, size_t n, con
     if (!ctx || (n && (!proofs192 || !verdict))) throw Error(DR_EINVAL, "bad argument");
     ctx->activate();
     if (!n) return DR_OK;
-    SuiteDev su = suite_from_abi(suite);
+    SuiteDev su = suite_param(suite);
     ItemsDev items;
     upload_items(ctx, items, n, blob, in_off, in_len, ad_off, ad_len);
     const uint32_t m = (uint32_t)n;
@@ -385,7 +330,7 @@ static void ietf_verify_batch(Ctx* ctx, const dr_vrf_suite* suite, uint32_t thin
     if (!ctx || (n && (!public_keys32 || !proofs || !verdict))) throw Error(DR_EINVAL, "bad argument");
     ctx->activate();
     if (!n) return;
-    SuiteDev su = suite_from_abi(suite);
+    SuiteDev su = suite_param(suite);
     ItemsDev items;
     upload_items(ctx, items, n, blob, in_off, in_len, ad_off, ad_len);
     const uint32_t m = (uint32_t)n, npts = thin ? 3 : 2, plen = thin ? 96 : 80;
@@ -435,7 +380,7 @@ static void vrf_prove_batch(Ctx* ctx, const dr_vrf_suite* suite, int kind, size_
     if (!ctx || (n && (!sks32 || !out))) throw Error(DR_EINVAL, "bad argument");
     ctx->activate();
     if (!n) return;
-    SuiteDev su = suite_from_abi(suite);
+    SuiteDev su = suite_param(suite);
     auto g_table = ctx->fixed_table(su.generator), b_table = ctx->fixed_table(su.blinding_base);
     su.g_tab = g_table->tab.p;
     su.b_tab = b_table->tab.p;
@@ -533,13 +478,11 @@ int dr_ring_verifier_create(dr_ctx* c, const dr_ring_params* prm, const uint8_t*
     DR_API_BEGIN
     Ctx* ctx = (Ctx*)c;
     if (!ctx || !prm || !g1_0_be96 || !g2_be192 || !root144 || !out) throw Error(DR_EINVAL, "bad argument");
-    const uint32_t N = prm->domain_size;
-    if (N < 512 || N > 65536 || (N & (N - 1))) throw Error(DR_EINVAL, "domain_size must be a power of two in [512, 65536]");
-    if (prm->suite_id_len > 32 || prm->h2c_dst_len > 64) throw Error(DR_EINVAL, "suite id / DST too long");
-    if (prm->hash_id > 1) throw Error(DR_EINVAL, "unknown suite hash");
+    check_domain_size(prm->domain_size);
     ctx->activate();
     auto v = std::make_unique<RingVerifier>();
     v->ctx = ctx;
+    v->suite = suite_param(*prm);
     // RingRoot.decode (root.py:89-109): three compressed points, no subgroup check (blst); the transcript absorbs their
     // uncompressed encodings
     uint8_t fixed_be96[288];
@@ -548,15 +491,8 @@ int dr_ring_verifier_create(dr_ctx* c, const dr_ring_params* prm, const uint8_t*
         if (!g1_decode(a, root144 + 48 * i, 48)) throw Error(DR_EINVAL, "invalid BLS12-381 G1 encoding in ring root");
         g1_serialize(fixed_be96 + 96 * i, a);
     }
-    v->vk = make_verifier_key(ctx, N, fr_param(prm->omega), te_param(prm->seed), prm->suite_id, prm->suite_id_len, g1_0_be96, g2_be192, fixed_be96, v->lines);
+    v->vk = make_verifier_key(ctx, prm->domain_size, fr_param(prm->omega), te_param(prm->seed), prm->suite_id, prm->suite_id_len, g1_0_be96, g2_be192, fixed_be96, v->lines);
     for (int i = 0; i < 3; i++) v->vk.fixed_outside[i] = g1_in_subgroup(v->vk.fixed[i]) ? 0 : 1;
-    v->suite.generator = te_param(prm->generator);
-    v->suite.blinding_base = te_param(prm->blinding_base);
-    v->suite.suite_id_len = prm->suite_id_len;
-    memcpy(v->suite.suite_id, prm->suite_id, 32);
-    v->suite.dst_len = prm->h2c_dst_len;
-    memcpy(v->suite.dst, prm->h2c_dst, 64);
-    v->suite.hash_kind = prm->hash_id;
     memcpy(v->g1_0_be96, g1_0_be96, 96);
     *out = (dr_ring_verifier*)v.release();
     DR_API_END

@@ -25,8 +25,9 @@ namespace dr {
 
 constexpr uint32_t SCALAR_BITS = 253;
 
-// What a pass reads that depends only on the domain size N or on the suite, passed to kernels by value.  The ring's own data
-// (keys, fixed columns, transcript prefix) is in RingTab, so that one pass can prove items of several rings.
+// What a pass reads that depends only on the domain size N, and the accumulator seed, passed to kernels by value.  The ring's own
+// data (keys, fixed columns, transcript prefix) is in RingTab, so that one pass can prove items of several rings; the suite is a
+// SuiteDev, read only by the Pedersen stages.
 struct RingDev {
     uint32_t N, logN, last;            // last = N - 4 (last accumulator row)
     const Fr* tw_fwd;                  // [N/2] w^k
@@ -38,13 +39,17 @@ struct RingDev {
     Fr omega;                          // w
     Fr w_last;                         // w^(N-4)
     Fr tail[4];                        // coefficients of (X - w^(N-1))(X - w^(N-2))(X - w^(N-3))
-    TEAffine seed, blinding_base, generator;
-    const TEPre* g_tab;  // window tables of generator / blinding_base for te_mul_fixed (TeFixedTableBody)
+    TEAffine seed;
+};
+
+struct SuiteDev {  // VRF suite constants (dot_ring/curve/specs/bandersnatch.py:48-107)
+    TEAffine generator, blinding_base;
+    const TEPre* g_tab;  // te_mul_fixed window tables of the generator / blinding base (TeFixedTableBody)
     const TEPre* b_tab;
     uint32_t suite_id_len;
     uint8_t suite_id[32];
     uint32_t dst_len;
-    uint8_t dst[64];  // hash-to-curve DST (without the trailing length byte)
+    uint8_t dst[64];     // hash-to-curve DST (without the trailing length byte)
     uint32_t hash_kind;  // 0: SHA-512 suite (XMD h2c, counter-mode squeeze), 1: SHAKE128 suite (XOF h2c, direct squeeze)
 };
 
@@ -201,16 +206,15 @@ DR_HD void sha_absorb_point(VrfHash& s, const TEAffine& p) {
 }
 
 // expand_message_xmd(SHA-512) for 96 output bytes (curve.py:145-185; Z_pad = 48 bytes for this suite)
-template <class S>
-DR_HD_COLD void h2c_uniform_bytes(const S& rg, const uint8_t* msg, uint32_t msg_len, uint8_t* out96) {
-    uint8_t dst_prime_len = (uint8_t)rg.dst_len;
-    if (rg.hash_kind != 0) {  // expand_message_xof: SHAKE128(msg | I2OSP(96, 2) | DST | I2OSP(len(DST), 1))
+DR_HD_COLD void h2c_uniform_bytes(const SuiteDev& su, const uint8_t* msg, uint32_t msg_len, uint8_t* out96) {
+    uint8_t dst_prime_len = (uint8_t)su.dst_len;
+    if (su.hash_kind != 0) {  // expand_message_xof: SHAKE128(msg | I2OSP(96, 2) | DST | I2OSP(len(DST), 1))
         Shake128 x;
         x.init();
         x.absorb(msg, msg_len);
         uint8_t lib2[2] = {0, 96};
         x.absorb(lib2, 2);
-        x.absorb(rg.dst, rg.dst_len);
+        x.absorb(su.dst, su.dst_len);
         x.absorb_byte(dst_prime_len);
         x.squeeze_snapshot(out96, 96);
         return;
@@ -223,7 +227,7 @@ DR_HD_COLD void h2c_uniform_bytes(const S& rg, const uint8_t* msg, uint32_t msg_
     h.update(msg, msg_len);
     uint8_t lib[3] = {0, 96, 0};
     h.update(lib, 3);
-    h.update(rg.dst, rg.dst_len);
+    h.update(su.dst, su.dst_len);
     h.update_byte(dst_prime_len);
     uint8_t b0[64];
     h.final(b0);
@@ -235,16 +239,15 @@ DR_HD_COLD void h2c_uniform_bytes(const S& rg, const uint8_t* msg, uint32_t msg_
         for (int i = 0; i < 64; i++) x[i] = blk == 1 ? b0[i] : (uint8_t)(b0[i] ^ prev[i]);
         g.update(x, 64);
         g.update_byte((uint8_t)blk);
-        g.update(rg.dst, rg.dst_len);
+        g.update(su.dst, su.dst_len);
         g.update_byte(dst_prime_len);
         g.final(prev);
         for (int i = 0; i < 64 && 64 * (blk - 1) + i < 96; i++) out96[64 * (blk - 1) + i] = prev[i];
     }
 }
-template <class S>
-DR_HD TEAffine vrf_encode_to_curve(const S& rg, const uint8_t* msg, uint32_t msg_len) {
+DR_HD TEAffine vrf_encode_to_curve(const SuiteDev& su, const uint8_t* msg, uint32_t msg_len) {
     uint8_t u[96];
-    h2c_uniform_bytes(rg, msg, msg_len, u);
+    h2c_uniform_bytes(su, msg, msg_len, u);
     return te_encode_to_curve_from_u(fr_from_be48_mod(u), fr_from_be48_mod(u + 48));
 }
 
@@ -252,14 +255,13 @@ DR_HD TEAffine vrf_encode_to_curve(const S& rg, const uint8_t* msg, uint32_t msg
 // First half: everything up to the blinded key, in two steps around the blinding-base multiplication so that the cooperative
 // prover can run the multiplications on several lanes.
 // Step 1: public key and output point (given in extended coordinates), VRF transcript, blinding factor.  Writes O into out192.
-template <class S>
-DR_HD_COLD void pedersen_begin_transcript(const S& rg, const Fn& x, const TEAffine& input, const TEExt& pk_ext, const TEExt& output_ext, const uint8_t* ad,
+DR_HD_COLD void pedersen_begin_transcript(const SuiteDev& su, const Fn& x, const TEAffine& input, const TEExt& pk_ext, const TEExt& output_ext, const uint8_t* ad,
                                           uint32_t ad_len, uint8_t* out192, TEAffine& pk, uint32_t* blinding_raw, VrfHash& tr) {
     TEAffine output;
     te_to_affine2(pk_ext, output_ext, pk, output);
     // vrf_transcript (primitives.py:102-144) with one I/O pair
-    tr.init(rg.hash_kind);
-    tr.update(rg.suite_id, rg.suite_id_len);
+    tr.init(su.hash_kind);
+    tr.update(su.suite_id, su.suite_id_len);
     tr.update_byte(0x02);
     uint8_t le[8] = {1, 0, 0, 0, 0, 0, 0, 0};
     tr.update(le, 8);
@@ -283,18 +285,16 @@ DR_HD_COLD void pedersen_begin_blind(const TEAffine& pk, const TEExt& bB_ext, ui
 }
 // Writes O | Ybar into out192; returns the public key, the blinded key, the blinding factor and the transcript state the second
 // half continues from.  `input` is the hash-to-curve point.
-template <class S>
-DR_HD_COLD void pedersen_prove_begin(const S& rg, const uint8_t* sk32, const TEAffine& input, const uint8_t* ad, uint32_t ad_len, uint8_t* out192, TEAffine& pk,
+DR_HD_COLD void pedersen_prove_begin(const SuiteDev& su, const uint8_t* sk32, const TEAffine& input, const uint8_t* ad, uint32_t ad_len, uint8_t* out192, TEAffine& pk,
                                      TEAffine& blinded, uint32_t* blinding_raw, VrfHash& tr) {
     Fn x = fp_from_le_bytes_mod<Fn>(sk32, 32);
     uint32_t xr[8];
     fn_raw_limbs(xr, x);
-    pedersen_begin_transcript(rg, x, input, te_mul_fixed(rg.g_tab, xr), te_mul_glv(input, xr), ad, ad_len, out192, pk, blinding_raw, tr);
-    pedersen_begin_blind(pk, te_mul_fixed(rg.b_tab, blinding_raw), out192, blinded, tr);
+    pedersen_begin_transcript(su, x, input, te_mul_fixed(su.g_tab, xr), te_mul_glv(input, xr), ad, ad_len, out192, pk, blinding_raw, tr);
+    pedersen_begin_blind(pk, te_mul_fixed(su.b_tab, blinding_raw), out192, blinded, tr);
 }
 // Second half: nonces, R, Ok, challenge, responses.  Writes R | Ok | s | sb into out192 + 64.
-template <class S>
-DR_HD_COLD void pedersen_prove_finish(const S& rg, const uint8_t* sk32, const TEAffine& input, const uint32_t* blinding_raw, const VrfHash& tr, uint8_t* out192) {
+DR_HD_COLD void pedersen_prove_finish(const SuiteDev& su, const uint8_t* sk32, const TEAffine& input, const uint32_t* blinding_raw, const VrfHash& tr, uint8_t* out192) {
     Fn x = fp_from_le_bytes_mod<Fn>(sk32, 32);
     Fn b = Fn::zero();
     for (int i = 0; i < 8; i++) b.v[i] = blinding_raw[i];
@@ -305,7 +305,7 @@ DR_HD_COLD void pedersen_prove_finish(const S& rg, const uint8_t* sk32, const TE
     fn_raw_limbs(kr, k);
     fn_raw_limbs(kbr, kb);
     TEAffine R, ok;
-    te_to_affine2(te_add(te_mul_fixed(rg.g_tab, kr), te_mul_fixed(rg.b_tab, kbr)), te_mul_glv(input, kr), R, ok);
+    te_to_affine2(te_add(te_mul_fixed(su.g_tab, kr), te_mul_fixed(su.b_tab, kbr)), te_mul_glv(input, kr), R, ok);
     VrfHash tc = tr;
     tc.update_byte(0x40);
     sha_absorb_point(tc, R);
@@ -321,13 +321,12 @@ DR_HD_COLD void pedersen_prove_finish(const S& rg, const uint8_t* sk32, const TE
     fn_to_le_bytes(out192 + 160, sb);
 }
 // Writes O | Ybar | R | Ok | s | sb; returns the public key, the blinded key and the blinding factor.
-template <class S>
-DR_HD_COLD void pedersen_prove_core(const S& rg, const uint8_t* sk32, const uint8_t* msg, uint32_t msg_len, const uint8_t* ad, uint32_t ad_len, uint8_t* out192,
+DR_HD_COLD void pedersen_prove_core(const SuiteDev& su, const uint8_t* sk32, const uint8_t* msg, uint32_t msg_len, const uint8_t* ad, uint32_t ad_len, uint8_t* out192,
                                     TEAffine& pk, TEAffine& blinded, uint32_t* blinding_raw) {
-    TEAffine input = vrf_encode_to_curve(rg, msg, msg_len);
+    TEAffine input = vrf_encode_to_curve(su, msg, msg_len);
     VrfHash tr;
-    pedersen_prove_begin(rg, sk32, input, ad, ad_len, out192, pk, blinded, blinding_raw, tr);
-    pedersen_prove_finish(rg, sk32, input, blinding_raw, tr, out192);
+    pedersen_prove_begin(su, sk32, input, ad, ad_len, out192, pk, blinded, blinding_raw, tr);
+    pedersen_prove_finish(su, sk32, input, blinding_raw, tr, out192);
 }
 
 // Window table for te_mul_fixed: thread (w, c) of 32 x 16 writes the 16 entries d = 16c .. 16c + 15 of window w.
@@ -362,7 +361,7 @@ struct TeFixedTableBody {
 // table windows.  What remains on one lane: the affine conversions, the SHA-512 / SHAKE transcripts and the point encodings.
 DR_HD size_t pedersen_start_smem(uint32_t threads) { return (threads / COOP_LANES) * (sizeof(TeCoopState) + 2 * sizeof(TEAffine)); }
 struct PedersenStartBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProveInput* in, const uint8_t* blob, ProofState* st, uint32_t count) const {
+    DR_HD void operator()(const BlockCtx& ctx, SuiteDev su, const RingTab* tab, const ProveInput* in, const uint8_t* blob, ProofState* st, uint32_t count) const {
         const uint32_t items = ctx.nthreads / COOP_LANES;
         TeCoopState* cs = (TeCoopState*)ctx.smem;
         TEAffine* maps = (TEAffine*)(cs + items);  // [items][2]
@@ -373,7 +372,7 @@ struct PedersenStartBody {
             if (p < count && lane < 2) {
                 const ProveInput& pi = in[p];
                 uint8_t u[96];
-                h2c_uniform_bytes(rg, blob + pi.alpha_off, pi.alpha_len, u);
+                h2c_uniform_bytes(su, blob + pi.alpha_off, pi.alpha_len, u);
                 maps[2 * item + lane] = te_map_to_curve_ell2(fr_from_be48_mod(u + 48 * lane));
             }
         }
@@ -405,7 +404,7 @@ struct PedersenStartBody {
             if (s.live) {
                 uint32_t xr[8];
                 fn_raw_limbs(xr, fp_from_le_bytes_mod<Fn>(in[p].sk, 32));
-                te_mul_fixed_coop_partial(t % COOP_LANES, rg.g_tab, xr, s.part);
+                te_mul_fixed_coop_partial(t % COOP_LANES, su.g_tab, xr, s.part);
             }
         }
         DR_BLOCK_SYNC();
@@ -418,7 +417,7 @@ struct PedersenStartBody {
                 const ProveInput& pi = in[p];
                 const TEExt output{s.acc.c[CX], s.acc.c[CY], s.acc.c[CZ], s.acc.c[CT]};
                 TEAffine pk;
-                pedersen_begin_transcript(rg, fp_from_le_bytes_mod<Fn>(pi.sk, 32), ps.vrf_input, te_fold_fixed_coop(s.part), output, blob + pi.ad_off, pi.ad_len, ps.pedersen,
+                pedersen_begin_transcript(su, fp_from_le_bytes_mod<Fn>(pi.sk, 32), ps.vrf_input, te_fold_fixed_coop(s.part), output, blob + pi.ad_off, pi.ad_len, ps.pedersen,
                                           pk, ps.t, ps.vrf_tr);
                 s.m[0] = pk.x;
                 s.m[1] = pk.y;
@@ -429,7 +428,7 @@ struct PedersenStartBody {
         // E. b * B by windows
         DR_THREAD_LOOP(t, ctx) {
             TeCoopState& s = cs[t / COOP_LANES];
-            if (s.live) te_mul_fixed_coop_partial(t % COOP_LANES, rg.b_tab, s.k, s.part);
+            if (s.live) te_mul_fixed_coop_partial(t % COOP_LANES, su.b_tab, s.k, s.part);
         }
         DR_BLOCK_SYNC();
         // F. blinded key; ring-membership check of the producer key against the item's ring
@@ -459,7 +458,7 @@ struct PedersenStartBody {
 // hash-to-curve, no sk * G, no Pedersen transcript; the host has checked t < order and k < max_ring.
 DR_HD size_t ring_proof_start_smem(uint32_t threads) { return (size_t)threads * sizeof(TEExt); }
 struct RingProofStartBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const RingTab* tab, const ProveInput* in, ProofState* st, uint32_t count) const {
+    DR_HD void operator()(const BlockCtx& ctx, SuiteDev su, const RingTab* tab, const ProveInput* in, ProofState* st, uint32_t count) const {
         const uint32_t items = ctx.nthreads / COOP_LANES;
         TEExt* part = (TEExt*)ctx.smem;  // [items][COOP_LANES]
         auto limbs = [](uint32_t* out, const uint8_t* le32) {
@@ -471,7 +470,7 @@ struct RingProofStartBody {
             if (p < count) {
                 uint32_t tr[8];
                 limbs(tr, in[p].sk);
-                te_mul_fixed_coop_partial(t % COOP_LANES, rg.b_tab, tr, part + COOP_LANES * item);
+                te_mul_fixed_coop_partial(t % COOP_LANES, su.b_tab, tr, part + COOP_LANES * item);
             }
         }
         DR_BLOCK_SYNC();
@@ -494,12 +493,12 @@ struct RingProofStartBody {
 
 // Second half, one thread per proof; nothing of the ring proof depends on it, so it runs on the side stream.
 struct PedersenFinishBody {
-    DR_HD void operator()(const BlockCtx& ctx, RingDev rg, const ProveInput* in, ProofState* st, uint32_t count) const {
+    DR_HD void operator()(const BlockCtx& ctx, SuiteDev su, const ProveInput* in, ProofState* st, uint32_t count) const {
         DR_THREAD_LOOP(t, ctx) {
             uint32_t p = ctx.bx * ctx.nthreads + t;
             if (p < count) {
                 ProofState& ps = st[p];
-                pedersen_prove_finish(rg, in[p].sk, ps.vrf_input, ps.t, ps.vrf_tr, ps.pedersen);
+                pedersen_prove_finish(su, in[p].sk, ps.vrf_input, ps.t, ps.vrf_tr, ps.pedersen);
             }
         }
     }

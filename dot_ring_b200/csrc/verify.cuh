@@ -18,17 +18,6 @@
 
 namespace dr {
 
-struct SuiteDev {  // VRF suite constants (dot_ring/curve/specs/bandersnatch.py:48-107)
-    TEAffine generator, blinding_base;
-    const TEPre* g_tab;  // te_mul_fixed tables of the generator / blinding base (provers and the Pedersen verifier)
-    const TEPre* b_tab;
-    uint32_t suite_id_len;
-    uint8_t suite_id[32];
-    uint32_t dst_len;
-    uint8_t dst[64];
-    uint32_t hash_kind;  // 0 SHA-512, 1 SHAKE128 (ring.cuh: VrfHash)
-};
-
 struct VerifyInput {  // host-packed per item: salt|alpha and ad inside the blob
     uint32_t in_off, in_len, ad_off, ad_len;
 };
@@ -57,8 +46,7 @@ struct TeDecodeManyBody {
 };
 
 // Pedersen verification equations for one decoded proof; pts = O, Ybar, R, Ok.  Returns status bits.
-template <class S>
-DR_HD_COLD uint32_t pedersen_verify_core(const S& su, const TEAffine* pts, const uint8_t* ok4, const uint8_t* proof192, const uint8_t* msg, uint32_t msg_len,
+DR_HD_COLD uint32_t pedersen_verify_core(const SuiteDev& su, const TEAffine* pts, const uint8_t* ok4, const uint8_t* proof192, const uint8_t* msg, uint32_t msg_len,
                                          const uint8_t* ad, uint32_t ad_len) {
     if (!(ok4[0] && ok4[1] && ok4[2] && ok4[3])) return ST_MALFORMED;
     uint32_t ks[3][8];
